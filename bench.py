@@ -2,7 +2,7 @@
 """Headline benchmark: norm.coex on 100k cells x 20k genes (BASELINE.json metric), one process
 per GPU.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A step is one pass of the hot path over the synthetic matrix: residualise + quantise, (N > 1:
@@ -13,6 +13,8 @@ all-gather of the digit planes), tensor-core contraction with the fused r / P ep
 The reference arm (--impl reference) times the CPU port of the reference (oracle/) on the box's
 host cores on a bounded sample of the same workload and extrapolates by the reference's own
 tile count (association.py:854-894).
+--dump-outputs DIR writes what the last timed step computed (see dump_outputs); the inputs are
+generated from fixed seeds, so two builds run with the same arguments can be compared array by array.
 """
 import argparse
 import json
@@ -40,6 +42,31 @@ WORKLOADS = {
 METRIC = "coex gene-pairs/s (r+P)"
 UNIT = "pairs/s"
 SEED = 1004
+DUMP_SAMPLE = 1 << 19            # entries --dump-outputs keeps of a larger output
+DUMP_BYTES = 64 << 20            # and the most it writes in all
+
+
+def dump_outputs(path, arrays):
+    """Write each array of ``arrays`` (name -> host or device array, None skipped) as <path>/<name>.npy
+    in float64.  An array of more than DUMP_SAMPLE entries is written as the 1-D run of its entries at
+    DUMP_SAMPLE positions drawn with a fixed seed (the same positions for every array of that shape),
+    and the positions as <path>/<name>_index.npy: one row of coordinates per dimension."""
+    import torch
+    os.makedirs(path, exist_ok=True)
+    files = {}
+    for name, a in arrays.items():
+        if a is None:
+            continue
+        t = torch.as_tensor(a)
+        if t.numel() > DUMP_SAMPLE:
+            flat = np.sort(np.random.default_rng(SEED).choice(t.numel(), DUMP_SAMPLE, replace=False, shuffle=False))
+            files[name + "_index"] = np.array(np.unravel_index(flat, tuple(t.shape)), dtype=np.float64)
+            t = t.reshape(-1)[torch.from_numpy(flat).to(t.device)]
+        files[name] = t.to(torch.float64).cpu().numpy()
+    total = sum(v.nbytes for v in files.values())
+    assert total <= DUMP_BYTES, "--dump-outputs would write %d bytes" % total
+    for name, v in files.items():
+        np.save(os.path.join(path, name + ".npy"), v, allow_pickle=False)
 
 
 def cpu_sample_genes(cores, n_gene):
@@ -365,6 +392,9 @@ def run_ours(args, n_gene, n_cell, wl_name, wl_desc):
     ms_total = max_over_ranks(ev0.elapsed_time(ev1))
     launches = engine.LAUNCHES - launches0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        # what norm.coex returns: (P, dot, var)
+        dump_outputs(args.dump_outputs, {"P": P, "dot": D, "var": local_sl.var})
     ms_step = ms_total / args.steps
     value = pairs / (ms_step * 1e-3)
     k_list = [sum(e0.elapsed_time(e1) for e0, e1 in evs) for evs in contract_ms]
@@ -791,8 +821,10 @@ def run_de(args, wl_name):
     def step():
         return norm.de(p["dg"], p["dt"], p["dc"], single=single, precision=precision)
 
+    # each step's result stays alive while the next one runs, in the warm-up too, so that the timed steps
+    # find the allocator's cache already sized for two results
     for _ in range(args.warmup):
-        step()
+        res = step()
     barrier()
     sampler = ClockSampler(local)
     if rank == 0:
@@ -801,12 +833,15 @@ def run_de(args, wl_name):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        step()
+        res = step()
     e1.record()
     barrier()
     ms_step = max_over_ranks(e0.elapsed_time(e1)) / args.steps
     launches = engine.LAUNCHES - launches0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict(zip(("P", "gamma", "alpha", "varg", "vart"), res)))
+    del res
     phases, planes_x = de_phase_times(torch, ctx, p, single, n_slices, n_products)
 
     # ---- end to end: pinned host dg / dt / dc in, host P / gamma / variances out
@@ -1126,7 +1161,14 @@ def main():
     ap.add_argument("--no-de", action="store_true", help="skip the secondary DE tests/s measurement")
     ap.add_argument("--umma-pair", type=int, default=None, help="test hook: 1 = cta_group::2 kernel, 0 = single-CTA")
     ap.add_argument("--opt", action="append", default=[], help="test hook: name=value for nsr_set_option")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the arrays the last one computed as DIR/<name>.npy (float64; "
+                         "an array of more than %d entries as a fixed, seeded sample of its entries)" % DUMP_SAMPLE)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.gpus != 1 or int(os.environ.get("WORLD_SIZE", "1")) != 1):
+        ap.error("--dump-outputs takes --impl ours on one GPU")
     if args.workload in DE_WORKLOADS:
         if args.impl == "reference":
             run_de_reference(args, args.workload)
