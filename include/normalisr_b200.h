@@ -355,6 +355,23 @@ int nsr_lcpm_apply(nsr_ctx* ctx, uintptr_t stream, const void* reads, int itemsi
                    const double* noise, int64_t ld_noise, uint64_t seed, int64_t row0, const double* shift,
                    double* out, int64_t ldo);
 
+/* The same two passes on a CSR count matrix (genes x n, never expanded): row g holds the entries
+ * indptr[g] .. indptr[g + 1] - 1 of (indices, values), column indices ascending and unique within a row,
+ * values int32 or int64 (itemsize 4 / 8; device arrays; indptr holds absolute offsets, so a block of rows
+ * is passed as indptr + first row).  Cells without an entry have count 0.  Arguments and results as
+ * nsr_lcpm_colstats / nsr_lcpm_apply, and the same bits: a CTA expands the entries of 64 genes x 256 cells
+ * into shared memory (64 KB as int32, 128 KB as int64) and runs the dense kernels' per-cell loop on it.
+ * The counts are read once per pass (O(nnz)); n <= INT_MAX.  The min / max / total that resampling needs
+ * is nsr_lcpm_scan over the values as a 1 x nnz matrix, with 0 added when some entry is not stored. */
+int nsr_lcpm_colstats_csr(nsr_ctx* ctx, uintptr_t stream, const int64_t* indptr, const int32_t* indices,
+                          const void* values, int itemsize, int64_t genes, int64_t n, const double* lut,
+                          const double* lut_exp, int64_t lut_len, const double* lut_sd, const double* noise,
+                          int64_t ld_noise, uint64_t seed, int64_t row0, double* colstats, long long* minmax);
+int nsr_lcpm_apply_csr(nsr_ctx* ctx, uintptr_t stream, const int64_t* indptr, const int32_t* indices,
+                       const void* values, int itemsize, int64_t genes, int64_t n, const double* lut,
+                       int64_t lut_len, const double* lut_sd, const double* noise, int64_t ld_noise,
+                       uint64_t seed, int64_t row0, const double* shift, double* out, int64_t ldo);
+
 /* compute_var (norm.compute_var, src/normalisr/norm.py:56-128), column pass: with res = X - coef Qt
  * (the covariate-projection residual, not materialised; coef from nsr_project_coef),
  *   out[k] = sum_g ((res[g][k] - mean[g]) * inv_std[g])^2      (norm.py:103).   rank <= 16. */

@@ -80,6 +80,10 @@ _SIGNATURES = {
                                   ctypes.c_uint64, c_i64, c_vp, c_vp]),
     "nsr_lcpm_apply": (c_int, [c_vp, c_up, c_vp, c_int, c_i64, c_i64, c_i64, c_vp, c_i64, c_vp, c_vp, c_i64,
                                ctypes.c_uint64, c_i64, c_vp, c_vp, c_i64]),
+    "nsr_lcpm_colstats_csr": (c_int, [c_vp, c_up, c_vp, c_vp, c_vp, c_int, c_i64, c_i64, c_vp, c_vp, c_i64, c_vp,
+                                      c_vp, c_i64, ctypes.c_uint64, c_i64, c_vp, c_vp]),
+    "nsr_lcpm_apply_csr": (c_int, [c_vp, c_up, c_vp, c_vp, c_vp, c_int, c_i64, c_i64, c_vp, c_i64, c_vp, c_vp, c_i64,
+                                   ctypes.c_uint64, c_i64, c_vp, c_vp, c_i64]),
     "nsr_colvar": (c_int, [c_vp, c_up, c_vp, c_i64, c_i64, c_i64, c_vp, c_int, c_i64, c_vp, c_i64, c_vp, c_vp, c_vp]),
     "nsr_cov_gram": (c_int, [c_vp, c_up, c_vp, c_int, c_i64, c_i64, c_vp]),
     "nsr_cov_apply": (c_int, [c_vp, c_up, c_vp, c_int, c_int, c_vp, c_i64, c_i64, c_vp, c_i64]),

@@ -89,6 +89,91 @@ lcpm_scan_kernel(const T* __restrict__ reads, int64_t genes, int64_t n, int64_t 
     }
 }
 
+// The per-cell loops of both passes for the CSR kernels: count(g) is the count of gene g in the thread's cell,
+// read from the shared-memory tile the kernel expanded its entries into.  Each is the loop of the dense kernel
+// below (lcpm_colstats_kernel, lcpm_apply_kernel) statement for statement, so that both paths compute the same
+// bits; the dense kernels keep their own copy because calling these through a strided-load accessor changes
+// their SASS.  Genes [g0, g1): one range of at most kLcGeneSplit.
+// Column pass: the sum of exponentials starts at 0.0 for the range and takes the genes in batches of 8, in gene
+// order (table values first, then the exponentials of counts beyond the table); every gene contributes, zeros
+// included, so this order is part of the result.
+template <typename T, bool NOISY, typename Count>
+__device__ __forceinline__ void lc_colstats_cell(Count count, int64_t g0, int64_t g1, int64_t k, const double* __restrict__ lut,
+                                                 const double* __restrict__ lut_exp, T len_t, const LcNoise& nz_,
+                                                 double& se, unsigned long long& tot, int& nz, T& any_or, T& mx) {
+    constexpr int kBatch = 8;                    // counts loaded before any of them is used: the table gather
+                                                 // and the rare large-count branch must not serialise the loads
+#pragma unroll 1
+    for (int64_t g = g0; g < g1; g += kBatch) {
+        T cc[kBatch];
+#pragma unroll
+        for (int i = 0; i < kBatch; ++i) cc[i] = g + i < g1 ? count(g + i) : (T)0;
+        bool big = false;
+#pragma unroll
+        for (int i = 0; i < kBatch; ++i) {
+            const T c = cc[i];
+            const bool in = g + i < g1;
+            const T ci = c < 0 ? (T)0 : (c >= len_t ? (T)(len_t - 1) : c);
+            if (NOISY) {
+                if (in) {
+                    const double z = nz_.noise ? nz_.noise[(g + i) * nz_.ld_noise + k]
+                                               : philox_normal((uint64_t)((nz_.row0 + g + i) * nz_.n_total + k), nz_.seed);
+                    se += exp(fma(nz_.lut_sd[ci], z, lut[ci]));
+                }
+            } else {
+                // exp(lut[c]) tabulated: the pass is a pure gather; counts beyond the table are added below
+                const double v = lut_exp[ci];
+                se += (in && c < len_t) ? v : 0.0;
+                big = big || c >= len_t;
+            }
+            tot += (unsigned long long)(long long)c;
+            nz += c != 0 ? 1 : 0;
+            any_or |= c;
+            mx = c > mx ? c : mx;
+        }
+        if (!NOISY && big) {
+#pragma unroll
+            for (int i = 0; i < kBatch; ++i)
+                if (cc[i] >= len_t) se += exp(lc_digamma(1.0 + (double)cc[i]));
+        }
+    }
+}
+
+// Apply pass: out[g][k] = value - sh for the genes of the range.
+template <bool NOISY, typename Count>
+__device__ __forceinline__ void lc_apply_cell(Count count, int64_t g0, int64_t g1, int64_t k, const double* __restrict__ lut,
+                                              int64_t lut_len, const LcNoise& nz_, double sh, double* __restrict__ out,
+                                              int64_t ldo) {
+#pragma unroll 8
+    for (int64_t g = g0; g < g1; ++g) {
+        const long long c = (long long)count(g);
+        const long long ci = c < 0 ? 0 : (c >= lut_len ? lut_len - 1 : c);
+        double v = (NOISY || c < lut_len) ? lut[ci] : lc_digamma(1.0 + (double)c);
+        if (NOISY) {
+            const double z = nz_.noise ? nz_.noise[g * nz_.ld_noise + k]
+                                       : philox_normal((uint64_t)((nz_.row0 + g) * nz_.n_total + k), nz_.seed);
+            v = fma(nz_.lut_sd[ci], z, v);
+        }
+        out[g * ldo + k] = v - sh;
+    }
+}
+
+// Negativity check and largest count of the CTA (one atomic per warp)
+template <typename T>
+__device__ __forceinline__ void lc_minmax(T any_or, T mx, long long* __restrict__ minmax) {
+    long long neg = any_or < 0 ? -1 : 0, m = (long long)mx;
+#pragma unroll
+    for (int d = 16; d >= 1; d >>= 1) {
+        neg |= __shfl_xor_sync(0xffffffffu, neg, d);
+        const long long b = __shfl_xor_sync(0xffffffffu, m, d);
+        m = b > m ? b : m;
+    }
+    if ((threadIdx.x & 31) == 0) {
+        if (neg < 0) atomicMin(minmax, -1ll);    // "some count is negative" (lcpm.py:88-89); rare
+        if (m > *(volatile long long*)(minmax + 1)) atomicMax(minmax + 1, m);
+    }
+}
+
 template <typename T, bool NOISY>
 __global__ void __launch_bounds__(kLcThreads)
 lcpm_colstats_kernel(const T* __restrict__ reads, int64_t genes, int64_t n, int64_t ld,
@@ -191,6 +276,147 @@ lcpm_apply_kernel(const T* __restrict__ reads, int64_t genes, int64_t n, int64_t
     }
 }
 
+
+// ---- CSR counts (lcpm on sparse read-count matrices, never expanded to genes x cells) ----
+// A CTA owns one range of kLcGeneSplit genes (blockIdx.y, as the dense kernels) and a span of consecutive
+// 256-cell windows (blockIdx.x).  Per window it expands the range's stored entries into a 64 x 256 shared-memory
+// tile of counts (zeros elsewhere) and runs the dense kernels' per-cell loop on it: the same per-cell order of
+// operations, hence the same bits.  Column indices are ascending and unique within a row; each row keeps a cursor
+// that only moves forward through the span (one binary search per row at the start of the span), so the counts
+// are read once per pass: O(nnz) global traffic plus the (genes x cells) output of the apply pass.
+constexpr int kLcCsrCtasPerSm = 3;     // 64 KB int32 tile per CTA (a 128 KB int64 tile for counts >= 2^31: one)
+
+template <typename T>
+struct LcCsrTile {
+    T* tile;                           // [kLcGeneSplit][kLcThreads]
+    int64_t* cur;                      // per row: next entry to place
+    int64_t* stop;                     // per row: end of the row's entries
+    int rows;
+
+    // cursors of the range's rows at the first entry of column >= k_first
+    __device__ __forceinline__ void begin(const int64_t* __restrict__ indptr, const int32_t* __restrict__ idx,
+                                          int64_t k_first) {
+        const int t = threadIdx.x;
+        if (t < rows) {
+            int64_t lo = indptr[t], hi = indptr[t + 1];
+            stop[t] = hi;
+            while (lo < hi) {
+                const int64_t mid = (lo + hi) >> 1;
+                if ((int64_t)idx[mid] < k_first) lo = mid + 1;
+                else hi = mid;
+            }
+            cur[t] = lo;
+        }
+        __syncthreads();
+    }
+
+    // the counts of cells [k0, k0 + kLcThreads) into the tile: a warp owns 8 rows and takes 32 entries of a row at a
+    // time; the entries of the window are a prefix of what is left of the row.  The first 32 of all 8 rows are
+    // loaded together (independent loads), only rows with more than 32 entries in the window go round again.
+    __device__ __forceinline__ void expand(const int32_t* __restrict__ idx, const T* __restrict__ val, int64_t k0) {
+        constexpr int kWarps = kLcThreads / 32, kRows = kLcGeneSplit / kWarps;
+#pragma unroll 8
+        for (int g = 0; g < kLcGeneSplit; ++g) tile[g * kLcThreads + threadIdx.x] = (T)0;
+        __syncthreads();
+        const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+        int64_t p[kRows], c[kRows];
+        T v[kRows];
+#pragma unroll
+        for (int q = 0; q < kRows; ++q) {
+            const int r = warp + q * kWarps;
+            p[q] = r < rows ? cur[r] : 0;
+            const int64_t j = p[q] + lane;
+            const bool live = r < rows && j < stop[r];
+            c[q] = live ? (int64_t)idx[j] : LLONG_MAX;
+            v[q] = live ? val[j] : (T)0;
+        }
+#pragma unroll
+        for (int q = 0; q < kRows; ++q) {
+            const int r = warp + q * kWarps;
+            for (;;) {
+                const bool in = c[q] < k0 + kLcThreads;
+                if (in) tile[r * kLcThreads + (int)(c[q] - k0)] = v[q];
+                const int m = __popc(__ballot_sync(0xffffffffu, in));
+                p[q] += m;
+                if (m < 32) break;
+                const int64_t j = p[q] + lane;
+                const bool live = j < stop[r];
+                c[q] = live ? (int64_t)idx[j] : LLONG_MAX;
+                v[q] = live ? val[j] : (T)0;
+            }
+            if (lane == 0 && r < rows) cur[r] = p[q];
+        }
+        __syncthreads();
+    }
+};
+
+template <typename T, bool NOISY>
+__global__ void __launch_bounds__(kLcThreads, kLcCsrCtasPerSm)
+lcpm_colstats_csr_kernel(const int64_t* __restrict__ indptr, const int32_t* __restrict__ idx, const T* __restrict__ val,
+                         int64_t genes, int64_t n, int64_t span, const double* __restrict__ lut,
+                         const double* __restrict__ lut_exp, int64_t lut_len, LcNoise nz_, double* __restrict__ partial,
+                         long long* __restrict__ minmax) {
+    extern __shared__ __align__(16) unsigned char lc_smem[];
+    __shared__ int64_t cur[kLcGeneSplit], stop[kLcGeneSplit];
+    const int64_t g0 = (int64_t)blockIdx.y * kLcGeneSplit, g1 = min(genes, g0 + kLcGeneSplit);
+    LcCsrTile<T> t{reinterpret_cast<T*>(lc_smem), cur, stop, (int)(g1 - g0)};
+    const int64_t windows = (n + kLcThreads - 1) / kLcThreads;
+    const int64_t w0 = (int64_t)blockIdx.x * span, w1 = min(windows, w0 + span);
+    t.begin(indptr + g0, idx, w0 * kLcThreads);
+    const T len_t = (T)(lut_len > (int64_t)INT_MAX ? (int64_t)INT_MAX : lut_len);
+    T any_or = 0, mx = 0;
+    const T* my = t.tile + threadIdx.x - g0 * kLcThreads;
+    for (int64_t w = w0; w < w1; ++w) {
+        t.expand(idx, val, w * kLcThreads);
+        const int64_t k = w * kLcThreads + threadIdx.x;
+        if (k < n) {
+            double se = 0.0;
+            unsigned long long tot = 0;
+            int nz = 0;
+            lc_colstats_cell<T, NOISY>([&](int64_t g) { return my[g * kLcThreads]; }, g0, g1, k, lut, lut_exp, len_t,
+                                       nz_, se, tot, nz, any_or, mx);
+            double* o = partial + ((int64_t)blockIdx.y * 3) * n + k;
+            o[0] = se;
+            o[n] = (double)(long long)tot;
+            o[2 * n] = (double)nz;
+        }
+        __syncthreads();                               // the tile is refilled for the next window
+    }
+    if (minmax != nullptr) lc_minmax(any_or, mx, minmax);
+}
+
+template <typename T, bool NOISY>
+__global__ void __launch_bounds__(kLcThreads, kLcCsrCtasPerSm)
+lcpm_apply_csr_kernel(const int64_t* __restrict__ indptr, const int32_t* __restrict__ idx, const T* __restrict__ val,
+                      int64_t genes, int64_t n, int64_t span, const double* __restrict__ lut, int64_t lut_len, LcNoise nz_,
+                      const double* __restrict__ shift, double* __restrict__ out, int64_t ldo) {
+    extern __shared__ __align__(16) unsigned char lc_smem[];
+    __shared__ int64_t cur[kLcGeneSplit], stop[kLcGeneSplit];
+    const int64_t g0 = (int64_t)blockIdx.y * kLcGeneSplit, g1 = min(genes, g0 + kLcGeneSplit);
+    LcCsrTile<T> t{reinterpret_cast<T*>(lc_smem), cur, stop, (int)(g1 - g0)};
+    const int64_t windows = (n + kLcThreads - 1) / kLcThreads;
+    const int64_t w0 = (int64_t)blockIdx.x * span, w1 = min(windows, w0 + span);
+    t.begin(indptr + g0, idx, w0 * kLcThreads);
+    const T* my = t.tile + threadIdx.x - g0 * kLcThreads;
+    for (int64_t w = w0; w < w1; ++w) {
+        t.expand(idx, val, w * kLcThreads);
+        const int64_t k = w * kLcThreads + threadIdx.x;
+        if (k < n) {
+            const double sh = shift ? shift[k] : 0.0;
+            lc_apply_cell<NOISY>([&](int64_t g) { return my[g * kLcThreads]; }, g0, g1, k, lut, lut_len, nz_, sh, out, ldo);
+        }
+        __syncthreads();
+    }
+}
+
+// windows per CTA: enough CTAs for about four waves at kLcCsrCtasPerSm, one window each on small problems
+int64_t lc_csr_span(const nsr_ctx* ctx, int64_t n, int n_split) {
+    const int64_t windows = (n + kLcThreads - 1) / kLcThreads;
+    const int64_t want = (int64_t)ctx->sm_count * kLcCsrCtasPerSm * 4;
+    const int64_t per_range = max((int64_t)1, min(windows, (want + n_split - 1) / n_split));
+    return (windows + per_range - 1) / per_range;
+}
+
 }  // namespace
 
 extern "C" int nsr_lcpm_scan(nsr_ctx* ctx, uintptr_t stream, const void* reads, int itemsize, int64_t genes, int64_t n,
@@ -251,6 +477,71 @@ extern "C" int nsr_lcpm_apply(nsr_ctx* ctx, uintptr_t stream, const void* reads,
     if (itemsize == 4) { if (lut_sd) NSR_LA(int32_t, true); else NSR_LA(int32_t, false); }
     else { if (lut_sd) NSR_LA(int64_t, true); else NSR_LA(int64_t, false); }
 #undef NSR_LA
+    NSR_CHECK(cudaGetLastError());
+    return 0;
+}
+
+extern "C" int nsr_lcpm_colstats_csr(nsr_ctx* ctx, uintptr_t stream, const int64_t* indptr, const int32_t* indices,
+                                     const void* values, int itemsize, int64_t genes, int64_t n, const double* lut,
+                                     const double* lut_exp, int64_t lut_len, const double* lut_sd, const double* noise,
+                                     int64_t ld_noise, uint64_t seed, int64_t row0, double* colstats, long long* minmax) {
+    NSR_REQUIRE(ctx && indptr && indices && values && lut && colstats && (lut_sd || lut_exp),
+                "nsr_lcpm_colstats_csr: null argument");
+    NSR_REQUIRE((itemsize == 4 || itemsize == 8) && genes >= 1 && n >= 1 && n <= (int64_t)INT_MAX && lut_len >= 1 &&
+                    (!noise || ld_noise >= n),
+                "nsr_lcpm_colstats_csr: bad arguments (itemsize %d)", itemsize);
+    NSR_CHECK(cudaSetDevice(ctx->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    const int n_split = (int)((genes + kLcGeneSplit - 1) / kLcGeneSplit);
+    NSR_REQUIRE(n_split <= 65535, "nsr_lcpm_colstats_csr: too many genes for one call");
+    void* scratch = nullptr;
+    if (nsr_scratch(ctx, (size_t)n_split * 3 * n * sizeof(double), &scratch)) return 1;
+    const int64_t span = lc_csr_span(ctx, n, n_split);
+    const dim3 grid((unsigned)((n + kLcThreads * span - 1) / (kLcThreads * span)), (unsigned)n_split);
+    const size_t smem = (size_t)kLcGeneSplit * kLcThreads * itemsize;
+    const LcNoise nz{lut_sd, noise, ld_noise, seed, row0, n};
+#define NSR_LCS(T_, N_)                                                                                                \
+    do {                                                                                                               \
+        NSR_CHECK(cudaFuncSetAttribute((const void*)lcpm_colstats_csr_kernel<T_, N_>,                                  \
+                                       cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));                       \
+        lcpm_colstats_csr_kernel<T_, N_><<<grid, kLcThreads, smem, st>>>(indptr, indices, (const T_*)values, genes, n, \
+                                                                         span, lut, lut_exp, lut_len, nz,              \
+                                                                         (double*)scratch, minmax);                    \
+    } while (0)
+    if (itemsize == 4) { if (lut_sd) NSR_LCS(int32_t, true); else NSR_LCS(int32_t, false); }
+    else { if (lut_sd) NSR_LCS(int64_t, true); else NSR_LCS(int64_t, false); }
+#undef NSR_LCS
+    lcpm_colreduce_kernel<<<(unsigned)((3 * n + 255) / 256), 256, 0, st>>>((const double*)scratch, n, n_split, colstats);
+    NSR_CHECK(cudaGetLastError());
+    return 0;
+}
+
+extern "C" int nsr_lcpm_apply_csr(nsr_ctx* ctx, uintptr_t stream, const int64_t* indptr, const int32_t* indices,
+                                  const void* values, int itemsize, int64_t genes, int64_t n, const double* lut,
+                                  int64_t lut_len, const double* lut_sd, const double* noise, int64_t ld_noise,
+                                  uint64_t seed, int64_t row0, const double* shift, double* out, int64_t ldo) {
+    NSR_REQUIRE(ctx && indptr && indices && values && lut && out, "nsr_lcpm_apply_csr: null argument");
+    NSR_REQUIRE((itemsize == 4 || itemsize == 8) && genes >= 1 && n >= 1 && n <= (int64_t)INT_MAX && ldo >= n &&
+                    lut_len >= 1 && (!noise || ld_noise >= n),
+                "nsr_lcpm_apply_csr: bad arguments (itemsize %d)", itemsize);
+    NSR_CHECK(cudaSetDevice(ctx->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    const int n_split = (int)((genes + kLcGeneSplit - 1) / kLcGeneSplit);
+    NSR_REQUIRE(n_split <= 65535, "nsr_lcpm_apply_csr: too many genes for one call");
+    const int64_t span = lc_csr_span(ctx, n, n_split);
+    const dim3 grid((unsigned)((n + kLcThreads * span - 1) / (kLcThreads * span)), (unsigned)n_split);
+    const size_t smem = (size_t)kLcGeneSplit * kLcThreads * itemsize;
+    const LcNoise nz{lut_sd, noise, ld_noise, seed, row0, n};
+#define NSR_LAS(T_, N_)                                                                                                \
+    do {                                                                                                               \
+        NSR_CHECK(cudaFuncSetAttribute((const void*)lcpm_apply_csr_kernel<T_, N_>,                                     \
+                                       cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));                       \
+        lcpm_apply_csr_kernel<T_, N_><<<grid, kLcThreads, smem, st>>>(indptr, indices, (const T_*)values, genes, n,    \
+                                                                      span, lut, lut_len, nz, shift, out, ldo);        \
+    } while (0)
+    if (itemsize == 4) { if (lut_sd) NSR_LAS(int32_t, true); else NSR_LAS(int32_t, false); }
+    else { if (lut_sd) NSR_LAS(int64_t, true); else NSR_LAS(int64_t, false); }
+#undef NSR_LAS
     NSR_CHECK(cudaGetLastError());
     return 0;
 }

@@ -54,6 +54,30 @@ def release():
     _SLOTS.clear()
 
 
+def to_device(ctx, src, tag="flat"):
+    """A 1-D host tensor -> a new device tensor on the current stream, through the page-locked slots: the array is
+    taken as rows of 1 MB (and a shorter last row), at most STAGE_BYTES per slot.  Returns once the slots are free
+    again (the copies out of them are done), so the next call may use the same tag."""
+    n, es = src.numel(), src.element_size()
+    dst = torch.empty(max(1, n), dtype=src.dtype, device=ctx.device)[:n]
+    stream = torch.cuda.current_stream(ctx.device)
+    width = max(1, min(n, (1 << 20) // es))
+    rows = n // width
+    if rows:
+        step = max(1, min(rows, STAGE_BYTES // (width * es)))
+        stager = InputStager(src[:rows * width].view(rows, width), step, ctx.device, tag=tag)
+        for r0 in range(0, rows, step):
+            r1 = min(rows, r0 + step)
+            stager.copy_rows(dst[r0 * width:r1 * width].view(r1 - r0, width), r0, r1, stream)
+        stager.wait()
+    if rows * width < n:
+        tail = src[rows * width:].view(1, n - rows * width)
+        stager = InputStager(tail, 1, ctx.device, tag=tag + "-tail")
+        stager.copy_rows(dst[rows * width:].view(tail.shape), 0, 1, stream)
+        stager.wait()
+    return dst
+
+
 class InputStager:
     """Rows [r0, r1) of a 2-D host matrix (any dtype) -> a device buffer of the same dtype, asynchronously on a
     stream."""
@@ -91,6 +115,12 @@ class InputStager:
             ev = torch.cuda.Event()
             ev.record(stream)
         self.events[i] = ev
+
+    def wait(self):
+        """Until the copies out of the page-locked slots are done."""
+        for ev in (self.events if not self.pinned else ()):
+            if ev is not None:
+                ev.synchronize()
 
 
 class OutputDrain:
@@ -179,8 +209,8 @@ class RowBlocks:
 
     def __init__(self, ctx, src, rows_max, out_row_bytes=0, tag="blocks"):
         self.ctx = ctx
-        self.src = src
-        self.stager = InputStager(src, rows_max, ctx.device, tag=tag + "-in")
+        self.src = src                     # None: results only (the source is on the device already)
+        self.stager = InputStager(src, rows_max, ctx.device, tag=tag + "-in") if src is not None else None
         self.drain = OutputDrain(ctx, max(1 << 20, rows_max * out_row_bytes), count=2, tag=tag + "-out") \
             if out_row_bytes else None
 
