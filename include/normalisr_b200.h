@@ -63,6 +63,12 @@ int nsr_ctx_destroy(nsr_ctx* ctx);
 int64_t nsr_padded_cells(int64_t n);
 int nsr_cell_splits(int64_t n);
 
+/* The tile list of the cta_group::2 pair kernel, made from a list of n_tiles (tile_row, tile_col) pairs:
+ * entries (row block of CTA 0, row block of CTA 1 or -1, column block), at most n_tiles of them in `out`
+ * (3 int32 each); returns their count.  Every tile of the input is covered exactly once, as itself or - with
+ * `symmetric` (one operand against itself, tile_row <= tile_col) - as its transpose. */
+int64_t nsr_pair_tiles(const int32_t* tiles, int64_t n_tiles, int symmetric, int32_t* out);
+
 /* Residualise `rows` variables against an orthonormal covariate basis and quantise.
  *
  * Replaces association.py:226-233 (dx1 = dx - (dci (dc dx^T))^T dc; var = mean(dx1^2),
@@ -438,8 +444,9 @@ int nsr_tsv_write(const char* path, char delimiter, const double* data, int64_t 
 int nsr_mtx_shape(const char* path, int64_t* rows, int64_t* cols, int64_t* nnz, int* is_integer);
 int nsr_mtx_read(const char* path, int64_t nnz, int32_t* row, int32_t* col, double* val, int* symmetric, int threads);
 
-/* Test hooks: "hadamard" (0/1, default 1), "umma_pair" (1 = cta_group::2 kernel;
- * 0 = single-CTA kernel, default), "umma_kblock" (64 or 128 cells per pipeline stage of the single-CTA
+/* Test hooks: "hadamard" (0/1, default 1), "umma_pair" (-1 = the cta_group::2 pair kernel for single-segment
+ * NSR_MODE_COEX at 3 planes / 8 products, default; 0 = always the single-CTA kernel; 1 = the pair kernel wherever
+ * it applies), "umma_kblock" (64 or 128 cells per pipeline stage of the single-CTA
  * kernel, default 128), "umma_dynamic" (1 = tiles claimed from a global counter, default; 0 = static
  * round-robin), "split_k" (1 = launches with fewer than two waves of tiles split the cells into parts - work
  * items (tile, part) over all SMs, partial sums added in a fixed order by a second small kernel; default 1),

@@ -32,6 +32,7 @@ _SIGNATURES = {
     "nsr_padded_cells": (c_i64, [c_i64]),
     "nsr_set_option": (c_int, [ctypes.c_char_p, c_int]),
     "nsr_cell_splits": (c_int, [c_i64]),
+    "nsr_pair_tiles": (c_i64, [c_vp, c_i64, c_int, c_vp]),
     "nsr_residualize": (c_int, [c_vp, c_up, c_vp, c_i64, c_i64, c_i64, c_vp, c_int, c_i64, c_int, c_vp,
                                 c_i64, c_i64, c_vp, c_vp, c_vp, c_vp]),
     "nsr_contract": (c_int, [c_vp, c_up, c_int, c_int,

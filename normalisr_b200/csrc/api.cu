@@ -2,6 +2,8 @@
 #include <stdarg.h>
 #include <string.h>
 
+#include <algorithm>
+#include <array>
 #include <unordered_map>
 #include <vector>
 
@@ -128,7 +130,7 @@ extern "C" int nsr_ctx_destroy(nsr_ctx* ctx) {
 extern "C" int nsr_set_option(const char* name, int value) {
     if (!strcmp(name, "hadamard")) { nsr_use_hadamard = value ? 1 : 0; return 0; }
     if (!strcmp(name, "prefetch")) { nsr_prefetch = value ? 1 : 0; return 0; }
-    if (!strcmp(name, "umma_pair")) { nsr_umma_pair = value ? 1 : 0; return 0; }
+    if (!strcmp(name, "umma_pair")) { nsr_umma_pair = value < 0 ? -1 : (value ? 1 : 0); return 0; }
     if (!strcmp(name, "umma_dynamic")) { nsr_umma_dynamic = value ? 1 : 0; return 0; }
     if (!strcmp(name, "split_k")) { nsr_split_k = value ? 1 : 0; return 0; }
     if (!strcmp(name, "adaptive_min_cells")) { nsr_adaptive_min_cells = value < 0 ? 0 : value; return 0; }
@@ -147,6 +149,72 @@ extern "C" int nsr_set_option(const char* name, int value) {
     }
     nsr_set_error("nsr_set_option: unknown option %s", name);
     return 2;
+}
+
+// Pair tiles for the cta_group::2 kernel: entries (row block of CTA 0, row block of CTA 1 or -1, column block).
+// Tiles of one column are paired in the order they arrive, so an entry's rows usually are adjacent blocks.  A
+// column with an odd number of tiles leaves one CTA of a pair idle; with `symmetric` (co-expression of one
+// operand with itself: tile (j, i) holds the same sums as (i, j), and the epilogue writes both triangles) the
+// next column with an odd count gives up its tile (lo, hi) as the transposed tile (hi, lo) of the column lo,
+// which makes both counts even: 20,000 genes (157 block columns, 79 of them odd) leave one half-tile idle
+// instead of 79.  Entries keep the order in which the caller's list first reaches them (it carries the
+// L2-locality plan).  Returns the number of entries written to out (room for 3 * n_tiles).
+extern "C" int64_t nsr_pair_tiles(const int32_t* tiles, int64_t n_tiles, int symmetric, int32_t* out) {
+    struct Col { int32_t c; int64_t live; std::vector<int32_t> rows; std::vector<int64_t> pos; };
+    std::vector<Col> cols;
+    std::unordered_map<int32_t, size_t> col_of;
+    std::unordered_map<uint64_t, size_t> slot_of;            // (column, row) -> index in the column's rows
+    for (int64_t t = 0; t < n_tiles; ++t) {
+        const int32_t r = tiles[2 * t], c = tiles[2 * t + 1];
+        auto it = col_of.find(c);
+        if (it == col_of.end()) { it = col_of.emplace(c, cols.size()).first; cols.push_back(Col{c, 0, {}, {}}); }
+        Col& col = cols[it->second];
+        slot_of.emplace(((uint64_t)(uint32_t)c << 32) | (uint32_t)r, col.rows.size());
+        col.rows.push_back(r);
+        col.pos.push_back(t);
+        ++col.live;
+    }
+    if (symmetric) {
+        int64_t pending = -1;                                 // earlier column with an odd count
+        for (size_t k = 0; k < cols.size(); ++k) {
+            if (cols[k].live % 2 == 0) continue;
+            if (pending >= 0) {
+                Col& a = cols[(size_t)pending];
+                Col& b = cols[k];
+                Col& lo = a.c < b.c ? a : b;
+                Col& hi = a.c < b.c ? b : a;
+                auto it = slot_of.find(((uint64_t)(uint32_t)hi.c << 32) | (uint32_t)lo.c);
+                if (it != slot_of.end()) {                    // tile (lo, hi) exists: move it as (hi, lo)
+                    lo.rows.push_back(hi.c);
+                    lo.pos.push_back(hi.pos[it->second]);
+                    ++lo.live;
+                    hi.rows[it->second] = -1;
+                    --hi.live;
+                    slot_of.erase(it);
+                    pending = -1;
+                    continue;
+                }
+            }
+            pending = (int64_t)k;
+        }
+    }
+    std::vector<std::pair<int64_t, std::array<int32_t, 3>>> ent;
+    ent.reserve((size_t)n_tiles);
+    for (const Col& col : cols) {
+        int64_t first = -1;
+        int32_t r0 = -1;
+        for (size_t q = 0; q < col.rows.size(); ++q) {
+            if (col.rows[q] < 0) continue;
+            if (r0 < 0) { r0 = col.rows[q]; first = col.pos[q]; continue; }
+            ent.push_back({std::min(first, col.pos[q]), {r0, col.rows[q], col.c}});
+            r0 = -1;
+        }
+        if (r0 >= 0) ent.push_back({first, {r0, -1, col.c}});
+    }
+    std::stable_sort(ent.begin(), ent.end(), [](const auto& x, const auto& y) { return x.first < y.first; });
+    for (size_t e = 0; e < ent.size(); ++e)
+        for (int q = 0; q < 3; ++q) out[3 * e + q] = ent[e].second[q];
+    return (int64_t)ent.size();
 }
 
 // Shared implementation of nsr_contract / nsr_contract_ab / nsr_contract_segments.
@@ -208,32 +276,25 @@ static int contract_impl(nsr_ctx* ctx, uintptr_t stream, int engine, int mode, c
     }
     cudaStream_t st = (cudaStream_t)stream;
     NSR_CHECK(cudaSetDevice(ctx->device));
-    // the cta_group::2 kernel works on 256 x 128 pair tiles: fold (tr, tc) into (tr/2, tc, half mask),
-    // keeping first-appearance order (the caller's order carries the L2-locality plan)
-    const bool pair = engine == NSR_ENGINE_UMMA && nsr_umma_pair != 0 && n_segs == 1 && n_slices_a == n_slices_b &&
-                      n_slices_a >= 3;
+    // the cta_group::2 kernel works on pair tiles, two 128-row blocks of A against one block of B (nsr_pair_tiles).
+    // umma_pair < 0 (default): the pair kernel takes single-segment co-expression launches at 3 planes / 8 products,
+    // where it runs the stacked-B schedule (4.5 % faster than the single-CTA kernel at 100k x 20k), unless the
+    // adaptive 6 / 8 product schedule was asked for.
+    const bool pair_ok = engine == NSR_ENGINE_UMMA && n_segs == 1 && n_slices_a == n_slices_b && n_slices_a >= 3;
+    const bool pair_auto = mode == NSR_MODE_COEX && segs[0].info.mode == NSR_MODE_COEX && n_slices_a == 3 && wmax == 5 &&
+                           !(nsr_adaptive_min_cells > 0 && n >= nsr_adaptive_min_cells);
+    const bool pair = pair_ok && (nsr_umma_pair > 0 || (nsr_umma_pair < 0 && pair_auto));
     std::vector<int32_t> folded;
     int64_t n_upload = n_tiles * 2;
     const int32_t* upload = packed.data();
     int64_t n_entries = n_tiles;
     if (pair) {
-        std::unordered_map<uint64_t, int64_t> seen;
-        seen.reserve((size_t)n_tiles * 2);
-        folded.reserve((size_t)n_tiles * 3);
-        for (int64_t t = 0; t < n_tiles; ++t) {
-            const int32_t tr = packed[2 * t], tc = packed[2 * t + 1];
-            const uint64_t key = ((uint64_t)(uint32_t)(tr >> 1) << 32) | (uint32_t)tc;
-            auto it = seen.find(key);
-            if (it == seen.end()) {
-                seen.emplace(key, (int64_t)folded.size() / 3);
-                folded.push_back(tr >> 1);
-                folded.push_back(tc);
-                folded.push_back(1 << (tr & 1));
-            } else {
-                folded[(size_t)it->second * 3 + 2] |= 1 << (tr & 1);
-            }
-        }
-        n_entries = (int64_t)folded.size() / 3;
+        // a transposed tile (j, i) holds the sums of (i, j) bit for bit when both operands are the same planes
+        const SegInfo& s0 = segs[0].info;
+        const int sym = mode == NSR_MODE_COEX && s0.mode == NSR_MODE_COEX && segs[0].slices == a_slices &&
+                        s0.qb == quantum_a && s0.vb == var_a;
+        folded.resize((size_t)n_tiles * 3);
+        n_entries = nsr_pair_tiles(packed.data(), n_tiles, sym, folded.data());
         n_upload = n_entries * 3;
         upload = folded.data();
     }
