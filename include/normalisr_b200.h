@@ -318,9 +318,10 @@ int nsr_de4_solve(nsr_ctx* ctx, uintptr_t stream, double* Gxx, int nx, const dou
 int nsr_sym_pinv(nsr_ctx* ctx, uintptr_t stream, const double* G, int64_t batch, int n, double tol,
                  double* pinv, int32_t* rank);
 
-/* Adaptive digit-product schedule of nsr_contract, opt-in (tcgen05 engine, n_slices = 3,
+/* Adaptive digit-product schedule of nsr_contract, opt-in (tcgen05 engine, one segment, n_slices = 3,
  * n_products = 8, k_chunk = 0, any mode but RAW, n >= option "adaptive_min_cells"; default 0 = off,
- * 8192 or more sensible; pays only when extremely significant pairs are confined to few tiles): every
+ * 8192 or more sensible; an explicit "umma_pair" = 1 takes precedence, see nsr_set_option; pays only when
+ * extremely significant pairs are confined to few tiles): every
  * tile first runs 6 products; a tile holding a pair with r^2 n > 64 is recomputed with all 8 by a
  * second launch whose tile list and count stay on the device.  Unrefined pairs carry |dr| ~
  * 1e-6 / sqrt(n) (random sign) from the two dropped weight-5 products, i.e. a relative error of P
@@ -444,15 +445,36 @@ int nsr_tsv_write(const char* path, char delimiter, const double* data, int64_t 
 int nsr_mtx_shape(const char* path, int64_t* rows, int64_t* cols, int64_t* nnz, int* is_integer);
 int nsr_mtx_read(const char* path, int64_t nnz, int32_t* row, int32_t* col, double* val, int* symmetric, int threads);
 
-/* Test hooks: "hadamard" (0/1, default 1), "umma_pair" (-1 = the cta_group::2 pair kernel for single-segment
- * NSR_MODE_COEX at 3 planes / 8 products, default; 0 = always the single-CTA kernel; 1 = the pair kernel wherever
- * it applies), "umma_kblock" (64 or 128 cells per pipeline stage of the single-CTA
- * kernel, default 128), "umma_dynamic" (1 = tiles claimed from a global counter, default; 0 = static
- * round-robin), "split_k" (1 = launches with fewer than two waves of tiles split the cells into parts - work
- * items (tile, part) over all SMs, partial sums added in a fixed order by a second small kernel; default 1),
- * "adaptive_min_cells" (see nsr_last_refined), "prefetch" (1 = L2 prefetch of the next
- * cell block in the residual pass; measured neutral, default 0), "binnet_keys" (1 = nsr_binnet keeps rows as 2-byte
- * bin keys, four rows per SM, default; 0 = the 8-byte row staged with one bulk copy).  Process-wide. */
+/* Process-wide options, mostly test hooks.  Which kernel nsr_contract runs is decided by the first rule that
+ * applies (nsr_contract_route in csrc/contract_route.h):
+ *   1. the dp4a engine (NSR_ENGINE_SIMT) runs as asked;
+ *   2. the cta_group::2 pair kernel, for one segment with equal plane counts of at least 3, when "umma_pair" is 1,
+ *      or when it is -1 and the call is single-segment NSR_MODE_COEX at 3 planes / 8 products without the adaptive
+ *      schedule (n < "adaptive_min_cells" or that option 0);
+ *   3. the adaptive schedule (see nsr_last_refined), for one segment at 3 planes / 8 products, any mode but RAW,
+ *      k_chunk = 0 (or >= n_pad) and n >= "adaptive_min_cells" > 0;
+ *   4. the split over the cells, when "split_k" is 1, for one segment in NSR_MODE_DE or NSR_MODE_RAW with fewer
+ *      than two waves of tiles (one tile per SM) that would leave more than a quarter of their SM slots idle
+ *      (4 tiles < 3 waves x SMs): work items (tile, part of the cells) over all SMs, partial sums added in a
+ *      fixed order by a second small kernel.  It needs at least two parts, at least as many as the k_chunk
+ *      chunks, and at most 1 GiB of partial-sum slabs; otherwise rule 5;
+ *   5. the single-CTA tcgen05 kernel, once per k_chunk chunk of the cells.
+ * Options:
+ *   "umma_pair"           -1 (default), 0 (never the pair kernel) or 1 (wherever it applies), as above;
+ *   "adaptive_min_cells"  0 = off (default), 8192 or more sensible: rule 3;
+ *   "split_k"             1 (default) / 0: rule 4;
+ *   "umma_dynamic"        1 = tcgen05 kernels claim tiles from a global counter (default), 0 = static round-robin;
+ *   "umma_kblock"         64 or 128 cells per pipeline stage of the single-CTA kernel (default 128; 64 whenever
+ *                         the two operands have more than 6 planes together);
+ *   "umma_stack"          1 = N = 256 MMAs over two stacked B planes in the single-CTA kernel at 128-cell stages
+ *                         (default), 0 = one N = 128 MMA per digit product;
+ *   "epi_warps"           8 (default) or 16 epilogue warps in the single-CTA kernel;
+ *   "epi_sleep_ns"        back-off in ns of the tcgen05 epilogue warps while they wait for a tile (default 500,
+ *                         0 = spin);
+ *   "hadamard"            1 = Walsh-Hadamard mixing in nsr_residualize (default), 0 = off;
+ *   "prefetch"            1 = L2 prefetch of the next cell block in the residual pass; measured neutral, default 0;
+ *   "binnet_keys"         1 = nsr_binnet keeps rows as 2-byte bin keys, four rows per SM (default); 0 = the
+ *                         8-byte row staged with one bulk copy. */
 int nsr_set_option(const char* name, int value);
 
 /* Debug / test helper: reconstruct z' (float64, rows x n_pad) from slices and quantum. */

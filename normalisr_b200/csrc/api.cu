@@ -9,21 +9,13 @@
 
 #include <cuda.h>
 
+#include "contract_route.h"
 #include "epilogue.cuh"
 
 int nsr_launch_contract_simt(cudaStream_t st, const int8_t* a, int64_t rows_alloc_a, int n_slices_a, const int8_t* b,
                              int64_t rows_alloc_b, int n_slices_b, int64_t n_pad, int wmax,
                              const int32_t* tiles_dev, int64_t n_tiles, const ContractParams& ep,
                              int64_t cell_begin, int64_t cell_end);
-int nsr_launch_contract_umma(nsr_ctx* ctx, cudaStream_t st, const int8_t* a, int64_t rows_a,
-                             int64_t rows_alloc_a, int n_slices_a, const NsrSegOperand* segs, int n_segs,
-                             int64_t n_pad, int n_slices_b, int wmax,
-                             const int32_t* tiles_dev, int64_t n_tiles, const ContractParams& ep,
-                             int64_t cell_begin, int64_t cell_end, const int* n_tiles_dev, int n_parts = 1,
-                             double* part_out = nullptr, int64_t part_stride = 0);
-int nsr_launch_contract_finish(cudaStream_t st, const int32_t* tiles_dev, int64_t n_tiles, const ContractParams& ep,
-                               const SegInfo& sg, int n_parts, const double* part, int64_t part_stride);
-int nsr_umma_parts(int64_t cells, int n_slices_a, int n_slices_b, int n_parts);
 extern int nsr_use_hadamard;
 extern int nsr_prefetch;
 extern int nsr_umma_kblock;
@@ -32,7 +24,7 @@ extern int nsr_epi_warps;
 extern int nsr_umma_stack;
 extern int nsr_binnet_keys;
 extern int nsr_umma_dynamic;
-int nsr_split_k = 1;          // 1: few-tile launches split the cells over work items (see contract_impl)
+int nsr_split_k = 1;          // 1: few-tile launches split the cells over work items (nsr_contract_route)
 extern int nsr_epi_sleep_ns;
 
 // Adaptive digit-product schedule, OPT-IN (tcgen05 engine, 3 planes / 8 products, one pass over the
@@ -126,7 +118,7 @@ extern "C" int nsr_ctx_destroy(nsr_ctx* ctx) {
     return 0;
 }
 
-// test hooks: "hadamard" (0/1), "umma_kblock" (64/128)
+// the options and their values: include/normalisr_b200.h
 extern "C" int nsr_set_option(const char* name, int value) {
     if (!strcmp(name, "hadamard")) { nsr_use_hadamard = value ? 1 : 0; return 0; }
     if (!strcmp(name, "prefetch")) { nsr_prefetch = value ? 1 : 0; return 0; }
@@ -217,220 +209,253 @@ extern "C" int64_t nsr_pair_tiles(const int32_t* tiles, int64_t n_tiles, int sym
     return (int64_t)ent.size();
 }
 
-// Shared implementation of nsr_contract / nsr_contract_ab / nsr_contract_segments.
-// tile_stride = 2: host_tiles holds (tile_row, tile_col), one segment; 3: (segment, tile_row, tile_col).
 // tile list: page-locked host memory (read over PCIe, zero-copy) -> device memory
 __global__ void tiles_upload_kernel(int4* __restrict__ dst, const int4* __restrict__ src, int64_t n_vec) {
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_vec; i += (int64_t)gridDim.x * blockDim.x)
         dst[i] = src[i];
 }
 
-static int contract_impl(nsr_ctx* ctx, uintptr_t stream, int engine, int mode, const int8_t* a_slices, int64_t rows_a,
-                         int64_t rows_alloc_a, int n_slices_a, const double* quantum_a, const double* var_a,
-                         const NsrSegOperand* segs, int n_segs, int n_slices_b, int64_t n, int64_t n_pad, int n_products,
-                         const int32_t* host_tiles, int tile_stride, int64_t n_tiles, double dof_a, double* P,
-                         double* out2, int64_t ld, int64_t k_chunk) {
-    NSR_REQUIRE(ctx != nullptr, "nsr_contract: null context");
-    NSR_REQUIRE(engine == NSR_ENGINE_UMMA || engine == NSR_ENGINE_SIMT, "nsr_contract: unknown engine %d", engine);
-    NSR_REQUIRE(n_segs >= 1 && n_segs <= NSR_MAX_SEGMENTS && segs != nullptr, "nsr_contract: %d segments (1..%d)", n_segs,
-                NSR_MAX_SEGMENTS);
-    NSR_REQUIRE(n_segs == 1 || engine == NSR_ENGINE_UMMA, "nsr_contract: segments need the tcgen05 engine");
-    NSR_REQUIRE(rows_a > 0 && n > 0 && n_pad == nsr_padded_cells(n), "nsr_contract: bad shape rows_a=%lld n=%lld n_pad=%lld",
-                (long long)rows_a, (long long)n, (long long)n_pad);
-    const int wmax = nsr_wmax_ab(n_slices_a, n_slices_b, n_products);
-    NSR_REQUIRE(wmax > 0, "nsr_contract: unsupported (n_slices_a=%d, n_slices_b=%d, n_products=%d)", n_slices_a, n_slices_b,
-                n_products);
-    NSR_REQUIRE(out2 != nullptr && quantum_a && a_slices, "nsr_contract: null buffer");
-    NSR_REQUIRE(((uintptr_t)a_slices & 15) == 0, "nsr_contract: slice planes must be 16-byte aligned");
-    bool need_p = false;
-    for (int s = 0; s < n_segs; ++s) {
-        const SegInfo& si = segs[s].info;
+// One nsr_contract / nsr_contract_ab / nsr_contract_segments call.
+// tile_stride = 2: host_tiles holds (tile_row, tile_col), one segment; 3: (segment, tile_row, tile_col).
+struct ContractCall {
+    int engine, mode;
+    const int8_t* a_slices;
+    int64_t rows_a, rows_alloc_a;
+    int n_slices_a;
+    const double* quantum_a;
+    const double* var_a;
+    const NsrSegOperand* segs;
+    int n_segs, n_slices_b;
+    int64_t n, n_pad;
+    int n_products;
+    const int32_t* host_tiles;
+    int tile_stride;
+    int64_t n_tiles;
+    double dof_a;
+    double* P;
+    double* out2;
+    int64_t ld, k_chunk;
+};
+
+// Checks a call's arguments but the tile list; *wmax = the largest digit weight kept, *need_p = P is written.
+static int check_call(const ContractCall& c, int* wmax, bool* need_p) {
+    NSR_REQUIRE(c.engine == NSR_ENGINE_UMMA || c.engine == NSR_ENGINE_SIMT, "nsr_contract: unknown engine %d", c.engine);
+    NSR_REQUIRE(c.n_segs >= 1 && c.n_segs <= NSR_MAX_SEGMENTS && c.segs != nullptr, "nsr_contract: %d segments (1..%d)",
+                c.n_segs, NSR_MAX_SEGMENTS);
+    NSR_REQUIRE(c.n_segs == 1 || c.engine == NSR_ENGINE_UMMA, "nsr_contract: segments need the tcgen05 engine");
+    NSR_REQUIRE(c.rows_a > 0 && c.n > 0 && c.n_pad == nsr_padded_cells(c.n),
+                "nsr_contract: bad shape rows_a=%lld n=%lld n_pad=%lld", (long long)c.rows_a, (long long)c.n,
+                (long long)c.n_pad);
+    *wmax = nsr_wmax_ab(c.n_slices_a, c.n_slices_b, c.n_products);
+    NSR_REQUIRE(*wmax > 0, "nsr_contract: unsupported (n_slices_a=%d, n_slices_b=%d, n_products=%d)", c.n_slices_a,
+                c.n_slices_b, c.n_products);
+    NSR_REQUIRE(c.out2 != nullptr && c.quantum_a && c.a_slices, "nsr_contract: null buffer");
+    NSR_REQUIRE(((uintptr_t)c.a_slices & 15) == 0, "nsr_contract: slice planes must be 16-byte aligned");
+    *need_p = false;
+    for (int s = 0; s < c.n_segs; ++s) {
+        const SegInfo& si = c.segs[s].info;
         NSR_REQUIRE(si.mode == NSR_MODE_COEX || si.mode == NSR_MODE_DE || si.mode == NSR_MODE_RAW ||
                         si.mode == NSR_MODE_COEX_UPPER || si.mode == NSR_MODE_COEX_RECT,
                     "nsr_contract: unknown mode %d", si.mode);
         const bool sym = si.mode == NSR_MODE_COEX || si.mode == NSR_MODE_COEX_UPPER;
-        NSR_REQUIRE(si.rows_b > 0 && si.col0 >= 0 && ld >= si.col0 + si.rows_b && (!sym || rows_a == si.rows_b),
+        NSR_REQUIRE(si.rows_b > 0 && si.col0 >= 0 && c.ld >= si.col0 + si.rows_b && (!sym || c.rows_a == si.rows_b),
                     "nsr_contract: bad segment %d (rows_b=%lld col0=%lld ld=%lld)", s, (long long)si.rows_b,
-                    (long long)si.col0, (long long)ld);
-        NSR_REQUIRE(si.mode != NSR_MODE_COEX || n_segs == 1, "nsr_contract: NSR_MODE_COEX (mirrored) takes one segment");
-        NSR_REQUIRE(segs[s].slices && si.qb && ((uintptr_t)segs[s].slices & 15) == 0, "nsr_contract: segment %d: bad planes", s);
+                    (long long)si.col0, (long long)c.ld);
+        NSR_REQUIRE(si.mode != NSR_MODE_COEX || c.n_segs == 1, "nsr_contract: NSR_MODE_COEX (mirrored) takes one segment");
+        NSR_REQUIRE(c.segs[s].slices && si.qb && ((uintptr_t)c.segs[s].slices & 15) == 0,
+                    "nsr_contract: segment %d: bad planes", s);
         NSR_REQUIRE(si.mode == NSR_MODE_RAW || si.vb != nullptr, "nsr_contract: segment %d: var missing", s);
-        need_p = need_p || si.mode != NSR_MODE_RAW;
+        *need_p = *need_p || si.mode != NSR_MODE_RAW;
     }
-    NSR_REQUIRE(!need_p || (P != nullptr && var_a != nullptr && dof_a > 0.0), "nsr_contract: P / var / dof missing");
-    if (n_tiles == 0) return 0;
-    NSR_REQUIRE(host_tiles != nullptr && n_tiles > 0 && n_tiles < (1ll << 30), "nsr_contract: bad tile list");
-    const int64_t tr_max = (rows_a + NSR_TILE - 1) / NSR_TILE;
-    std::vector<int32_t> packed((size_t)n_tiles * 2);
-    for (int64_t t = 0; t < n_tiles; ++t) {
-        const int32_t sg = tile_stride == 3 ? host_tiles[3 * t] : 0;
-        const int32_t tr = host_tiles[tile_stride * t + tile_stride - 2], tc = host_tiles[tile_stride * t + tile_stride - 1];
-        NSR_REQUIRE(sg >= 0 && sg < n_segs, "nsr_contract: tile %lld: segment %d out of range", (long long)t, sg);
-        const int64_t tc_max = (segs[sg].info.rows_b + NSR_TILE - 1) / NSR_TILE;
+    NSR_REQUIRE(!*need_p || (c.P != nullptr && c.var_a != nullptr && c.dof_a > 0.0), "nsr_contract: P / var / dof missing");
+    return 0;
+}
+
+// Checks the call's tile list and packs it as (tile_row, tile_col | segment << 24).
+static int pack_tiles(const ContractCall& c, std::vector<int32_t>& packed) {
+    NSR_REQUIRE(c.host_tiles != nullptr && c.n_tiles > 0 && c.n_tiles < (1ll << 30), "nsr_contract: bad tile list");
+    const int64_t tr_max = (c.rows_a + NSR_TILE - 1) / NSR_TILE;
+    const int ts = c.tile_stride;
+    packed.resize((size_t)c.n_tiles * 2);
+    for (int64_t t = 0; t < c.n_tiles; ++t) {
+        const int32_t sg = ts == 3 ? c.host_tiles[3 * t] : 0;
+        const int32_t tr = c.host_tiles[ts * t + ts - 2], tc = c.host_tiles[ts * t + ts - 1];
+        NSR_REQUIRE(sg >= 0 && sg < c.n_segs, "nsr_contract: tile %lld: segment %d out of range", (long long)t, sg);
+        const int64_t tc_max = (c.segs[sg].info.rows_b + NSR_TILE - 1) / NSR_TILE;
         NSR_REQUIRE(tr >= 0 && tr < tr_max && tc >= 0 && tc < tc_max && tc < (1 << 24),
                     "nsr_contract: tile %lld = (%d,%d) out of range", (long long)t, tr, tc);
-        const int m = segs[sg].info.mode;
+        const int m = c.segs[sg].info.mode;
         NSR_REQUIRE(!(m == NSR_MODE_COEX || m == NSR_MODE_COEX_UPPER) || tr <= tc, "nsr_contract: COEX tiles must have row <= col");
         packed[2 * t] = tr;
         packed[2 * t + 1] = tc | (sg << 24);
     }
-    cudaStream_t st = (cudaStream_t)stream;
-    NSR_CHECK(cudaSetDevice(ctx->device));
-    // the cta_group::2 kernel works on pair tiles, two 128-row blocks of A against one block of B (nsr_pair_tiles).
-    // umma_pair < 0 (default): the pair kernel takes single-segment co-expression launches at 3 planes / 8 products,
-    // where it runs the stacked-B schedule (4.5 % faster than the single-CTA kernel at 100k x 20k), unless the
-    // adaptive 6 / 8 product schedule was asked for.
-    const bool pair_ok = engine == NSR_ENGINE_UMMA && n_segs == 1 && n_slices_a == n_slices_b && n_slices_a >= 3;
-    const bool pair_auto = mode == NSR_MODE_COEX && segs[0].info.mode == NSR_MODE_COEX && n_slices_a == 3 && wmax == 5 &&
-                           !(nsr_adaptive_min_cells > 0 && n >= nsr_adaptive_min_cells);
-    const bool pair = pair_ok && (nsr_umma_pair > 0 || (nsr_umma_pair < 0 && pair_auto));
-    std::vector<int32_t> folded;
-    int64_t n_upload = n_tiles * 2;
-    const int32_t* upload = packed.data();
-    int64_t n_entries = n_tiles;
-    if (pair) {
-        // a transposed tile (j, i) holds the sums of (i, j) bit for bit when both operands are the same planes
-        const SegInfo& s0 = segs[0].info;
-        const int sym = mode == NSR_MODE_COEX && s0.mode == NSR_MODE_COEX && segs[0].slices == a_slices &&
-                        s0.qb == quantum_a && s0.vb == var_a;
-        folded.resize((size_t)n_tiles * 3);
-        n_entries = nsr_pair_tiles(packed.data(), n_tiles, sym, folded.data());
-        n_upload = n_entries * 3;
-        upload = folded.data();
-    }
-    // The tile list travels through a pinned staging buffer owned by the context (a pageable source
-    // would make cudaMemcpyAsync block the host until the stream drains, and would tie the lifetime of
-    // the vectors above to that staging behaviour); an event guards its reuse by the next call.
-    if ((size_t)n_upload > ctx->tiles_cap) {
+    return 0;
+}
+
+// The epilogue's parameters of a call (segment 0 stands for the B operand).
+static ContractParams contract_params(const ContractCall& c, int wmax, bool need_p) {
+    const SegInfo& s0 = c.segs[0].info;
+    ContractParams ep;
+    ep.mode = c.mode;
+    ep.n_groups = wmax - 1 < c.n_slices_a + c.n_slices_b - 1 ? wmax - 1 : c.n_slices_a + c.n_slices_b - 1;
+    ep.rows_a = c.rows_a; ep.rows_b = s0.rows_b; ep.ld = c.ld;
+    ep.qa = c.quantum_a; ep.va = c.var_a; ep.qb = s0.qb; ep.vb = s0.vb;
+    ep.P = c.P; ep.out2 = c.out2;
+    ep.inv_n = 1.0 / (double)c.n;
+    ep.acc_in = 0;
+    ep.raw_out = 0;
+    ep.refine_r2 = -1.0;
+    ep.need = nullptr;
+    for (int g = 0; g < 4; ++g) ep.group_scale[g] = (g < ep.n_groups) ? ldexp(1.0, 8 * (ep.n_groups - 1 - g)) : 0.0;
+    ep.scale_all = ldexp(1.0, 8 * (c.n_slices_a + c.n_slices_b - 1 - ep.n_groups));
+    ep.pv = nsr_pval_params(need_p ? c.dof_a : 1.0);
+    return ep;
+}
+
+// Puts n int32 of the tile list into ctx->tiles_dev.  The list travels through a pinned staging buffer owned by
+// the context (a pageable source would make cudaMemcpyAsync block the host until the stream drains, and would tie
+// the lifetime of the caller's vector to that staging behaviour); an event guards its reuse by the next call.
+static int stage_tiles(nsr_ctx* ctx, cudaStream_t st, const int32_t* tiles, int64_t n) {
+    if ((size_t)n > ctx->tiles_cap) {
         NSR_CHECK(cudaStreamSynchronize(st));
         if (ctx->tiles_dev) NSR_CHECK(cudaFree(ctx->tiles_dev));
         if (ctx->tiles_pinned) NSR_CHECK(cudaFreeHost(ctx->tiles_pinned));
         ctx->tiles_dev = nullptr;
         ctx->tiles_pinned = nullptr;
         ctx->tiles_cap = 0;
-        NSR_CHECK(cudaMalloc(&ctx->tiles_dev, (size_t)n_upload * sizeof(int32_t) * 2));
-        NSR_CHECK(cudaMallocHost(&ctx->tiles_pinned, (size_t)n_upload * sizeof(int32_t) * 2));
-        ctx->tiles_cap = (size_t)n_upload * 2;
+        NSR_CHECK(cudaMalloc(&ctx->tiles_dev, (size_t)n * sizeof(int32_t) * 2));
+        NSR_CHECK(cudaMallocHost(&ctx->tiles_pinned, (size_t)n * sizeof(int32_t) * 2));
+        ctx->tiles_cap = (size_t)n * 2;
     }
     if (ctx->tiles_event == nullptr) NSR_CHECK(cudaEventCreateWithFlags(&ctx->tiles_event, cudaEventDisableTiming));
     else NSR_CHECK(cudaEventSynchronize(ctx->tiles_event));       // previous upload has left the staging buffer
-    memcpy(ctx->tiles_pinned, upload, (size_t)n_upload * sizeof(int32_t));
+    memcpy(ctx->tiles_pinned, tiles, (size_t)n * sizeof(int32_t));
     // NOT a cudaMemcpyAsync: a host-to-device copy queues on the H2D copy engine, and in the streamed pipelines that
     // engine is busy with the next gigabyte-sized chunk of the expression matrix - the tile list then waits ~22 ms
     // behind it and so does the contraction (measured: every strip's launch started one chunk late, 350 -> 3xx ms
     // end to end at 100k x 20k).  A small kernel reads the page-locked list over PCIe instead.
-    {
-        const int64_t n_vec = (n_upload + 3) / 4;            // the buffers are allocated with twice the room asked for
-        const int blocks = (int)((n_vec + 255) / 256 < 16 ? (n_vec + 255) / 256 : 16);
-        tiles_upload_kernel<<<blocks > 0 ? blocks : 1, 256, 0, st>>>(reinterpret_cast<int4*>(ctx->tiles_dev),
-                                                                    reinterpret_cast<const int4*>(ctx->tiles_pinned), n_vec);
-        NSR_CHECK(cudaGetLastError());
-    }
+    const int64_t n_vec = (n + 3) / 4;                     // the buffers are allocated with twice the room asked for
+    const int blocks = (int)((n_vec + 255) / 256 < 16 ? (n_vec + 255) / 256 : 16);
+    tiles_upload_kernel<<<blocks > 0 ? blocks : 1, 256, 0, st>>>(reinterpret_cast<int4*>(ctx->tiles_dev),
+                                                                reinterpret_cast<const int4*>(ctx->tiles_pinned), n_vec);
+    NSR_CHECK(cudaGetLastError());
     NSR_CHECK(cudaEventRecord(ctx->tiles_event, st));
+    return 0;
+}
 
-    ContractParams ep;
-    ep.mode = mode;
-    ep.n_groups = wmax - 1 < n_slices_a + n_slices_b - 1 ? wmax - 1 : n_slices_a + n_slices_b - 1;
-    ep.rows_a = rows_a; ep.rows_b = segs[0].info.rows_b; ep.ld = ld;
-    ep.qa = quantum_a; ep.va = var_a; ep.qb = segs[0].info.qb; ep.vb = segs[0].info.vb;
-    ep.P = P; ep.out2 = out2;
-    ep.inv_n = 1.0 / (double)n;
-    ep.acc_in = 0;
-    ep.raw_out = 0;
-    ep.refine_r2 = -1.0;
-    ep.need = nullptr;
-    for (int g = 0; g < 4; ++g) ep.group_scale[g] = (g < ep.n_groups) ? ldexp(1.0, 8 * (ep.n_groups - 1 - g)) : 0.0;
-    ep.scale_all = ldexp(1.0, 8 * (n_slices_a + n_slices_b - 1 - ep.n_groups));
-    ep.pv = nsr_pval_params(need_p ? dof_a : 1.0);
-
-    // Cell chunking: int32 accumulators are exact only while no partial sum can overflow; the caller
-    // bounds that (Cauchy-Schwarz on the digit-plane energies) and passes the chunk length.  Chunks
-    // but the last leave the float64 running sum in out2; the last one adds it and finishes.
-    NSR_REQUIRE(k_chunk >= 0 && k_chunk % NSR_KBLOCK == 0, "nsr_contract: k_chunk must be a multiple of %d", NSR_KBLOCK);
-    const int64_t chunk = (k_chunk == 0 || k_chunk >= n_pad) ? n_pad : k_chunk;
-    if (engine == NSR_ENGINE_UMMA && !pair && n_segs == 1 && chunk == n_pad && mode != NSR_MODE_RAW && n_slices_a == 3 &&
-        n_slices_b == 3 && wmax == 5 && nsr_adaptive_min_cells > 0 && n >= nsr_adaptive_min_cells) {
-        // ---- adaptive schedule: 6 products everywhere, 8 where a pair is extremely significant
-        const size_t want = 3 * (size_t)n_tiles + 4;
-        if (want > ctx->refine_cap) {
-            if (ctx->refine_dev) NSR_CHECK(cudaFree(ctx->refine_dev));
-            ctx->refine_dev = nullptr;
-            ctx->refine_cap = 0;
-            NSR_CHECK(cudaMalloc(&ctx->refine_dev, want * 2 * sizeof(int32_t)));
-            ctx->refine_cap = want * 2;
-        }
-        int* need = ctx->refine_dev;
-        int32_t* list = ctx->refine_dev + n_tiles;
-        int* count = ctx->refine_dev + 3 * n_tiles;
-        NSR_CHECK(cudaMemsetAsync(need, 0, (size_t)n_tiles * sizeof(int32_t), st));
-        NSR_CHECK(cudaMemsetAsync(count, 0, sizeof(int32_t), st));
-        ContractParams ep1 = ep;
-        ep1.n_groups = 3;                                             // wmax = 4
-        for (int g = 0; g < 4; ++g) ep1.group_scale[g] = (g < 3) ? ldexp(1.0, 8 * (2 - g)) : 0.0;
-        ep1.scale_all = ldexp(1.0, 8 * (2 * 3 - 4));
-        ep1.refine_r2 = kRefineZ2 / (double)n;
-        ep1.need = need;
-        int rc = nsr_launch_contract_umma(ctx, st, a_slices, rows_a, rows_alloc_a, 3, segs, 1, n_pad, 3, 4, ctx->tiles_dev,
-                                          n_tiles, ep1, 0, n_pad, nullptr);
-        if (rc) return rc;
-        refine_compact_kernel<<<(unsigned)((n_tiles + 255) / 256 < 64 ? (n_tiles + 255) / 256 : 64), 256, 0, st>>>(
-            need, ctx->tiles_dev, (int)n_tiles, list, count);
-        NSR_CHECK(cudaGetLastError());
-        return nsr_launch_contract_umma(ctx, st, a_slices, rows_a, rows_alloc_a, 3, segs, 1, n_pad, 3, 5, list, n_tiles, ep,
-                                        0, n_pad, count);
-    }
-    // Few tiles, many cells (de: a few hundred groupings against every gene; the groupings' own Gram matrix):
-    // with one CTA per tile the last wave of tiles leaves most SMs idle.  Split the cells into parts instead -
-    // work items (tile, part) over all SMs, partial sums into per-part slabs, one small kernel that adds the
-    // slabs in a fixed order and finishes.  The parts also serve as the overflow chunks (each part <= chunk).
-    // Only the rectangular modes: their sums (two different variables, or an exact small-integer operand) stay
-    // below 2^53, so the parts add up exactly and the result is the single-pass one bit for bit; co-expression
-    // keeps its one-pass tiles (self-products of 24-bit values over 1e5 cells exceed 2^53, and its results are
-    // promised to be identical across tilings and GPU counts).
-    // Worth it when the one-CTA-per-tile launch would leave more than a quarter of the machine idle (its last wave):
-    // the second kernel and the slabs cost about as much as a 20 % imbalance on these short launches (measured at
-    // 300 x 10k x 50k cells: 237 tiles = 1.6 waves ran 0.52 ms one-pass, 0.6 ms split; 160 tiles over 1M cells ran
-    // 10.6 ms one-pass, 7.9 ms split).
-    const int64_t waves = (n_tiles + ctx->sm_count - 1) / ctx->sm_count;
-    const bool unbalanced = 4 * n_tiles < 3 * waves * (int64_t)ctx->sm_count;
-    if (engine == NSR_ENGINE_UMMA && !pair && n_segs == 1 && nsr_split_k != 0 && n_tiles < 2 * (int64_t)ctx->sm_count &&
-        unbalanced && (mode == NSR_MODE_DE || mode == NSR_MODE_RAW)) {
-        const int64_t target = 4 * (int64_t)ctx->sm_count;                  // ~4 waves of work items
-        int64_t want = (target + n_tiles - 1) / n_tiles;
-        const int64_t for_overflow = (n_pad + chunk - 1) / chunk;
-        if (want < for_overflow) want = for_overflow;
-        const int64_t max_parts = n_pad / (8 * NSR_KBLOCK) > 0 ? n_pad / (8 * NSR_KBLOCK) : 1;   // >= 1024 cells per part
-        if (want > max_parts && max_parts >= for_overflow) want = max_parts;
-        const int64_t slab = rows_a * ld;                                   // one (rows_a x ld) image of out2 per part
-        const int parts = nsr_umma_parts(n_pad, n_slices_a, n_slices_b, (int)want);
-        if (parts > 1 && parts >= for_overflow && (size_t)parts * (size_t)slab * sizeof(double) <= ((size_t)1 << 30)) {
-            void* scratch = nullptr;
-            if (nsr_scratch(ctx, (size_t)parts * (size_t)slab * sizeof(double), &scratch)) return 1;
-            int rc = nsr_launch_contract_umma(ctx, st, a_slices, rows_a, rows_alloc_a, n_slices_a, segs, 1, n_pad, n_slices_b,
-                                              wmax, ctx->tiles_dev, n_tiles, ep, 0, n_pad, nullptr, parts, (double*)scratch,
-                                              slab);
-            if (rc) return rc;
-            return nsr_launch_contract_finish(st, ctx->tiles_dev, n_tiles, ep, segs[0].info, parts, (const double*)scratch,
-                                              slab);
-        }
-    }
+// Cell chunking: int32 accumulators are exact only while no partial sum can overflow; the caller
+// bounds that (Cauchy-Schwarz on the digit-plane energies) and passes the chunk length.  Chunks
+// but the last leave the float64 running sum in out2; the last one adds it and finishes.
+template <class Launch>
+static int over_chunks(ContractParams ep, int64_t n_pad, int64_t chunk, Launch launch) {
     for (int64_t c0 = 0; c0 < n_pad; c0 += chunk) {
         const int64_t c1 = c0 + chunk < n_pad ? c0 + chunk : n_pad;
         ep.acc_in = c0 > 0;
         ep.raw_out = c1 < n_pad;
-        int rc;
-        if (engine == NSR_ENGINE_SIMT) {
-            rc = nsr_launch_contract_simt(st, a_slices, rows_alloc_a, n_slices_a, segs[0].slices, segs[0].rows_alloc,
-                                          n_slices_b, n_pad, wmax, ctx->tiles_dev, n_tiles, ep, c0, c1);
-            if (rc) {
-                nsr_set_error("nsr_contract: SIMT launch failed: %s", cudaGetErrorString(cudaGetLastError()));
-                return 1;
-            }
-        } else {
-            rc = nsr_launch_contract_umma(ctx, st, a_slices, rows_a, rows_alloc_a, n_slices_a, segs, n_segs, n_pad,
-                                          n_slices_b, wmax, ctx->tiles_dev, pair ? -n_entries : n_tiles, ep, c0, c1, nullptr);
-            if (rc) return rc;
-        }
+        if (int rc = launch(ep, c0, c1)) return rc;
+    }
+    return 0;
+}
+
+// Adaptive schedule: 6 products on every tile of l, then all 8 on the tiles the first phase flagged, whose list
+// and count stay on the device.
+static int contract_adaptive(nsr_ctx* ctx, cudaStream_t st, UmmaLaunch l, const ContractParams& ep, int64_t n) {
+    const int64_t n_tiles = l.n_tiles;
+    const size_t want = 3 * (size_t)n_tiles + 4;
+    if (want > ctx->refine_cap) {
+        if (ctx->refine_dev) NSR_CHECK(cudaFree(ctx->refine_dev));
+        ctx->refine_dev = nullptr;
+        ctx->refine_cap = 0;
+        NSR_CHECK(cudaMalloc(&ctx->refine_dev, want * 2 * sizeof(int32_t)));
+        ctx->refine_cap = want * 2;
+    }
+    int* need = ctx->refine_dev;
+    int32_t* list = ctx->refine_dev + n_tiles;
+    int* count = ctx->refine_dev + 3 * n_tiles;
+    NSR_CHECK(cudaMemsetAsync(need, 0, (size_t)n_tiles * sizeof(int32_t), st));
+    NSR_CHECK(cudaMemsetAsync(count, 0, sizeof(int32_t), st));
+    ContractParams ep1 = ep;
+    ep1.n_groups = 3;                                             // wmax = 4
+    for (int g = 0; g < 4; ++g) ep1.group_scale[g] = (g < 3) ? ldexp(1.0, 8 * (2 - g)) : 0.0;
+    ep1.scale_all = ldexp(1.0, 8 * (2 * 3 - 4));
+    ep1.refine_r2 = kRefineZ2 / (double)n;
+    ep1.need = need;
+    l.wmax = 4;
+    if (int rc = nsr_launch_contract_umma(ctx, st, l, ep1)) return rc;
+    refine_compact_kernel<<<(unsigned)((n_tiles + 255) / 256 < 64 ? (n_tiles + 255) / 256 : 64), 256, 0, st>>>(
+        need, l.tiles, (int)n_tiles, list, count);
+    NSR_CHECK(cudaGetLastError());
+    l.wmax = 5;
+    l.tiles = list;
+    l.n_tiles_dev = count;
+    return nsr_launch_contract_umma(ctx, st, l, ep);
+}
+
+// Split over the cells: each of `parts` parts of the cells stores its partial sums in a slab of its own, then one
+// small kernel adds the slabs in a fixed order and finishes.
+static int contract_split(nsr_ctx* ctx, cudaStream_t st, const UmmaLaunch& l, const ContractParams& ep, int parts,
+                          int64_t slab) {
+    void* scratch = nullptr;
+    if (nsr_scratch(ctx, (size_t)parts * (size_t)slab * sizeof(double), &scratch)) return 1;
+    if (int rc = nsr_launch_contract_umma_splitk(ctx, st, l, ep, parts, (double*)scratch, slab)) return rc;
+    return nsr_launch_contract_finish(st, l.tiles, l.n_tiles, ep, l.segs[0].info, parts, (const double*)scratch, slab);
+}
+
+// Shared implementation of nsr_contract / nsr_contract_ab / nsr_contract_segments: check the call, pack its tile
+// list, route it (nsr_contract_route), stage the list on the device and run the route.
+static int contract_impl(nsr_ctx* ctx, uintptr_t stream, const ContractCall& c) {
+    NSR_REQUIRE(ctx != nullptr, "nsr_contract: null context");
+    int wmax;
+    bool need_p;
+    if (int rc = check_call(c, &wmax, &need_p)) return rc;
+    if (c.n_tiles == 0) return 0;
+    NSR_REQUIRE(c.k_chunk >= 0 && c.k_chunk % NSR_KBLOCK == 0, "nsr_contract: k_chunk must be a multiple of %d", NSR_KBLOCK);
+    std::vector<int32_t> tiles;
+    if (int rc = pack_tiles(c, tiles)) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    NSR_CHECK(cudaSetDevice(ctx->device));
+
+    const NsrSegOperand& s0 = c.segs[0];
+    const int64_t chunk = (c.k_chunk == 0 || c.k_chunk >= c.n_pad) ? c.n_pad : c.k_chunk;
+    const ContractRouteChoice rt = nsr_contract_route({c.engine, c.mode, c.n_segs, s0.info.mode, c.n_slices_a, c.n_slices_b,
+                                                       wmax, c.n, c.n_pad, chunk, c.n_tiles, ctx->sm_count, c.rows_a * c.ld,
+                                                       nsr_umma_pair, nsr_adaptive_min_cells, nsr_split_k, nsr_umma_kblock});
+    int64_t n_entries = c.n_tiles;
+    if (rt.route == ContractRoute::PAIR) {
+        // a transposed tile (j, i) holds the sums of (i, j) bit for bit when both operands are the same planes
+        const int sym = c.mode == NSR_MODE_COEX && s0.info.mode == NSR_MODE_COEX && s0.slices == c.a_slices &&
+                        s0.info.qb == c.quantum_a && s0.info.vb == c.var_a;
+        std::vector<int32_t> entries((size_t)c.n_tiles * 3);
+        n_entries = nsr_pair_tiles(tiles.data(), c.n_tiles, sym, entries.data());
+        entries.resize((size_t)n_entries * 3);
+        tiles.swap(entries);
+    }
+    if (int rc = stage_tiles(ctx, st, tiles.data(), (int64_t)tiles.size())) return rc;
+
+    const ContractParams ep = contract_params(c, wmax, need_p);
+    UmmaLaunch l = {c.a_slices, c.rows_a, c.rows_alloc_a, c.n_slices_a, c.segs, c.n_segs, c.n_slices_b, c.n_pad, wmax,
+                    ctx->tiles_dev, n_entries, nullptr, 0, c.n_pad};
+    switch (rt.route) {
+    case ContractRoute::SIMT:
+        return over_chunks(ep, c.n_pad, chunk, [&](const ContractParams& e, int64_t c0, int64_t c1) {
+            if (nsr_launch_contract_simt(st, c.a_slices, c.rows_alloc_a, c.n_slices_a, s0.slices, s0.rows_alloc,
+                                         c.n_slices_b, c.n_pad, wmax, l.tiles, l.n_tiles, e, c0, c1) == 0)
+                return 0;
+            nsr_set_error("nsr_contract: SIMT launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+            return 1;
+        });
+    case ContractRoute::ONE_PASS:
+    case ContractRoute::PAIR:
+        return over_chunks(ep, c.n_pad, chunk, [&](const ContractParams& e, int64_t c0, int64_t c1) {
+            l.cell_begin = c0;
+            l.cell_end = c1;
+            return rt.route == ContractRoute::PAIR ? nsr_launch_contract_umma2(ctx, st, l, e)
+                                                   : nsr_launch_contract_umma(ctx, st, l, e);
+        });
+    case ContractRoute::ADAPTIVE:
+        return contract_adaptive(ctx, st, l, ep, c.n);
+    case ContractRoute::SPLIT_CELLS:
+        return contract_split(ctx, st, l, ep, rt.parts, c.rows_a * c.ld);
     }
     return 0;
 }
@@ -449,8 +474,8 @@ extern "C" int nsr_contract_ab(nsr_ctx* ctx, uintptr_t stream, int engine, int m
     sg.info.ready = nullptr; sg.info.ready_value = 0; sg.info.done = nullptr;
     const bool mir = mode == NSR_MODE_COEX;          // both triangles of the same matrix
     sg.info.mP = mir ? P : nullptr; sg.info.mO = mir ? out2 : nullptr; sg.info.ldm = ld;
-    return contract_impl(ctx, stream, engine, mode, a_slices, rows_a, rows_alloc_a, n_slices_a, quantum_a, var_a, &sg, 1,
-                         n_slices_b, n, n_pad, n_products, host_tiles, 2, n_tiles, dof_a, P, out2, ld, k_chunk);
+    return contract_impl(ctx, stream, {engine, mode, a_slices, rows_a, rows_alloc_a, n_slices_a, quantum_a, var_a, &sg, 1,
+                                       n_slices_b, n, n_pad, n_products, host_tiles, 2, n_tiles, dof_a, P, out2, ld, k_chunk});
 }
 
 extern "C" int nsr_contract(nsr_ctx* ctx, uintptr_t stream, int engine, int mode,
@@ -485,9 +510,9 @@ extern "C" int nsr_contract_segments(nsr_ctx* ctx, uintptr_t stream, const int8_
                     "nsr_contract_segments: segment %d: bad mirror (ld_mirror=%lld)", s, (long long)in.ld_mirror);
         sg[s].info.mP = in.mirror_P; sg[s].info.mO = in.mirror_out2; sg[s].info.ldm = in.ld_mirror;
     }
-    return contract_impl(ctx, stream, NSR_ENGINE_UMMA, NSR_MODE_COEX_RECT, a_slices, rows_a, rows_alloc_a, n_slices, quantum_a,
-                         var_a, sg, n_segments, n_slices, n, n_pad, n_products, host_tiles, 3, n_tiles, dof_a, P, out2, ld,
-                         k_chunk);
+    return contract_impl(ctx, stream, {NSR_ENGINE_UMMA, NSR_MODE_COEX_RECT, a_slices, rows_a, rows_alloc_a, n_slices,
+                                       quantum_a, var_a, sg, n_segments, n_slices, n, n_pad, n_products, host_tiles, 3,
+                                       n_tiles, dof_a, P, out2, ld, k_chunk});
 }
 
 // Stream-ordered 32-bit flag operations (cuStreamWriteValue32 / cuStreamWaitValue32): no kernel, no SM.

@@ -26,11 +26,14 @@
 #define NSR_SPLITK_TU 0
 #endif
 
+#include "contract_route.h"
 #include "epilogue.cuh"
 
 extern int nsr_epi_warps;
 extern int nsr_umma_stack;
 extern int nsr_umma_dynamic;
+extern int nsr_umma_kblock;
+extern int nsr_epi_sleep_ns;
 
 namespace {
 
@@ -829,6 +832,60 @@ int launch(nsr_ctx* ctx, cudaStream_t st, const CUtensorMap& ma, const SegMaps& 
     return launch_ew<SA, SB, WMAX, KB, 8>(ctx, st, ma, mb, g);
 }
 
+// The UmmaArgs fields every kernel takes alike; segments beyond l.n_segs repeat segment 0.  With dynamic claiming
+// the launch gets a tile counter of its own, zeroed on the stream.
+int fill_args(nsr_ctx* ctx, cudaStream_t st, const UmmaLaunch& l, const ContractParams& ep, int kb, UmmaArgs& g) {
+    g.tiles = l.tiles;
+    g.n_tiles = (int)l.n_tiles;
+    g.num_kb = (int)((l.cell_end - l.cell_begin) / kb);
+    g.kb_begin = (int)(l.cell_begin / kb);
+    g.n_tiles_dev = l.n_tiles_dev;
+    g.epi_sleep_ns = nsr_epi_sleep_ns;
+    g.n_segs = l.n_segs;
+    for (int s = 0; s < kMaxSegs; ++s) g.seg[s] = l.segs[s < l.n_segs ? s : 0].info;
+    g.ep = ep;
+    g.tile_counter = nullptr;
+    if (nsr_umma_dynamic && ctx->tile_counters) {
+        g.tile_counter = ctx->tile_counters + (ctx->launch_seq++ % NSR_TILE_COUNTERS);
+        NSR_CHECK(cudaMemsetAsync(g.tile_counter, 0, sizeof(int), st));
+    }
+    return 0;
+}
+
+// The single-CTA kernel; `split(g)` sets the split-over-cells fields of the arguments (contract_umma_splitk.cu).
+template <class Split>
+int launch_single(nsr_ctx* ctx, cudaStream_t st, const UmmaLaunch& l, const ContractParams& ep, Split split) {
+    if (l.n_segs < 1 || l.n_segs > kMaxSegs) {
+        nsr_set_error("nsr_contract: %d segments (1..%d)", l.n_segs, kMaxSegs);
+        return 2;
+    }
+    const int kb = nsr_umma_kb(l.n_slices_a, l.n_slices_b, nsr_umma_kblock);
+    CUtensorMap ma;
+    SegMaps mb;
+    if (make_map(ctx, &ma, l.a, l.rows_a, l.rows_alloc_a, l.n_pad, l.n_slices_a, kb)) return 1;
+    for (int s = 0; s < l.n_segs; ++s)
+        if (make_map(ctx, &mb.b[s], l.segs[s].slices, l.segs[s].info.rows_b, l.segs[s].rows_alloc, l.n_pad, l.n_slices_b,
+                     kb))
+            return 1;
+    for (int s = l.n_segs; s < kMaxSegs; ++s) mb.b[s] = mb.b[0];
+    UmmaArgs g;
+    if (int rc = fill_args(ctx, st, l, ep, kb, g)) return rc;
+    g.stack_b = (nsr_umma_stack != 0 && kb == 128) ? 1 : 0;
+    split(g);
+    const int sa = l.n_slices_a, sb = l.n_slices_b, wmax = l.wmax;
+    if (sa == 3 && sb == 3 && wmax == 4 && kb == 128) return launch<3, 3, 4, 128>(ctx, st, ma, mb, g);
+    if (sa == 3 && sb == 3 && wmax == 5 && kb == 128) return launch<3, 3, 5, 128>(ctx, st, ma, mb, g);
+    if (sa == 3 && sb == 3 && wmax == 4 && kb == 64) return launch<3, 3, 4, 64>(ctx, st, ma, mb, g);
+    if (sa == 3 && sb == 3 && wmax == 5 && kb == 64) return launch<3, 3, 5, 64>(ctx, st, ma, mb, g);
+    if (sa == 4 && sb == 4 && wmax == 5) return launch<4, 4, 5, 64>(ctx, st, ma, mb, g);
+    if (sa == 1 && sb == 3 && wmax == 4 && kb == 128) return launch<1, 3, 4, 128>(ctx, st, ma, mb, g);
+    if (sa == 1 && sb == 4 && wmax == 5 && kb == 128) return launch<1, 4, 5, 128>(ctx, st, ma, mb, g);
+    if (sa == 1 && sb == 1 && wmax == 2 && kb == 128) return launch<1, 1, 2, 128>(ctx, st, ma, mb, g);
+    nsr_set_error("nsr_contract: unsupported (n_slices_a=%d, n_slices_b=%d, wmax=%d, kblock=%d) for the tcgen05 engine",
+                  sa, sb, wmax, kb);
+    return 2;
+}
+
 #if !NSR_SPLITK_TU
 template <int S, int WMAX>
 int launch2(nsr_ctx* ctx, cudaStream_t st, const CUtensorMap& ma, const CUtensorMap& mb, const UmmaArgs& g) {
@@ -860,8 +917,31 @@ contract_finish_kernel(const int32_t* __restrict__ tiles, ContractParams ep, Seg
                        (ep.qa[i] * sg.qb[j]) * acc, mP, sg.mO, sg.ldm);
     }
 }
+#endif  // !NSR_SPLITK_TU
 
 }  // namespace
+
+#if NSR_SPLITK_TU
+int nsr_launch_contract_umma_splitk(nsr_ctx* ctx, cudaStream_t st, const UmmaLaunch& l, const ContractParams& ep,
+                                    int n_parts, double* part_out, int64_t part_stride) {
+    if (n_parts < 2 || part_out == nullptr) {
+        nsr_set_error("nsr_contract: the split-over-cells launch takes at least two parts");
+        return 2;
+    }
+    return launch_single(ctx, st, l, ep, [&](UmmaArgs& g) {
+        g.kb_per_part = (g.num_kb + n_parts - 1) / n_parts;
+        g.n_parts = (g.num_kb + g.kb_per_part - 1) / g.kb_per_part;      // no empty part
+        g.part_out = part_out;
+        g.part_stride = part_stride;
+    });
+}
+#else
+int nsr_umma_stack = 1;      // test hook: stacked-B N = 256 MMAs in the single-CTA kernel
+int nsr_epi_warps = 8;       // test hook: epilogue warps of the single-CTA kernel (8 or 16)
+int nsr_umma_pair = -1;      // -1: cta_group::2 kernel for single-segment co-expression at 3 planes / 8 products (default), 0: single-CTA kernel, 1: pair kernel wherever it applies
+int nsr_epi_sleep_ns = 500;  // test hook: epilogue wait back-off
+int nsr_umma_kblock = 128;   // test hook (nsr_set_option): 128 -> SWIZZLE_128B stages, 64 -> SWIZZLE_64B
+int nsr_umma_dynamic = 1;    // 1: tiles claimed from a global counter, 0: static round-robin
 
 int nsr_launch_contract_finish(cudaStream_t st, const int32_t* tiles_dev, int64_t n_tiles, const ContractParams& ep,
                                const SegInfo& sg, int n_parts, const double* part, int64_t part_stride) {
@@ -870,136 +950,29 @@ int nsr_launch_contract_finish(cudaStream_t st, const int32_t* tiles_dev, int64_
     return 0;
 }
 
-extern int nsr_umma_kblock;
-// number of parts the kernel will really use for a request of n_parts over `cells` cells
-int nsr_umma_parts(int64_t cells, int n_slices_a, int n_slices_b, int n_parts) {
-    const int kb = (n_slices_a + n_slices_b > 6) ? 64 : nsr_umma_kblock;
-    const int num_kb = (int)(cells / kb);
-    if (n_parts <= 1 || num_kb < 1) return 1;
-    const int per = (num_kb + n_parts - 1) / n_parts;
-    return (num_kb + per - 1) / per;
+int nsr_launch_contract_umma(nsr_ctx* ctx, cudaStream_t st, const UmmaLaunch& l, const ContractParams& ep) {
+    return launch_single(ctx, st, l, ep, [](UmmaArgs&) {});
 }
 
-int nsr_launch_contract_umma_splitk(nsr_ctx* ctx, cudaStream_t st, const int8_t* a, int64_t rows_a,
-                                    int64_t rows_alloc_a, int n_slices_a, const NsrSegOperand* segs, int n_segs,
-                                    int64_t n_pad, int n_slices_b, int wmax,
-                                    const int32_t* tiles_dev, int64_t n_tiles, const ContractParams& ep,
-                                    int64_t cell_begin, int64_t cell_end, const int* n_tiles_dev, int n_parts,
-                                    double* part_out, int64_t part_stride);
-
-int nsr_umma_stack = 1;      // test hook: stacked-B N = 256 MMAs in the single-CTA kernel
-int nsr_epi_warps = 8;       // test hook: epilogue warps of the single-CTA kernel (8 or 16)
-int nsr_umma_pair = -1;      // -1: cta_group::2 kernel for single-segment co-expression at 3 planes / 8 products (default), 0: single-CTA kernel, 1: pair kernel wherever it applies
-int nsr_epi_sleep_ns = 500;  // test hook: epilogue wait back-off
-int nsr_umma_kblock = 128;   // test hook (nsr_set_option): 128 -> SWIZZLE_128B stages, 64 -> SWIZZLE_64B
-int nsr_umma_dynamic = 1;    // 1: tiles claimed from a global counter, 0: static round-robin (single-CTA kernel)
-
-#else   // NSR_SPLITK_TU
-}  // namespace
-extern int nsr_umma_kblock;
-extern int nsr_epi_sleep_ns;
-#endif
-
-#if NSR_SPLITK_TU
-int nsr_launch_contract_umma_splitk(nsr_ctx* ctx, cudaStream_t st, const int8_t* a, int64_t rows_a,
-                                    int64_t rows_alloc_a, int n_slices_a, const NsrSegOperand* segs, int n_segs,
-                                    int64_t n_pad, int n_slices_b, int wmax,
-                                    const int32_t* tiles_dev, int64_t n_tiles, const ContractParams& ep,
-                                    int64_t cell_begin, int64_t cell_end, const int* n_tiles_dev, int n_parts,
-                                    double* part_out, int64_t part_stride) {
-    if (n_tiles < 0 || n_parts < 2 || part_out == nullptr) {
-        nsr_set_error("nsr_contract: the split-over-cells launch takes a plain tile list and at least two parts");
+// l.tiles: pair-tile entries (row block of CTA 0, row block of CTA 1 or -1, column block), l.n_tiles of them
+int nsr_launch_contract_umma2(nsr_ctx* ctx, cudaStream_t st, const UmmaLaunch& l, const ContractParams& ep) {
+    if (l.n_segs != 1 || l.n_slices_a != l.n_slices_b) {
+        nsr_set_error("nsr_contract: the cta_group::2 engine takes one segment and equal plane counts");
         return 2;
     }
-#else
-int nsr_launch_contract_umma(nsr_ctx* ctx, cudaStream_t st, const int8_t* a, int64_t rows_a,
-                             int64_t rows_alloc_a, int n_slices_a, const NsrSegOperand* segs, int n_segs,
-                             int64_t n_pad, int n_slices_b, int wmax,
-                             const int32_t* tiles_dev, int64_t n_tiles, const ContractParams& ep,
-                             int64_t cell_begin, int64_t cell_end, const int* n_tiles_dev, int n_parts,
-                             double* part_out, int64_t part_stride) {
-    if (n_parts > 1 && part_out != nullptr)
-        return nsr_launch_contract_umma_splitk(ctx, st, a, rows_a, rows_alloc_a, n_slices_a, segs, n_segs, n_pad, n_slices_b,
-                                               wmax, tiles_dev, n_tiles, ep, cell_begin, cell_end, n_tiles_dev, n_parts,
-                                               part_out, part_stride);
-    if (n_tiles < 0) {
-        // pair-tile list (row block, row block or -1, column block), -n_tiles entries: cta_group::2 kernel
-        if (n_segs != 1 || n_slices_a != n_slices_b) {
-            nsr_set_error("nsr_contract: the cta_group::2 engine takes one segment and equal plane counts");
-            return 2;
-        }
-        const int n_slices = n_slices_a;
-        CUtensorMap ma, mb;
-        if (make_map(ctx, &ma, a, rows_a, rows_alloc_a, n_pad, n_slices, 128, NSR_TILE)) return 1;
-        if (make_map(ctx, &mb, segs[0].slices, segs[0].info.rows_b, segs[0].rows_alloc, n_pad, n_slices, 128, NSR_TILE / 2)) return 1;
-        UmmaArgs g;
-        g.tiles = tiles_dev;
-        g.n_tiles = (int)(-n_tiles);
-        g.num_kb = (int)((cell_end - cell_begin) / 128);
-        g.kb_begin = (int)(cell_begin / 128);
-        g.stack_b = 0;
-        g.tile_counter = nullptr;
-        if (nsr_umma_dynamic && ctx->tile_counters) {
-            g.tile_counter = ctx->tile_counters + (ctx->launch_seq++ % NSR_TILE_COUNTERS);
-            NSR_CHECK(cudaMemsetAsync(g.tile_counter, 0, sizeof(int), st));
-        }
-        g.n_tiles_dev = nullptr;
-        g.epi_sleep_ns = nsr_epi_sleep_ns;
-        g.n_segs = 1;
-        g.seg[0] = segs[0].info;
-        g.ep = ep;
-        if (n_slices == 3 && wmax == 4) return launch2<3, 4>(ctx, st, ma, mb, g);
-        if (n_slices == 3 && wmax == 5) return launch2<3, 5>(ctx, st, ma, mb, g);
-        if (n_slices == 4 && wmax == 5) return launch2<4, 5>(ctx, st, ma, mb, g);
-        nsr_set_error("nsr_contract: unsupported (n_slices=%d, wmax=%d) for the tcgen05 pair engine", n_slices, wmax);
-        return 2;
-    }
-#endif
-    if (n_segs < 1 || n_segs > kMaxSegs) {
-        nsr_set_error("nsr_contract: %d segments (1..%d)", n_segs, kMaxSegs);
-        return 2;
-    }
-    // two stages of (SA + SB) planes x 128 rows x KB cells must fit the operand ring
-    const int kb = (n_slices_a + n_slices_b > 6) ? 64 : nsr_umma_kblock;
-    CUtensorMap ma;
-    SegMaps mb;
-    if (make_map(ctx, &ma, a, rows_a, rows_alloc_a, n_pad, n_slices_a, kb)) return 1;
+    const int n_slices = l.n_slices_a;
+    CUtensorMap ma, mb;
+    if (make_map(ctx, &ma, l.a, l.rows_a, l.rows_alloc_a, l.n_pad, n_slices, 128, NSR_TILE)) return 1;
+    if (make_map(ctx, &mb, l.segs[0].slices, l.segs[0].info.rows_b, l.segs[0].rows_alloc, l.n_pad, n_slices, 128,
+                 NSR_TILE / 2))
+        return 1;
     UmmaArgs g;
-    for (int s = 0; s < n_segs; ++s) {
-        if (make_map(ctx, &mb.b[s], segs[s].slices, segs[s].info.rows_b, segs[s].rows_alloc, n_pad, n_slices_b, kb)) return 1;
-        g.seg[s] = segs[s].info;
-    }
-    for (int s = n_segs; s < kMaxSegs; ++s) { mb.b[s] = mb.b[0]; g.seg[s] = segs[0].info; }
-    g.n_segs = n_segs;
-    g.tiles = tiles_dev;
-    g.n_tiles = (int)n_tiles;
-    g.num_kb = (int)((cell_end - cell_begin) / kb);
-    g.kb_begin = (int)(cell_begin / kb);
-#if NSR_SPLITK_TU
-    g.kb_per_part = (g.num_kb + n_parts - 1) / n_parts;
-    g.n_parts = (g.num_kb + g.kb_per_part - 1) / g.kb_per_part;      // no empty part
-    g.part_out = part_out;
-    g.part_stride = part_stride;
-#endif
-    g.stack_b = (nsr_umma_stack != 0 && kb == 128) ? 1 : 0;
-    g.tile_counter = nullptr;
-    g.n_tiles_dev = n_tiles_dev;
-    if (nsr_umma_dynamic && ctx->tile_counters) {
-        g.tile_counter = ctx->tile_counters + (ctx->launch_seq++ % NSR_TILE_COUNTERS);
-        NSR_CHECK(cudaMemsetAsync(g.tile_counter, 0, sizeof(int), st));
-    }
-    g.epi_sleep_ns = nsr_epi_sleep_ns;
-    g.ep = ep;
-    const int sa = n_slices_a, sb = n_slices_b;
-    if (sa == 3 && sb == 3 && wmax == 4 && kb == 128) return launch<3, 3, 4, 128>(ctx, st, ma, mb, g);
-    if (sa == 3 && sb == 3 && wmax == 5 && kb == 128) return launch<3, 3, 5, 128>(ctx, st, ma, mb, g);
-    if (sa == 3 && sb == 3 && wmax == 4 && kb == 64) return launch<3, 3, 4, 64>(ctx, st, ma, mb, g);
-    if (sa == 3 && sb == 3 && wmax == 5 && kb == 64) return launch<3, 3, 5, 64>(ctx, st, ma, mb, g);
-    if (sa == 4 && sb == 4 && wmax == 5) return launch<4, 4, 5, 64>(ctx, st, ma, mb, g);
-    if (sa == 1 && sb == 3 && wmax == 4 && kb == 128) return launch<1, 3, 4, 128>(ctx, st, ma, mb, g);
-    if (sa == 1 && sb == 4 && wmax == 5 && kb == 128) return launch<1, 4, 5, 128>(ctx, st, ma, mb, g);
-    if (sa == 1 && sb == 1 && wmax == 2 && kb == 128) return launch<1, 1, 2, 128>(ctx, st, ma, mb, g);
-    nsr_set_error("nsr_contract: unsupported (n_slices_a=%d, n_slices_b=%d, wmax=%d, kblock=%d) for the tcgen05 engine",
-                  sa, sb, wmax, kb);
+    if (int rc = fill_args(ctx, st, l, ep, 128, g)) return rc;
+    g.stack_b = 0;
+    if (n_slices == 3 && l.wmax == 4) return launch2<3, 4>(ctx, st, ma, mb, g);
+    if (n_slices == 3 && l.wmax == 5) return launch2<3, 5>(ctx, st, ma, mb, g);
+    if (n_slices == 4 && l.wmax == 5) return launch2<4, 5>(ctx, st, ma, mb, g);
+    nsr_set_error("nsr_contract: unsupported (n_slices=%d, wmax=%d) for the tcgen05 pair engine", n_slices, l.wmax);
     return 2;
 }
+#endif

@@ -54,6 +54,33 @@ struct NsrSegOperand {
     SegInfo info;
 };
 
+// One tcgen05 contraction launch as the host describes it: the A operand, the B segments, the device tile list
+// and the cell range [cell_begin, cell_end) of this launch.
+struct UmmaLaunch {
+    const int8_t* a;
+    int64_t rows_a, rows_alloc_a;
+    int n_slices_a;
+    const NsrSegOperand* segs;
+    int n_segs;
+    int n_slices_b;
+    int64_t n_pad;
+    int wmax;
+    const int32_t* tiles;        // (tile_row, tile_col | segment << 24); pair kernel: nsr_pair_tiles entries
+    int64_t n_tiles;             // entries of `tiles`
+    const int* n_tiles_dev;      // if set, the count is read on the device (adaptive second phase), else nullptr
+    int64_t cell_begin, cell_end;
+};
+
+// contract_umma.cu: the single-CTA kernel, the cta_group::2 pair kernel (one segment, equal plane counts) and, from
+// contract_umma_splitk.cu, the single-CTA kernel split over the cells into n_parts parts whose unscaled sums go to
+// slabs of part_stride doubles at part_out; nsr_launch_contract_finish adds those slabs and finishes.
+int nsr_launch_contract_umma(nsr_ctx* ctx, cudaStream_t st, const UmmaLaunch& l, const ContractParams& ep);
+int nsr_launch_contract_umma2(nsr_ctx* ctx, cudaStream_t st, const UmmaLaunch& l, const ContractParams& ep);
+int nsr_launch_contract_umma_splitk(nsr_ctx* ctx, cudaStream_t st, const UmmaLaunch& l, const ContractParams& ep,
+                                    int n_parts, double* part_out, int64_t part_stride);
+int nsr_launch_contract_finish(cudaStream_t st, const int32_t* tiles_dev, int64_t n_tiles, const ContractParams& ep,
+                               const SegInfo& sg, int n_parts, const double* part, int64_t part_stride);
+
 // From sum = sum_k res_i res_j over ALL cells to the stored statistics of one output element (i = row in A,
 // j = row in B); with `mP` the transposed element is written too (COEX, i != j tile: the other triangle of the
 // same matrix; multi-GPU block pairs: the mirrored block).  Returns true when the element asks for the

@@ -453,13 +453,16 @@ def test_coex_adaptive_against_oracle():
 
 
 def test_dynamic_and_static_tile_schedulers_agree():
-    """The tcgen05 kernel claims tiles from a global counter by default; the static round-robin
-    order gives the same bits (few tiles, many tiles, and a tile count below the SM count)."""
+    """The single-CTA tcgen05 kernel (``umma_pair=0``: co-expression at the default preset would take the
+    pair kernel, whose claiming test_contract_pair.py covers) claims tiles from a global counter by default;
+    the static round-robin order gives the same bits (few tiles, many tiles, and a tile count below the SM
+    count)."""
     for rows, n in ((300, 700), (2500, 2048), (5000, 256)):
         ctx, p, A, rank, prods = _sliced(rows, n)
         dof = (n - 1 - rank) / 2
         outs = []
         try:
+            engine.set_option("umma_pair", 0)
             for dyn in (1, 0, 1):
                 engine.set_option("umma_dynamic", dyn)
                 P = torch.zeros((rows, rows), dtype=torch.float64, device="cuda")
@@ -468,6 +471,7 @@ def test_dynamic_and_static_tile_schedulers_agree():
                 outs.append((P, D))
         finally:
             engine.set_option("umma_dynamic", 1)
+            engine.set_option("umma_pair", -1)
         torch.cuda.synchronize()
         for P, D in outs[1:]:
             assert torch.equal(P, outs[0][0]) and torch.equal(D, outs[0][1])
