@@ -405,9 +405,30 @@ int nsr_binnet(nsr_ctx* ctx, uintptr_t stream, const double* P, int64_t rows, in
                int64_t ld, int64_t diag0, double qcut, uint8_t* net, int64_t ld_net,
                unsigned long long* stats);
 
-/* Strided device<->host copy on `stream` (cudaMemcpy2DAsync): lets the host layer return
- * finished blocks of P / dot while later tiles are still being computed.  kind: 0 = device to
- * host, 1 = host to device.  Pitches and width in bytes. */
+/* First half of the sparse (CSR) network: the row procedure of nsr_binnet (same kernels, same
+ * "binnet_keys" choice, same arguments and stats), but instead of the uint8 row it writes, per row i,
+ * the threshold thr[i] (double; -1 when the row has no edge) and the edge count count[i] (int64).
+ * Entry (i, j) is an edge iff j != i + diag0 and P[i][j] <= thr[i]: exactly the entries nsr_binnet sets. */
+int nsr_binnet_count(nsr_ctx* ctx, uintptr_t stream, const double* P, int64_t rows, int64_t cols,
+                     int64_t ld, int64_t diag0, double qcut, double* thr, int64_t* count,
+                     unsigned long long* stats);
+
+/* Second half: CSR compaction.  One CTA per row re-reads the row and writes the column indices of its
+ * edges (by the rule above, given thr from nsr_binnet_count) in ascending order into
+ * indices[indptr[i] .. indptr[i+1]), as int32 (index_bytes = 4) or int64 (8).  indptr: rows + 1 int64
+ * row pointers (the exclusive prefix sum of count; indptr[0] need not be 0).  With p_out / d_out given
+ * (both or neither), the same pass stores P[i][j] and D[i][j] (D: rows x cols, leading dimension ld_d)
+ * beside every index.  A row whose number of edges differs from its indptr range writes nothing past
+ * that range and adds 1 to *err (device uint64), which the caller turns into an error. */
+int nsr_binnet_csr_fill(nsr_ctx* ctx, uintptr_t stream, const double* P, int64_t rows, int64_t cols,
+                        int64_t ld, int64_t diag0, const double* thr, const int64_t* indptr,
+                        void* indices, int index_bytes, const double* D, int64_t ld_d, double* p_out,
+                        double* d_out, unsigned long long* err);
+
+/* Strided copy on `stream` (cudaMemcpy2DAsync): lets the host layer return finished blocks of
+ * P / dot while later tiles are still being computed.  kind: 0 = device to host, 1 = host to
+ * device, 2 = device to device (also between two GPUs of the process with peer access: the
+ * multi-GPU coexnet gathers complete rows of P with it).  Pitches and width in bytes. */
 int nsr_copy2d(nsr_ctx* ctx, uintptr_t stream, void* dst, int64_t dst_pitch, const void* src,
                int64_t src_pitch, int64_t width_bytes, int64_t height, int kind);
 
@@ -473,8 +494,8 @@ int nsr_mtx_read(const char* path, int64_t nnz, int32_t* row, int32_t* col, doub
  *                         0 = spin);
  *   "hadamard"            1 = Walsh-Hadamard mixing in nsr_residualize (default), 0 = off;
  *   "prefetch"            1 = L2 prefetch of the next cell block in the residual pass; measured neutral, default 0;
- *   "binnet_keys"         1 = nsr_binnet keeps rows as 2-byte bin keys, four rows per SM (default); 0 = the
- *                         8-byte row staged with one bulk copy. */
+ *   "binnet_keys"         1 = nsr_binnet and nsr_binnet_count keep rows as 2-byte bin keys, four rows per SM
+ *                         (default); 0 = the 8-byte row staged with one bulk copy. */
 int nsr_set_option(const char* name, int value);
 
 /* Debug / test helper: reconstruct z' (float64, rows x n_pad) from slices and quantum. */

@@ -65,6 +65,9 @@ _SIGNATURES = {
     "nsr_copy_peer": (c_int, [c_vp, c_up, c_vp, c_vp, c_int, c_i64]),
     "nsr_unslice": (c_int, [c_vp, c_up, c_vp, c_i64, c_i64, c_i64, c_int, c_vp, c_vp]),
     "nsr_binnet": (c_int, [c_vp, c_up, c_vp, c_i64, c_i64, c_i64, c_i64, c_dbl, c_vp, c_i64, c_vp]),
+    "nsr_binnet_count": (c_int, [c_vp, c_up, c_vp, c_i64, c_i64, c_i64, c_i64, c_dbl, c_vp, c_vp, c_vp]),
+    "nsr_binnet_csr_fill": (c_int, [c_vp, c_up, c_vp, c_i64, c_i64, c_i64, c_i64, c_vp, c_vp, c_vp, c_int, c_vp, c_i64,
+                                    c_vp, c_vp, c_vp]),
     "nsr_project_coef": (c_int, [c_vp, c_up, c_vp, c_i64, c_i64, c_i64, c_vp, c_int, c_i64, c_vp, c_vp]),
     "nsr_group_stats": (c_int, [c_vp, c_up, c_vp, c_i64, c_i64, c_vp, c_int, c_i64, c_vp, c_int, c_vp]),
     "nsr_normvar_width": (c_int, [c_int]),

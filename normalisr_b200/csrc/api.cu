@@ -546,15 +546,41 @@ extern "C" int nsr_last_refined(nsr_ctx* ctx, uintptr_t stream, int64_t n_tiles,
     return 0;
 }
 
+namespace {
+// lets the current device (ctx->device) reach `other`'s memory directly (NVLink / PCIe peer path); where it
+// cannot, the driver stages peer copies through the host
+int enable_peer(nsr_ctx* ctx, int other) {
+    if (other == ctx->device) return 0;
+    int can = 0;
+    NSR_CHECK(cudaDeviceCanAccessPeer(&can, ctx->device, other));
+    if (can) {
+        cudaError_t e = cudaDeviceEnablePeerAccess(other, 0);
+        if (e == cudaErrorPeerAccessAlreadyEnabled) (void)cudaGetLastError();
+        else NSR_CHECK(e);
+    }
+    return 0;
+}
+}  // namespace
+
 extern "C" int nsr_copy2d(nsr_ctx* ctx, uintptr_t stream, void* dst, int64_t dst_pitch, const void* src,
                           int64_t src_pitch, int64_t width_bytes, int64_t height, int kind) {
     NSR_REQUIRE(ctx != nullptr && dst && src && width_bytes >= 0 && height >= 0 && dst_pitch >= width_bytes &&
-                    src_pitch >= width_bytes && (kind == 0 || kind == 1),
+                    src_pitch >= width_bytes && kind >= 0 && kind <= 2,
                 "nsr_copy2d: bad arguments");
     if (width_bytes == 0 || height == 0) return 0;
     NSR_CHECK(cudaSetDevice(ctx->device));
+    cudaMemcpyKind how = kind == 0 ? cudaMemcpyDeviceToHost : cudaMemcpyHostToDevice;
+    if (kind == 2) {                               // device to device, either end possibly another GPU
+        for (const void* p : {(const void*)dst, src}) {
+            cudaPointerAttributes a;
+            NSR_CHECK(cudaPointerGetAttributes(&a, p));
+            NSR_REQUIRE(a.type == cudaMemoryTypeDevice, "nsr_copy2d: kind 2 takes device memory");
+            if (enable_peer(ctx, a.device)) return 1;
+        }
+        how = cudaMemcpyDefault;                   // unified addressing: the driver routes a copy between two GPUs
+    }
     NSR_CHECK(cudaMemcpy2DAsync(dst, (size_t)dst_pitch, src, (size_t)src_pitch, (size_t)width_bytes, (size_t)height,
-                                kind == 0 ? cudaMemcpyDeviceToHost : cudaMemcpyHostToDevice, (cudaStream_t)stream));
+                                how, (cudaStream_t)stream));
     return 0;
 }
 
@@ -562,15 +588,7 @@ extern "C" int nsr_copy_peer(nsr_ctx* ctx, uintptr_t stream, void* dst, const vo
     NSR_REQUIRE(ctx != nullptr && dst && src && nbytes >= 0 && src_device >= 0, "nsr_copy_peer: bad arguments");
     if (nbytes == 0) return 0;
     NSR_CHECK(cudaSetDevice(ctx->device));
-    if (src_device != ctx->device) {
-        int can = 0;
-        NSR_CHECK(cudaDeviceCanAccessPeer(&can, ctx->device, src_device));
-        if (can) {                                 // direct NVLink / PCIe peer path; otherwise the driver stages through the host
-            cudaError_t e = cudaDeviceEnablePeerAccess(src_device, 0);
-            if (e == cudaErrorPeerAccessAlreadyEnabled) (void)cudaGetLastError();
-            else NSR_CHECK(e);
-        }
-    }
+    if (enable_peer(ctx, src_device)) return 1;
     NSR_CHECK(cudaMemcpyPeerAsync(dst, ctx->device, src, src_device, (size_t)nbytes, (cudaStream_t)stream));
     return 0;
 }

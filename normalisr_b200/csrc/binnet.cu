@@ -13,6 +13,9 @@
 // (binnet.py:122-124 computes w = cumsum / n0 and p / w), so the boolean output is bit-identical.
 // One CTA per row: the row is read from HBM once into shared memory (rows up to 25,000 entries;
 // wider rows re-read themselves from L2).
+// The sparse (CSR) network takes two launches: the same row kernels instantiated with kCount write each
+// row's threshold and edge count instead of the uint8 row (nsr_binnet_count), then binnet_csr_fill_kernel
+// re-reads the rows and compacts the edges (nsr_binnet_csr_fill): 16 B read per entry + 4 B per edge.
 #include "nsr_common.cuh"
 
 namespace {
@@ -86,9 +89,13 @@ struct RowShared {
 };
 
 
+// kCount: instead of the uint8 row, write the row's threshold (thr_out, -1 without an edge) and its edge count
+// (count_out): entry j is an edge iff j is not the diagonal and P[j] <= thr_out (nsr_binnet_csr_fill).
+template <bool kCount>
 __global__ void __launch_bounds__(kThreads)
 binnet_rows_smem_kernel(const double* __restrict__ P, int64_t cols, int64_t ld, int64_t diag0, double qcut,
-                        uint8_t* __restrict__ net, int64_t ld_net, unsigned long long* __restrict__ stats) {
+                        uint8_t* __restrict__ net, int64_t ld_net, unsigned long long* __restrict__ stats,
+                        double* __restrict__ thr_out, int64_t* __restrict__ count_out) {
     extern __shared__ __align__(16) double s_row[];
     __shared__ RowShared sh;
     const int64_t row = blockIdx.x;
@@ -98,7 +105,11 @@ binnet_rows_smem_kernel(const double* __restrict__ P, int64_t cols, int64_t ld, 
     const int64_t n0 = cols - (has_diag ? 1 : 0);
     const double n0d = (double)n0;
     if (n0 <= 0) {                                       // a 1 x 1 block holding only its diagonal entry
-        for (int64_t j = threadIdx.x; j < cols; j += kThreads) net[row * ld_net + j] = 0;
+        if constexpr (kCount) {
+            if (threadIdx.x == 0) { thr_out[row] = -1.0; count_out[row] = 0; }
+        } else {
+            for (int64_t j = threadIdx.x; j < cols; j += kThreads) net[row * ld_net + j] = 0;
+        }
         return;
     }
 
@@ -297,24 +308,28 @@ binnet_rows_smem_kernel(const double* __restrict__ P, int64_t cols, int64_t ld, 
         }
     }
     // ---- output (thr = -1 when nothing passes; the patched diagonal holds 2.0)
-    uint8_t* o_row = net + row * ld_net;
-    int64_t done = 0;
-    if (((uintptr_t)o_row & 7) == 0) {                   // 8 entries -> one 8-byte store
-        const double2* v = reinterpret_cast<const double2*>(s_row);
-        const int64_t oct = cols >> 3;
-        for (int64_t j = threadIdx.x; j < oct; j += kThreads) {
-            uint64_t out_bits = 0;
+    if constexpr (kCount) {
+        if (threadIdx.x == 0) { thr_out[row] = c > 0 ? thr : -1.0; count_out[row] = c > 0 ? c : 0; }
+    } else {
+        uint8_t* o_row = net + row * ld_net;
+        int64_t done = 0;
+        if (((uintptr_t)o_row & 7) == 0) {               // 8 entries -> one 8-byte store
+            const double2* v = reinterpret_cast<const double2*>(s_row);
+            const int64_t oct = cols >> 3;
+            for (int64_t j = threadIdx.x; j < oct; j += kThreads) {
+                uint64_t out_bits = 0;
 #pragma unroll
-            for (int q = 0; q < 4; ++q) {
-                const double2 p = v[4 * j + q];
-                out_bits |= (uint64_t)(p.x <= thr ? 1 : 0) << (16 * q);
-                out_bits |= (uint64_t)(p.y <= thr ? 1 : 0) << (16 * q + 8);
+                for (int q = 0; q < 4; ++q) {
+                    const double2 p = v[4 * j + q];
+                    out_bits |= (uint64_t)(p.x <= thr ? 1 : 0) << (16 * q);
+                    out_bits |= (uint64_t)(p.y <= thr ? 1 : 0) << (16 * q + 8);
+                }
+                reinterpret_cast<uint64_t*>(o_row)[j] = out_bits;
             }
-            reinterpret_cast<uint64_t*>(o_row)[j] = out_bits;
+            done = oct << 3;
         }
-        done = oct << 3;
+        for (int64_t j = done + threadIdx.x; j < cols; j += kThreads) o_row[j] = s_row[j] <= thr ? 1 : 0;
     }
-    for (int64_t j = done + threadIdx.x; j < cols; j += kThreads) o_row[j] = s_row[j] <= thr ? 1 : 0;
     if (c > 0 && threadIdx.x == 0) atomicAdd(&stats[0], (unsigned long long)c);
 }
 
@@ -354,9 +369,11 @@ __device__ __forceinline__ int block_sum_k(int v, int* s_red) {
     return t;
 }
 
+template <bool kCount>
 __global__ void __launch_bounds__(kKeyThreads, 4)
 binnet_rows_key_kernel(const double* __restrict__ P, int64_t cols, int64_t ld, int64_t diag0, double qcut,
-                       uint8_t* __restrict__ net, int64_t ld_net, unsigned long long* __restrict__ stats) {
+                       uint8_t* __restrict__ net, int64_t ld_net, unsigned long long* __restrict__ stats,
+                       double* __restrict__ thr_out, int64_t* __restrict__ count_out) {
     extern __shared__ __align__(16) uint16_t s_key[];
     __shared__ KeyShared sh;
     const int64_t row = blockIdx.x;
@@ -367,7 +384,11 @@ binnet_rows_key_kernel(const double* __restrict__ P, int64_t cols, int64_t ld, i
     const int64_t n0 = cols - (has_diag ? 1 : 0);
     const double n0d = (double)n0;
     if (n0 <= 0) {                                       // a 1 x 1 block holding only its diagonal entry
-        for (int64_t j = threadIdx.x; j < cols; j += kKeyThreads) net[row * ld_net + j] = 0;
+        if constexpr (kCount) {
+            if (threadIdx.x == 0) { thr_out[row] = -1.0; count_out[row] = 0; }
+        } else {
+            for (int64_t j = threadIdx.x; j < cols; j += kKeyThreads) net[row * ld_net + j] = 0;
+        }
         return;
     }
     for (int b = threadIdx.x; b <= kKeyBins; b += kKeyThreads) sh.hist[b] = 0;
@@ -573,6 +594,11 @@ binnet_rows_key_kernel(const double* __restrict__ P, int64_t cols, int64_t ld, i
             thr = c > 0 ? bh_threshold((double)c / n0d, qcut) : -1.0;
         }
     }
+    if constexpr (kCount) {
+        if (threadIdx.x == 0) { thr_out[row] = c > 0 ? thr : -1.0; count_out[row] = c > 0 ? c : 0; }
+        if (c > 0 && threadIdx.x == 0) atomicAdd(&stats[0], (unsigned long long)c);
+        return;
+    }
     // ---- output from the keys (c == 0: nothing passes).  thr = t(c) with 1 <= c, so t1 <= thr <= qcut and
     // its bin needs no clamping.  Entries in the threshold's own bin are the undecided window: the vector path
     // writes them as 0 and they are patched from the window's values afterwards.
@@ -612,9 +638,11 @@ binnet_rows_key_kernel(const double* __restrict__ P, int64_t cols, int64_t ld, i
 }
 
 // Rows wider than shared memory: plain iteration, the row re-read from L2 every step.
+template <bool kCount>
 __global__ void __launch_bounds__(kThreads)
 binnet_rows_wide_kernel(const double* __restrict__ P, int64_t cols, int64_t ld, int64_t diag0, double qcut,
-                        uint8_t* __restrict__ net, int64_t ld_net, unsigned long long* __restrict__ stats) {
+                        uint8_t* __restrict__ net, int64_t ld_net, unsigned long long* __restrict__ stats,
+                        double* __restrict__ thr_out, int64_t* __restrict__ count_out) {
     __shared__ int s_red[kThreads / 32];
     const int64_t row = blockIdx.x;
     const double* p_row = P + row * ld;
@@ -622,7 +650,11 @@ binnet_rows_wide_kernel(const double* __restrict__ P, int64_t cols, int64_t ld, 
     const bool has_diag = diag >= 0 && diag < cols;
     const int64_t n0 = cols - (has_diag ? 1 : 0);
     if (n0 <= 0) {
-        for (int64_t j = threadIdx.x; j < cols; j += kThreads) net[row * ld_net + j] = 0;
+        if constexpr (kCount) {
+            if (threadIdx.x == 0) { thr_out[row] = -1.0; count_out[row] = 0; }
+        } else {
+            for (int64_t j = threadIdx.x; j < cols; j += kThreads) net[row * ld_net + j] = 0;
+        }
         return;
     }
     int bad = 0, mine = 0;
@@ -645,11 +677,88 @@ binnet_rows_wide_kernel(const double* __restrict__ P, int64_t cols, int64_t ld, 
         if (c_new == c) break;
         c = c_new;
     }
-    uint8_t* o_row = net + row * ld_net;
     if (c == 0) thr = -1.0;
+    if constexpr (kCount) {
+        if (threadIdx.x == 0) { thr_out[row] = thr; count_out[row] = c; }
+    } else {
+        uint8_t* o_row = net + row * ld_net;
 #pragma unroll 8
-    for (int64_t j = threadIdx.x; j < cols; j += kThreads) o_row[j] = (j != diag && p_row[j] <= thr) ? 1 : 0;
+        for (int64_t j = threadIdx.x; j < cols; j += kThreads) o_row[j] = (j != diag && p_row[j] <= thr) ? 1 : 0;
+    }
     if (c > 0 && threadIdx.x == 0) atomicAdd(&stats[0], (unsigned long long)c);
+}
+
+// ---------------------------------------------------------------------------------------------
+// CSR compaction of rows whose threshold nsr_binnet_count found: entry j of row i is kept iff
+// j != i + diag0 and P[j] <= thr[i] - the dense kernels' own decision (the key kernel's "key < key(thr)
+// => p < thr" and exact finish on the threshold's bin, the 8-byte and wide kernels' p <= thr).  One CTA
+// per row walks it in steps of 1024 entries: each warp takes 4 chunks of 32, a ballot per chunk gives the
+// kept lanes, and a CTA prefix over the warps' counts (double-buffered, one barrier a step) places them, so
+// the column indices come out ascending.  Optionally the same pass gathers P and a second matrix D at the
+// kept positions.  A row never writes past its indptr range; a count that disagrees with it raises *err.
+constexpr int kFillThreads = 256;
+constexpr int kFillChunks = 4;          // 32-entry chunks per warp and step
+
+template <typename Idx>
+__global__ void __launch_bounds__(kFillThreads)
+binnet_csr_fill_kernel(const double* __restrict__ P, int64_t cols, int64_t ld, int64_t diag0,
+                       const double* __restrict__ thr, const int64_t* __restrict__ indptr, Idx* __restrict__ indices,
+                       const double* __restrict__ D, int64_t ld_d, double* __restrict__ p_out,
+                       double* __restrict__ d_out, unsigned long long* __restrict__ err) {
+    __shared__ int s_tot[2][kFillThreads / 32];
+    const int64_t row = blockIdx.x;
+    const double t = thr[row];
+    const int64_t begin = indptr[row], want = indptr[row + 1] - begin;
+    if (!(t >= 0.0)) {                                   // a row without edges
+        if (want != 0 && threadIdx.x == 0) atomicAdd(err, 1ull);
+        return;
+    }
+    const double* p_row = P + row * ld;
+    const double* d_row = D != nullptr ? D + row * ld_d : nullptr;
+    const int64_t diag = row + diag0;
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const uint32_t lower = (1u << lane) - 1u;
+    int64_t written = 0;                                 // entries of the row placed by earlier steps
+    int par = 0;
+    for (int64_t j0 = 0; j0 < cols; j0 += kFillThreads * kFillChunks) {
+        const int64_t jw = j0 + (int64_t)warp * (32 * kFillChunks) + lane;
+        uint32_t m[kFillChunks];
+        double pv[kFillChunks];
+        int mine = 0;
+#pragma unroll
+        for (int u = 0; u < kFillChunks; ++u) {
+            const int64_t j = jw + 32 * u;
+            pv[u] = j < cols ? p_row[j] : 2.0;
+            m[u] = __ballot_sync(0xffffffffu, j != diag && pv[u] <= t);
+            mine += __popc(m[u]);
+        }
+        if (lane == 0) s_tot[par][warp] = mine;
+        __syncthreads();
+        int before = 0, total = 0;
+#pragma unroll
+        for (int w = 0; w < kFillThreads / 32; ++w) {
+            const int v = s_tot[par][w];
+            before += w < warp ? v : 0;
+            total += v;
+        }
+        int64_t pos = written + before;
+#pragma unroll
+        for (int u = 0; u < kFillChunks; ++u) {
+            const int64_t k = pos + __popc(m[u] & lower);
+            if (((m[u] >> lane) & 1u) && k < want) {
+                const int64_t j = jw + 32 * u;
+                indices[begin + k] = (Idx)j;
+                if (p_out != nullptr) {
+                    p_out[begin + k] = pv[u];
+                    d_out[begin + k] = d_row[j];
+                }
+            }
+            pos += __popc(m[u]);
+        }
+        written += total;
+        par ^= 1;
+    }
+    if (written != want && threadIdx.x == 0) atomicAdd(err, 1ull);
 }
 
 constexpr int kKeyRowMax = 100000;     // keys of a row kept in shared memory (200 KB; four rows per SM up to ~20,000)
@@ -658,29 +767,69 @@ constexpr int kKeyRowMax = 100000;     // keys of a row kept in shared memory (2
 
 int nsr_binnet_keys = 1;               // test hook (nsr_set_option "binnet_keys"): 0 = the 8-byte-row kernel
 
-extern "C" int nsr_binnet(nsr_ctx* ctx, uintptr_t stream, const double* P, int64_t rows, int64_t cols, int64_t ld,
-                          int64_t diag0, double qcut, uint8_t* net, int64_t ld_net, unsigned long long* stats) {
-    NSR_REQUIRE(ctx && P && net && stats, "nsr_binnet: null argument");
-    NSR_REQUIRE(rows >= 1 && cols >= 1 && ld >= cols && ld_net >= cols && rows < (1ll << 31),
+namespace {
+
+// the row kernel nsr_binnet_keys and the row width select; kCount as in binnet_rows_smem_kernel
+template <bool kCount>
+int binnet_launch(nsr_ctx* ctx, uintptr_t stream, const double* P, int64_t rows, int64_t cols, int64_t ld,
+                  int64_t diag0, double qcut, uint8_t* net, int64_t ld_net, unsigned long long* stats, double* thr,
+                  int64_t* count) {
+    NSR_REQUIRE(rows >= 1 && cols >= 1 && ld >= cols && (kCount || ld_net >= cols) && rows < (1ll << 31),
                 "nsr_binnet: bad shape rows=%lld cols=%lld", (long long)rows, (long long)cols);
     NSR_REQUIRE(qcut > 0.0 && qcut < 1.0, "nsr_binnet: qcut must be in (0, 1)");
     NSR_CHECK(cudaSetDevice(ctx->device));
     if (nsr_binnet_keys != 0 && cols <= kKeyRowMax) {
         const int smem = (int)(((cols + 7) & ~(int64_t)7) * sizeof(uint16_t));
-        NSR_CHECK(cudaFuncSetAttribute(binnet_rows_key_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+        NSR_CHECK(cudaFuncSetAttribute(binnet_rows_key_kernel<kCount>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                        kKeyRowMax * (int)sizeof(uint16_t)));
-        binnet_rows_key_kernel<<<(unsigned)rows, kKeyThreads, smem, (cudaStream_t)stream>>>(P, cols, ld, diag0, qcut, net,
-                                                                                            ld_net, stats);
+        binnet_rows_key_kernel<kCount><<<(unsigned)rows, kKeyThreads, smem, (cudaStream_t)stream>>>(
+            P, cols, ld, diag0, qcut, net, ld_net, stats, thr, count);
     } else if (cols <= kSmemRowMax) {
         const int smem = (int)(((cols + 1) & ~(int64_t)1) * sizeof(double));
-        NSR_CHECK(cudaFuncSetAttribute(binnet_rows_smem_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+        NSR_CHECK(cudaFuncSetAttribute(binnet_rows_smem_kernel<kCount>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                        kSmemRowMax * (int)sizeof(double)));
-        binnet_rows_smem_kernel<<<(unsigned)rows, kThreads, smem, (cudaStream_t)stream>>>(P, cols, ld, diag0, qcut, net,
-                                                                                          ld_net, stats);
+        binnet_rows_smem_kernel<kCount><<<(unsigned)rows, kThreads, smem, (cudaStream_t)stream>>>(
+            P, cols, ld, diag0, qcut, net, ld_net, stats, thr, count);
     } else {
-        binnet_rows_wide_kernel<<<(unsigned)rows, kThreads, 0, (cudaStream_t)stream>>>(P, cols, ld, diag0, qcut, net,
-                                                                                       ld_net, stats);
+        binnet_rows_wide_kernel<kCount><<<(unsigned)rows, kThreads, 0, (cudaStream_t)stream>>>(
+            P, cols, ld, diag0, qcut, net, ld_net, stats, thr, count);
     }
+    NSR_CHECK(cudaGetLastError());
+    return 0;
+}
+
+}  // namespace
+
+extern "C" int nsr_binnet(nsr_ctx* ctx, uintptr_t stream, const double* P, int64_t rows, int64_t cols, int64_t ld,
+                          int64_t diag0, double qcut, uint8_t* net, int64_t ld_net, unsigned long long* stats) {
+    NSR_REQUIRE(ctx && P && net && stats, "nsr_binnet: null argument");
+    return binnet_launch<false>(ctx, stream, P, rows, cols, ld, diag0, qcut, net, ld_net, stats, nullptr, nullptr);
+}
+
+extern "C" int nsr_binnet_count(nsr_ctx* ctx, uintptr_t stream, const double* P, int64_t rows, int64_t cols,
+                                int64_t ld, int64_t diag0, double qcut, double* thr, int64_t* count,
+                                unsigned long long* stats) {
+    NSR_REQUIRE(ctx && P && thr && count && stats, "nsr_binnet_count: null argument");
+    return binnet_launch<true>(ctx, stream, P, rows, cols, ld, diag0, qcut, nullptr, 0, stats, thr, count);
+}
+
+extern "C" int nsr_binnet_csr_fill(nsr_ctx* ctx, uintptr_t stream, const double* P, int64_t rows, int64_t cols,
+                                   int64_t ld, int64_t diag0, const double* thr, const int64_t* indptr, void* indices,
+                                   int index_bytes, const double* D, int64_t ld_d, double* p_out, double* d_out,
+                                   unsigned long long* err) {
+    NSR_REQUIRE(ctx && P && thr && indptr && indices && err, "nsr_binnet_csr_fill: null argument");
+    NSR_REQUIRE(index_bytes == 4 || index_bytes == 8, "nsr_binnet_csr_fill: index_bytes must be 4 or 8");
+    NSR_REQUIRE((p_out == nullptr) == (d_out == nullptr) && (p_out == nullptr || (D && ld_d >= cols)),
+                "nsr_binnet_csr_fill: p_out, d_out and D go together");
+    NSR_REQUIRE(rows >= 1 && cols >= 1 && ld >= cols && rows < (1ll << 31),
+                "nsr_binnet_csr_fill: bad shape rows=%lld cols=%lld", (long long)rows, (long long)cols);
+    NSR_CHECK(cudaSetDevice(ctx->device));
+    if (index_bytes == 4)
+        binnet_csr_fill_kernel<int32_t><<<(unsigned)rows, kFillThreads, 0, (cudaStream_t)stream>>>(
+            P, cols, ld, diag0, thr, indptr, (int32_t*)indices, D, ld_d, p_out, d_out, err);
+    else
+        binnet_csr_fill_kernel<int64_t><<<(unsigned)rows, kFillThreads, 0, (cudaStream_t)stream>>>(
+            P, cols, ld, diag0, thr, indptr, (int64_t*)indices, D, ld_d, p_out, d_out, err);
     NSR_CHECK(cudaGetLastError());
     return 0;
 }

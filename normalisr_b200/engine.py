@@ -531,6 +531,19 @@ def copy_rect_to_host(ctx, dst_host, dr0, dc0, src_dev, sr0, sc0, rows, cols, st
                                   cols * es, rows, 0), "nsr_copy2d")
 
 
+def copy_rect_to_peer(ctx, dst_dev, dr0, dc0, src_dev, sr0, sc0, rows, cols, stream=None):
+    """dst_dev[dr0:dr0+rows, dc0:dc0+cols] <- src_dev[sr0:sr0+rows, sc0:sc0+cols] (2-D float64, unit column
+    stride; src on ctx's device, dst on any GPU of this process), asynchronously on ``stream`` of ctx's device."""
+    if rows <= 0 or cols <= 0:
+        return
+    es = 8
+    st = stream.cuda_stream if stream is not None else _stream()
+    _lib.check(ctx.lib.nsr_copy2d(ctx.handle, st,
+                                  dst_dev.data_ptr() + (dr0 * dst_dev.stride(0) + dc0) * es, dst_dev.stride(0) * es,
+                                  src_dev.data_ptr() + (sr0 * src_dev.stride(0) + sc0) * es, src_dev.stride(0) * es,
+                                  cols * es, rows, 2), "nsr_copy2d")
+
+
 def copy_peer(ctx, dst, src, stream=None):
     """dst (contiguous tensor on ctx's device) <- src (contiguous tensor of the same byte size on another
     device of this process), asynchronously on ``stream`` of ctx's device (copy engines, no kernel)."""

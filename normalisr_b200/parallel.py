@@ -380,7 +380,7 @@ def _mirror_pair(device, k, blk):
 
 
 def contract_plan(ctx, local, rounds, rank, world, n_gene, dof_a, n_products, k_chunk, out=None, events=None,
-                  out_host=None, single_launch=True, home=None, skip_diag=False):
+                  out_host=None, single_launch=True, home=None, skip_diag=False, gather=None):
     """Contract everything ``rank`` owns under the pairs schedule: the upper triangle of its diagonal
     block, then the block pairs of ``rounds`` = [(src, parity, Sliced of block src, works)].
     ``works``: [] when the block is already there (the one-GPU emulation of the schedule in
@@ -399,6 +399,10 @@ def contract_plan(ctx, local, rounds, rank, world, n_gene, dof_a, n_products, k_
                  computes (diagonal block: into P itself; block pair: into a (rows_b x rows_a) buffer) and
                  both rectangles are copied home, so that after all ranks are done every entry of both
                  triangles has been written exactly once.
+      gather   = one (P, dot) pair of device tensors per rank (the (P, dot) of every rank's call, rows of its
+                 block x n_gene, on that rank's GPU): as with ``home`` the kernel writes the transposed copies,
+                 and those of block pair (rank, src) go peer to peer into gather[src] at the columns of this
+                 block, so that every rank ends up holding COMPLETE rows of its block once all ranks are done.
     ``skip_diag``: the diagonal block is already done and on its way home (``diag_block_streamed``: contracted
     in strips while the block's rows were still arriving from the host); only the block pairs are launched."""
     blk = local.rows_alloc
@@ -413,17 +417,18 @@ def contract_plan(ctx, local, rounds, rank, world, n_gene, dof_a, n_products, k_
     if not rows_a:
         return P, D
     r0 = rank * blk
-    to_host = out_host is not None or home is not None
+    mirrored = home is not None or gather is not None
+    to_host = out_host is not None or mirrored            # (gather: to the peers)
     copy_stream = _side_stream2(dev) if to_host else None
     main = torch.cuda.current_stream()
 
     segs, tiles, extra = [], [], []
     if not skip_diag:
         segs.append(dict(B=local, rows_b=rows_a, col0=r0, diagonal=True))
-        if home is not None:
+        if mirrored:
             segs[0]["mirror"] = (P.data_ptr() + 8 * r0, D.data_ptr() + 8 * r0, P.stride(0))
         tiles.append(engine.coex_tiles(rows_a))
-        extra.append(dict(works=[], rect=(0, rows_a, 0, rows_a), mbuf=None))
+        extra.append(dict(works=[], rect=(0, rows_a, 0, rows_a), mbuf=None, src=rank))
     n_pairs = sum(1 for r in rounds if block_rows(n_gene, world, r[0]))
     pairs_done = 0
     flag_driven = single_launch and not k_chunk and all(len(r[3]) == 0 or isinstance(r[3][0], _FlagWork) for r in rounds)
@@ -434,7 +439,7 @@ def contract_plan(ctx, local, rounds, rank, world, n_gene, dof_a, n_products, k_
         buf.rows = rows_b
         sg = dict(B=buf, rows_b=rows_b, col0=src * blk, diagonal=False)
         mbuf = None
-        if home is not None:
+        if mirrored:
             mbuf = _mirror_pair(dev, k, blk)
             sg["mirror"] = (mbuf[0].data_ptr(), mbuf[1].data_ptr(), blk)
         tl = pair_tiles(rows_a, rows_b, parity)
@@ -443,13 +448,13 @@ def contract_plan(ctx, local, rounds, rank, world, n_gene, dof_a, n_products, k_
         # (same operands, its own `done` counter), so that a strip leaves while the next one is contracted
         # instead of the whole rectangle waiting for its last tile
         n_sub = 1
-        if home is not None and len(tl) and flag_driven:
+        if mirrored and len(tl) and flag_driven:
             n_sub = max(1, min(PAIR_STRIPS, (MAX_SEGMENTS - len(segs)) // max(1, n_pairs - pairs_done)))
         pairs_done += 1
         for sel, rect in pair_strips(tl, (a0, a1, b0, b1), n_sub):
             segs.append(dict(sg))
             tiles.append(sel)
-            extra.append(dict(works=works, rect=rect, mbuf=mbuf))
+            extra.append(dict(works=works, rect=rect, mbuf=mbuf, src=src))
 
     def send(i):
         """queue the device-to-host copies of segment i on the copy stream"""
@@ -466,6 +471,11 @@ def contract_plan(ctx, local, rounds, rank, world, n_gene, dof_a, n_products, k_
                 if ex["mbuf"] is not None:
                     engine.copy_rect_to_host(ctx, dst_t, c0 + b0, r0 + a0, ex["mbuf"][t], b0, a0, b1 - b0, a1 - a0,
                                              stream=copy_stream)
+        if gather is not None and ex["mbuf"] is not None:
+            a0, a1, b0, b1 = ex["rect"]
+            for t in range(2):
+                engine.copy_rect_to_peer(ctx, gather[ex["src"]][t], b0, r0 + a0, ex["mbuf"][t], b0, a0, b1 - b0,
+                                         a1 - a0, stream=copy_stream)
 
     if not segs:
         return P, D
@@ -764,6 +774,9 @@ class _Team:
         self.stores = [None] * world          # peer-readable home of every device's block
         self.ready = [None] * world           # CUDA event: block residualised
         self.errors = [None] * world
+        self.outs = [None] * world            # coexnet: every device's (P, dot) rows, the targets of the peer copies
+        self.sent = [None] * world            # coexnet: CUDA event behind a device's copies to its peers
+        self.nets = [None] * world            # coexnet: every device's part of the network (host)
 
 
 _STORES = {}
@@ -796,7 +809,10 @@ def _pull_rounds(ctx, team, rank, world, local):
     return rounds
 
 
-def _device_worker(team, rank, world, dev, xh, dc, n_gene, precision, dimreduce, home, var_out):
+def _device_worker(team, rank, world, dev, xh, dc, n_gene, precision, dimreduce, home, var_out, net=None):
+    """One GPU of ``coex_all_devices``, or of ``coexnet_all_devices`` with ``net`` (a ``_NetJob``): then nothing
+    goes home; the transposed rectangles go to the peers that own their rows (``contract_plan``'s ``gather``),
+    and each device thresholds its complete rows (``_net_rows``)."""
     from .association import _residualize_any
     try:
         torch.cuda.set_device(dev)
@@ -827,7 +843,7 @@ def _device_worker(team, rank, world, dev, xh, dc, n_gene, precision, dimreduce,
                              torch.zeros((max(rows_a, 1), n_gene), dtype=torch.float64, device=dev))
         out = _STORES[okey]
         tail = None
-        streamed = rows_a > 0 and STREAM_DIAGONAL
+        streamed = rows_a > 0 and STREAM_DIAGONAL and net is None       # (streamed: the diagonal block goes home)
         if streamed:
             tail = diag_block_streamed(ctx, xh[r0:r0 + rows_a], Qt_dev, n_slices, n_products, dof_a, local, out, home, r0)
         elif rows_a:
@@ -835,10 +851,14 @@ def _device_worker(team, rank, world, dev, xh, dc, n_gene, precision, dimreduce,
         ev = torch.cuda.Event()
         ev.record()
         team.stores[rank], team.ready[rank] = store, ev
+        gather = None
+        if net is not None:
+            team.outs[rank] = out
+            gather = team.outs
         team.barrier.wait()                       # every block's event exists
         rounds = _pull_rounds(ctx, team, rank, world, local)
         contract_plan(ctx, local, rounds, rank, world, n_gene, dof_a, n_products, 0, out, None, None, home=home,
-                      skip_diag=streamed)
+                      skip_diag=streamed, gather=gather)
         # the optimistic single pass over the cells is verified like in _coex_pairs
         for r in rounds:
             wait_block(r[3])
@@ -849,9 +869,11 @@ def _device_worker(team, rank, world, dev, xh, dc, n_gene, precision, dimreduce,
         k_chunk = engine.plan_k_chunk(local, local, n_products, energies=(em_a, em_b))
         if k_chunk:
             contract_plan(ctx, local, [(r[0], r[1], r[2], []) for r in rounds], rank, world, n_gene, dof_a,
-                          n_products, k_chunk, out, None, None, home=home)
+                          n_products, k_chunk, out, None, None, home=home, gather=gather)
         if rows_a:
             var_out[r0:r0 + rows_a].copy_(local.var[:rows_a], non_blocking=True)
+        if net is not None:
+            _net_rows(ctx, team, rank, world, out, rows_a, r0, net)
         torch.cuda.current_stream().synchronize()
         if tail is not None:
             tail.synchronize()
@@ -859,6 +881,99 @@ def _device_worker(team, rank, world, dev, xh, dc, n_gene, precision, dimreduce,
     except BaseException as e:                    # noqa: BLE001 - re-raised by the caller
         team.errors[rank] = e
         team.barrier.abort()
+
+
+class _NetJob:
+    """What ``coexnet_all_devices`` asks of each device: the cutoff, the output form, and where the rows go."""
+
+    def __init__(self, qcut, sparse, edge_values, dense_out):
+        self.qcut, self.sparse, self.edge_values, self.dense_out = qcut, sparse, edge_values, dense_out
+
+
+def _net_rows(ctx, team, rank, world, out, rows_a, r0, job):
+    """Once every peer's copies into ``out`` are done, the network of this device's rows [r0, r0 + rows_a):
+    team.nets[rank] = (edges, invalid) with the uint8 rows written into job.dense_out, or (indptr, indices[, P_e,
+    dot_e]) as numpy arrays of this block's CSR piece."""
+    from .binnet import binnet_rows, csr_rows
+    main = torch.cuda.current_stream()
+    ev = torch.cuda.Event()
+    ev.record(main)                               # contract_plan left main behind the copies to the peers
+    team.sent[rank] = ev
+    team.barrier.wait()                           # every device's event exists
+    for s in range(world):
+        if s != rank:
+            main.wait_event(team.sent[s])
+    if not rows_a:
+        team.nets[rank] = (0, 0) if not job.sparse else \
+            (np.zeros(1, np.int64), np.zeros(0, np.int32)) + ((np.zeros(0), np.zeros(0)) if job.edge_values else ())
+        return
+    P, D = out[0][:rows_a], out[1][:rows_a]
+    stats = torch.zeros(2, dtype=torch.int64, device=P.device)
+    if not job.sparse:
+        rows, _ = binnet_rows(ctx, P, job.qcut, r0, stats=stats)
+        job.dense_out[r0:r0 + rows_a].copy_(rows, non_blocking=True)
+        team.nets[rank] = tuple(int(x) for x in stats.cpu())
+        return
+    piece = csr_rows(ctx, P, job.qcut, r0, stats, D=D if job.edge_values else None)
+    team.nets[rank] = tuple(t.cpu().numpy() for t in piece[:4 if job.edge_values else 2])
+
+
+def _run_team(devs, xh, dc, n_gene, precision, dimreduce, home, var_out, net=None):
+    """One ``_device_worker`` thread per GPU; re-raises the first error of any of them."""
+    import threading
+    world = len(devs)
+    team = _Team(world)
+    threads = [threading.Thread(target=_device_worker, name="nsr-gpu%d" % r,
+                                args=(team, r, world, devs[r], xh, dc, n_gene, precision, dimreduce, home, var_out,
+                                      net))
+               for r in range(world)]
+    for t in threads:
+        t.start()
+    for t in threads:
+        t.join()
+    first = [e for e in team.errors if e is not None and not isinstance(e, threading.BrokenBarrierError)]
+    if first:
+        raise first[0]
+    if any(e is not None for e in team.errors):
+        raise RuntimeError("coex_all_devices: a worker stopped at a broken barrier")
+    return team
+
+
+def _host_f64(dt):
+    xh = dt if isinstance(dt, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(dt))
+    if xh.is_cuda:
+        raise ValueError("coex_all_devices takes a host matrix")
+    return xh if xh.dtype == torch.float64 else xh.to(torch.float64)
+
+
+def coexnet_all_devices(dt, dc, qcut, sparse=False, edge_values=False, devices="all", precision="default",
+                        dimreduce=0):
+    """``coex.coexnet`` on every GPU of the box from ONE process: the pairs schedule of ``coex_all_devices``,
+    but no G x G matrix leaves the GPUs.  Each device ends up holding complete rows of its gene block of P and
+    dot (the transposed rectangles of the block pairs travel peer to peer over NVLink), thresholds them with the
+    per-row BH kernels and ships its uint8 rows, or its CSR piece, to the host.  Returns (net, var) or, with
+    ``edge_values``, (net, var, P_e, dot_e): net a numpy bool (G, G) array or a scipy csr_matrix, exactly
+    ``binnet(coex(dt, dc)[0], qcut)`` of one GPU."""
+    from .binnet import concat_csr, host_csr
+    devs = visible_devices(devices)
+    xh = _host_f64(dt)
+    n_gene = xh.shape[0]
+    dense_out = None if sparse else torch.empty((n_gene, n_gene), dtype=torch.uint8, pin_memory=True)
+    var_out = torch.empty(n_gene, dtype=torch.float64, pin_memory=True)
+    team = _run_team(devs, xh, dc, n_gene, precision, dimreduce, None, var_out,
+                     _NetJob(qcut, sparse, edge_values, dense_out))
+    var = var_out.numpy()
+    if not sparse:
+        if any(r[1] for r in team.nets):
+            raise AssertionError('net must be finite with values in [0, 1].')
+        if sum(r[0] for r in team.nets) == 0:
+            raise RuntimeError("Empty binary network.")
+        return dense_out.numpy().view(bool), var
+    parts = concat_csr(team.nets, n_gene)
+    if parts[1].size == 0:
+        raise RuntimeError("Empty binary network.")
+    net = host_csr(n_gene, parts[0], parts[1])
+    return (net, var) + tuple(parts[2:])
 
 
 def coex_all_devices(dt, dc, devices="all", precision="default", dimreduce=0, out=None):
@@ -871,32 +986,14 @@ def coex_all_devices(dt, dc, devices="all", precision="default", dimreduce=0, ou
 
     dt: (n_gene, n_cell) numpy array or CPU tensor (page-locked memory makes the copies asynchronous);
     out: optional (P, dot) page-locked CPU tensors to fill."""
-    import threading
     devs = visible_devices(devices)
-    world = len(devs)
-    xh = dt if isinstance(dt, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(dt))
-    if xh.is_cuda:
-        raise ValueError("coex_all_devices takes a host matrix")
-    if xh.dtype != torch.float64:
-        xh = xh.to(torch.float64)
+    xh = _host_f64(dt)
     n_gene = xh.shape[0]
     if out is None:
         out = (torch.empty((n_gene, n_gene), dtype=torch.float64, pin_memory=True),
                torch.empty((n_gene, n_gene), dtype=torch.float64, pin_memory=True))
     var_out = torch.empty(n_gene, dtype=torch.float64, pin_memory=True)
-    team = _Team(world)
-    threads = [threading.Thread(target=_device_worker, name="nsr-gpu%d" % r,
-                                args=(team, r, world, devs[r], xh, dc, n_gene, precision, dimreduce, out, var_out))
-               for r in range(world)]
-    for t in threads:
-        t.start()
-    for t in threads:
-        t.join()
-    first = [e for e in team.errors if e is not None and not isinstance(e, threading.BrokenBarrierError)]
-    if first:
-        raise first[0]
-    if any(e is not None for e in team.errors):
-        raise RuntimeError("coex_all_devices: a worker stopped at a broken barrier")
+    _run_team(devs, xh, dc, n_gene, precision, dimreduce, out, var_out)
     return out[0].numpy(), out[1].numpy(), var_out.numpy()
 
 
