@@ -154,6 +154,16 @@ def covariate_basis_device(ctx, dc, tol=1e-8):
     return res
 
 
+def basis_and_dof(ctx, dc, n, dimreduce):
+    """``covariate_basis_device`` and the reference's check that ``n`` cells leave degrees of freedom:
+    (Qt_dev, rank, W, dof_a), dof_a the first shape parameter of the P-value's beta function."""
+    Qt_dev, rank, W = covariate_basis_device(ctx, dc)
+    if n <= rank + dimreduce + 1:
+        raise ValueError('Insufficient number of cells: must be greater than degrees of freedom '
+                         'removed + covariate + 1.')
+    return Qt_dev, rank, W, (n - 1 - rank - dimreduce) / 2
+
+
 def basis_cache_key(ctx, dc, tol=1e-8, tag=None):
     """Identity of an unmodified CUDA covariate tensor (None for anything else)."""
     if _is_dev(dc) and dc.device == ctx.device:
@@ -341,7 +351,8 @@ def _coex_host_pipeline(ctx, xh, Qt_dev, n_slices, n_products, dof_a, eng, keep_
         done[i & 1] = torch.cuda.Event()
         done[i & 1].record(main)
         _mark("projected", i, main)
-        tiles = engine.coex_strip_tiles(r0 // engine.TILE, (r1 + engine.TILE - 1) // engine.TILE)
+        t1 = (r1 + engine.TILE - 1) // engine.TILE
+        tiles = engine.upper_tiles(0, t1, r0 // engine.TILE, t1)
         # optimistic single pass over the cells (planning would need a device->host sync per chunk
         # and stall the copy stream); the int32 bound is verified once at the end
         engine.contract(ctx, MODE_COEX, A, A, tiles, dof_a, P, D, n_products, eng, k_chunk=0)
@@ -479,11 +490,7 @@ def association_tests(dx, dy, dc, bsx=0, bsy=0, nth=1, lowmem=True, return_dot=T
     nc = dc.shape[0]
     if nc == 0:
         logging.warning('No covariate dc input.')
-    Qt_dev, rank, W = covariate_basis_device(ctx, dc)
-    if n <= rank + dimreduce + 1:
-        raise ValueError('Insufficient number of cells: must be greater than degrees of freedom '
-                         'removed + covariate + 1.')
-    dof_a = (n - 1 - rank - dimreduce) / 2
+    Qt_dev, rank, W, dof_a = basis_and_dof(ctx, dc, n, dimreduce)
     with torch.cuda.device(ctx.device):
         keep_coef = not lowmem
         piped = samexy and to_host

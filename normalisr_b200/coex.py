@@ -34,7 +34,7 @@ def coexnet(dt, dc, qcut, sparse=False, edge_values=False, devices=None, device=
     ``dimreduce`` as for ``coex``.  Raises like ``coex`` and ``binnet``."""
     from . import engine, parallel
     from ._lib import MODE_COEX
-    from .association import _is_dev, _residualize_any, covariate_basis_device
+    from .association import _is_dev, _residualize_any, basis_and_dof
     from .binnet import device_net
     if len(dt.shape) != 2 or len(dc.shape) != 2:
         raise ValueError('Incorrect dx/dy/dc size.')
@@ -63,11 +63,7 @@ def coexnet(dt, dc, qcut, sparse=False, edge_values=False, devices=None, device=
     to_host = not _is_dev(dt)
     ctx = engine.context(device if device is not None else (dt.device if not to_host else None))
     n_slices, n_products = engine.PRESETS[precision]
-    Qt_dev, rank, _ = covariate_basis_device(ctx, dc)
-    if n <= rank + dimreduce + 1:
-        raise ValueError('Insufficient number of cells: must be greater than degrees of freedom '
-                         'removed + covariate + 1.')
-    dof_a = (n - 1 - rank - dimreduce) / 2
+    Qt_dev, _, _, dof_a = basis_and_dof(ctx, dc, n, dimreduce)
     with torch.cuda.device(ctx.device):
         A = _residualize_any(ctx, dt, Qt_dev, n_slices, False)
         P = torch.empty((n_gene, n_gene), dtype=torch.float64, device=ctx.device)

@@ -269,18 +269,25 @@ def single1_finish(ctx, cu, yy_u, st, n_groups, nc, ci, cx, ccx, ns, vx, dof, P,
     LAUNCHES += 1
 
 
-@functools.lru_cache(maxsize=64)
-def coex_tiles(rows, strip=12):
-    """Upper-triangular 128x128 tile list (tile_row <= tile_col), ordered in column strips so
-    that the ~148 tiles in flight share few row blocks (L2 reuse of the operand planes)."""
-    t = (rows + TILE - 1) // TILE
+@functools.lru_cache(maxsize=256)
+def upper_tiles(row_lo, row_hi, col_lo, col_hi, strip=12):
+    """Upper-triangular 128x128 tiles (tile_row <= tile_col) with tile row in [row_lo, row_hi) and tile
+    column in [col_lo, col_hi), ordered in column strips of ``strip`` tiles from col_lo so that the ~148
+    tiles in flight share few row blocks (L2 reuse of the operand planes).  Cached: the streamed host
+    pipeline asks for one list per row chunk."""
     out = []
-    for js in range(0, t, strip):
-        je = min(js + strip, t)
-        for i in range(0, je):
+    for js in range(col_lo, col_hi, strip):
+        je = min(js + strip, col_hi)
+        for i in range(row_lo, min(row_hi, je)):
             for j in range(max(i, js), je):
                 out.append((i, j))
     return np.asarray(out, dtype=np.int32).reshape(-1, 2)
+
+
+def coex_tiles(rows, strip=12):
+    """Every upper-triangular tile of a (rows x rows) output."""
+    t = (rows + TILE - 1) // TILE
+    return upper_tiles(0, t, 0, t, strip)
 
 
 @functools.lru_cache(maxsize=64)
@@ -360,10 +367,12 @@ def plan_k_chunk(A, B, n_products, energies=None):
     return 32768 - _lib.KBLOCK
 
 
-def contract(ctx, mode, A, B, tiles, dof_a, P, out2, n_products, engine=ENGINE_UMMA, k_chunk=None):
+def contract(ctx, mode, A, B, tiles, dof_a, P, out2, n_products, engine=ENGINE_UMMA, k_chunk=None, row0=0):
     """Run the contraction + epilogue for ``tiles`` ((k,2) int32 numpy array of tile coords).
     A may be a single exact plane (``residualize_exact``): then every product with B's planes is kept
-    and ``n_products`` is ignored."""
+    and ``n_products`` is ignored.  ``row0``: P / out2 hold output rows [row0, ...) only (a strip of
+    tile rows); the library gets base pointers row0 rows before them and dereferences only rows of the
+    listed tiles."""
     assert A.n == B.n
     if A.n_slices != B.n_slices or A.n_slices == 1:
         assert A.n_slices == 1
@@ -374,13 +383,14 @@ def contract(ctx, mode, A, B, tiles, dof_a, P, out2, n_products, engine=ENGINE_U
     ld = out2.stride(0) if out2.shape[0] > 1 else out2.shape[1]
     assert out2.stride(1) == 1 and (P is None or P.shape == out2.shape and P.stride(1) == 1)
     assert P is None or out2.shape[0] == 1 or P.stride(0) == ld
+    off = row0 * ld * 8
     st = ctx.lib.nsr_contract_ab(
         ctx.handle, _stream(), engine, mode,
         A.slices.data_ptr(), A.rows, A.rows_alloc, A.n_slices, A.quantum.data_ptr(), A.var.data_ptr(),
         B.slices.data_ptr(), B.rows, B.rows_alloc, B.n_slices, B.quantum.data_ptr(), B.var.data_ptr(),
         A.n, A.n_pad, n_products,
         tiles.ctypes.data, tiles.shape[0], float(dof_a),
-        P.data_ptr() if P is not None else None, out2.data_ptr(), ld, int(k_chunk))
+        P.data_ptr() - off if P is not None else None, out2.data_ptr() - off, ld, int(k_chunk))
     _lib.check(st, "nsr_contract")
     global LAUNCHES
     LAUNCHES += 1 if not k_chunk else -(-A.n_pad // k_chunk)
@@ -552,18 +562,6 @@ def copy_peer(ctx, dst, src, stream=None):
     st = stream.cuda_stream if stream is not None else _stream()
     _lib.check(ctx.lib.nsr_copy_peer(ctx.handle, st, dst.data_ptr(), src.data_ptr(), src.device.index, nbytes),
                "nsr_copy_peer")
-
-
-@functools.lru_cache(maxsize=256)
-def coex_strip_tiles(t_begin, t_end, strip=12):
-    """Upper-triangular tiles whose tile column lies in [t_begin, t_end), in column sub-strips."""
-    out = []
-    for js in range(t_begin, t_end, strip):
-        je = min(js + strip, t_end)
-        for i in range(0, je):
-            for j in range(max(i, js), je):
-                out.append((i, j))
-    return np.asarray(out, dtype=np.int32).reshape(-1, 2)
 
 
 def set_option(name, value):

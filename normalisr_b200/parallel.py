@@ -24,6 +24,7 @@ The path shards naturally (SURVEY.md 8e):
     counters (``pair_strips``), so copy-in, tensor work and copy-out overlap.
 Because the sums over cells are exact integers, every schedule gives bit-identical results.
 """
+import collections
 import logging
 
 import numpy as np
@@ -32,7 +33,7 @@ import torch.distributed as dist
 
 from . import engine
 from ._lib import MAX_SEGMENTS, MODE_COEX_RECT, MODE_COEX_UPPER, MODE_DE, TILE
-from .association import covariate_basis_device
+from .association import basis_and_dof, covariate_basis_device
 
 
 def row_split(rows, world):
@@ -158,13 +159,7 @@ def strip_bounds(n_tile_rows, world):
 
 def strip_tiles(n_tile_rows, a, b, strip=12):
     """Upper-triangular tiles with tile row in [a, b), column-strip ordered for L2 reuse."""
-    out = []
-    for js in range(a, n_tile_rows, strip):
-        je = min(js + strip, n_tile_rows)
-        for i in range(a, min(b, je)):
-            for j in range(max(i, js), je):
-                out.append((i, j))
-    return np.asarray(out, dtype=np.int32).reshape(-1, 2)
+    return engine.upper_tiles(a, b, a, n_tile_rows, strip)
 
 
 def gather_sliced(local, rows_total, group=None):
@@ -202,32 +197,28 @@ def _symm_block(nbytes, device, group):
     return _SYMM[key]
 
 
-def start_exchange_ce(local_store, hdl, local, group=None, ctx=None):
-    """Copy-engine variant of ``start_exchange``: every remote block is PULLED from the owner's
-    peer-mapped buffer with an asynchronous device-to-device copy on a side stream, so the exchange
-    uses no SMs while the contraction runs.  Each copy is followed by a stream-ordered flag write
-    (``nsr_stream_signal``): the persistent contraction launch, already running, starts on a block's
-    tiles when its flag appears.  Returns [(src, parity, Sliced, _FlagWork)]."""
-    world = dist.get_world_size(group)
-    rank = dist.get_rank(group)
-    hdl.barrier(channel=1, timeout_ms=60000)            # every rank's planes are written
-    side = _side_stream(local.slices.device)
+def _pull_rounds(ctx, local, rank, world, stores, pull):
+    """Copy-engine variant of ``start_exchange``: every remote block is PULLED with an asynchronous copy
+    on a side stream, so the exchange uses no SMs while the contraction runs.  Each copy is followed by a
+    stream-ordered flag write (``nsr_stream_signal``): the persistent contraction launch, already running,
+    starts on a block's tiles when its flag appears.  Round d lands in ``stores[d]`` (uint8, the size of
+    ``Sliced.storage_bytes``); ``pull(src, store)`` queues on the current stream (the side stream) whatever
+    the copy must wait for and the copy of block src into ``store``.  Returns [(src, parity, Sliced,
+    [_FlagWork])]."""
+    dev = local.slices.device
+    side = _side_stream(dev, "pull")
     side.wait_stream(torch.cuda.current_stream())
-    nbytes = local_store.numel()
+    sync = _sync_words(ctx)
+    sync.epoch += 1
     rounds = []
-    sync = _sync_words(ctx) if ctx is not None else None
     for d, (_, src, parity) in enumerate(exchange_plan(world, rank)):
-        store = torch.empty(nbytes, dtype=torch.uint8, device=local.slices.device)
-        store.record_stream(side)
         with torch.cuda.stream(side):
-            store.copy_(hdl.get_buffer(src, (nbytes,), torch.uint8, 0), non_blocking=True)
+            pull(src, stores[d])
             ev = torch.cuda.Event()
             ev.record(side)
-            work = _EventWork(ev)
-            if sync is not None:
-                work = _FlagWork(ev, sync.ready_ptr(d + 1), sync.epoch)
-                engine.stream_signal(ctx, work.flag_ptr, work.value, stream=side)
-        buf = engine.Sliced(local.rows_alloc, local.n, local.n_slices, local.slices.device, storage=store, fresh=False)
+            work = _FlagWork(ev, sync.ready_ptr(d + 1), sync.epoch)
+            engine.stream_signal(ctx, work.flag_ptr, work.value, stream=side)
+        buf = engine.Sliced(local.rows_alloc, local.n, local.n_slices, dev, storage=stores[d], fresh=False)
         rounds.append((src, parity, buf, [work]))
     return rounds
 
@@ -235,8 +226,9 @@ def start_exchange_ce(local_store, hdl, local, group=None, ctx=None):
 _SIDE = {}
 
 
-def _side_stream(device):
-    key = torch.device(device).index
+def _side_stream(device, role):
+    """One stream per device and role: "pull" brings remote blocks in, "send" takes results out."""
+    key = (torch.device(device).index, role)
     if key not in _SIDE:
         _SIDE[key] = torch.cuda.Stream(device=device)
     return _SIDE[key]
@@ -268,35 +260,33 @@ def _sync_words(ctx):
     return _SYNC[key]
 
 
-class _EventWork:
-    """Adapter: ``wait()`` makes the current stream wait for a CUDA event (like a c10d Work)."""
+class _FlagWork:
+    """A block a copy engine is bringing in (``_pull_rounds``): ``wait()`` makes the current stream wait for
+    the copy's event (like a c10d Work); the single-launch contraction instead waits inside the kernel for
+    the device flag the copy stream sets to ``value``."""
 
-    def __init__(self, ev):
-        self.ev = ev
+    def __init__(self, ev, flag_ptr, value):
+        self.ev, self.flag_ptr, self.value = ev, flag_ptr, value
 
     def wait(self):
         torch.cuda.current_stream().wait_event(self.ev)
 
 
-class _FlagWork(_EventWork):
-    """A block whose arrival is also announced by a device flag (see ``start_exchange_ce``): the
-    single-launch contraction waits for the flag inside the kernel instead of on the stream."""
-
-    def __init__(self, ev, flag_ptr, value):
-        super().__init__(ev)
-        self.flag_ptr, self.value = flag_ptr, value
-
-
-def residualize_block(ctx, x_block, Qt_dev, n_slices, blk, storage=None):
-    """Residualise this rank's rows into a block padded to ``blk`` rows (padding rows are zero
-    planes with quantum 1, var 1)."""
-    out = engine.Sliced(blk, x_block.shape[1], n_slices, ctx.device, storage=storage)
-    rows = x_block.shape[0]
+def _own_block(blk, rows, n, n_slices, device, storage=None):
+    """A rank's block of ``blk`` rows for its ``rows`` genes, before they are residualised into it: the
+    padding rows past them are zero planes with quantum 1, var 1."""
+    out = engine.Sliced(blk, n, n_slices, device, storage=storage)
     if rows < blk:
         out.slices[:, rows:].zero_()
         out.quantum[rows:] = 1.0
         out.var[rows:] = 1.0
-    if rows:
+    return out
+
+
+def residualize_block(ctx, x_block, Qt_dev, n_slices, blk, storage=None):
+    """Residualise this rank's rows into a block padded to ``blk`` rows (``_own_block``)."""
+    out = _own_block(blk, x_block.shape[0], x_block.shape[1], n_slices, ctx.device, storage=storage)
+    if x_block.shape[0]:
         engine.residualize(ctx, x_block, Qt_dev, n_slices, out=out, row_offset=0)
     return out
 
@@ -315,46 +305,54 @@ def _timed(events, fn):
 
 def _coex_pairs(ctx, local, n_gene, dof_a, n_products, group, out, events=None, out_host=None, symm=None, home=None,
                 skip_diag=False):
-    """Pairs schedule on an already residualised block: post the exchange and contract everything this
-    rank owns - with the copy-engine transport in ONE persistent launch that starts on the diagonal
-    block and picks up each block pair when its planes have arrived.  Returns (P, dot, var_all).
-    ``events`` (a list) receives one CUDA event pair per contraction launch (bench bookkeeping).
-    ``out_host`` = (P, dot) pinned CPU tensors: every finished column block is copied back on a
-    side stream while the next block pair is contracted (column blocks this rank does not own are
-    not written).  ``home`` = (P, dot) FULL (n_gene, n_gene) host tensors shared by all ranks (see
-    ``contract_plan``): every rank writes the rectangles it computed and their transposes.
-
-    The int32 partial sums are bounded from the digit energies AFTER the launch is queued (the
-    energies of the remote blocks travel with them): the contraction runs optimistically in one pass
-    over the cells and is redone in cell chunks if the bound fails (not observed below ~260k cells)."""
+    """Pairs schedule under torchrun on an already residualised block: post the exchange (copy-engine pulls
+    from the peers' symmetric memory ``symm`` = (store, handle), else NCCL) and contract everything this rank
+    owns (``_pairs``).  Returns (P, dot, var_all).  ``events`` (a list) receives one CUDA event pair per
+    contraction launch (bench bookkeeping); ``out_host``, ``home``, ``skip_diag`` as for ``contract_plan``."""
     world = dist.get_world_size(group) if dist.is_initialized() else 1
     rank = dist.get_rank(group) if dist.is_initialized() else 0
-    blk = local.rows_alloc
-    var_all = local.var
     rounds = []
+    if world > 1 and symm is None:
+        rounds = start_exchange(local, group)
+    elif world > 1:
+        hdl = symm[1]
+        nbytes = symm[0].numel()
+        hdl.barrier(channel=1, timeout_ms=60000)            # every rank's planes are written
+        side = _side_stream(local.slices.device, "pull")
+        stores = []
+        for _ in exchange_plan(world, rank):
+            stores.append(torch.empty(nbytes, dtype=torch.uint8, device=local.slices.device))
+            stores[-1].record_stream(side)
+        rounds = _pull_rounds(ctx, local, rank, world, stores, lambda src, store: store.copy_(
+            hdl.get_buffer(src, (nbytes,), torch.uint8, 0), non_blocking=True))
+    P, D = _pairs(ctx, local, rounds, rank, world, n_gene, dof_a, n_products, out, events, out_host, home, skip_diag)
+    var_all = local.var
     if world > 1:
-        if symm is not None:
-            _sync_words(ctx).epoch += 1
-            rounds = start_exchange_ce(symm[0], symm[1], local, group, ctx=ctx)
-        else:
-            rounds = start_exchange(local, group)
-    P, D = contract_plan(ctx, local, rounds, rank, world, n_gene, dof_a, n_products, 0, out, events, out_host, home=home,
-                         skip_diag=skip_diag)
-    if world > 1:
-        var_all = torch.empty(blk * world, dtype=torch.float64, device=local.var.device)
+        var_all = torch.empty(local.rows_alloc * world, dtype=torch.float64, device=local.var.device)
         dist.all_gather_into_tensor(var_all, local.var, group=group)
-    # verification of the optimistic single pass: bound over this rank's rows x every block it used
+    return P, D, var_all[:n_gene]
+
+
+def _pairs(ctx, local, rounds, rank, world, n_gene, dof_a, n_products, out, events=None, out_host=None, home=None,
+           skip_diag=False, gather=None):
+    """Everything ``rank`` owns under the pairs schedule, given its residualised block and the ``rounds`` of
+    the exchange (``contract_plan``): one optimistic pass over the cells, then the int32 partial sums are
+    bounded from the digit energies of this rank's rows and of every block it used (the energies of the
+    remote blocks travel with them, so no collective is needed) and the plan is redone in cell chunks if the
+    bound fails (not observed below ~260k cells).  Returns (P, dot)."""
+    P, D = contract_plan(ctx, local, rounds, rank, world, n_gene, dof_a, n_products, 0, out, events, out_host,
+                         home=home, skip_diag=skip_diag, gather=gather)
     for r in rounds:
         wait_block(r[3])
     em_a = local.energy_max.cpu().numpy()
     em_b = em_a
     for r in rounds:
-        em_b = np.maximum(em_b, r[2].energy_max.cpu().numpy())
+        em_b = np.maximum(em_b, r[2].energy_max.cpu().numpy())     # NaN (non-finite input) propagates
     k_chunk = engine.plan_k_chunk(local, local, n_products, energies=(em_a, em_b))
     if k_chunk:
         P, D = contract_plan(ctx, local, [(r[0], r[1], r[2], []) for r in rounds], rank, world, n_gene, dof_a,
-                             n_products, k_chunk, (P, D), None, out_host, home=home)
-    return P, D, var_all[:n_gene]
+                             n_products, k_chunk, (P, D), None, out_host, home=home, gather=gather)
+    return P, D
 
 
 def _segment_rect(rows_a, rows_b, parity):
@@ -379,6 +377,41 @@ def _mirror_pair(device, k, blk):
     return _MIRROR[key]
 
 
+Segment = collections.namedtuple("Segment", "src rows_b col0 diagonal tiles rect k works")
+Segment.__doc__ = """One segment of ``contract_plan``: the rows of block ``rank`` x block ``src`` (``rows_b`` rows, output
+columns from ``col0``); ``diagonal`` for the rank's own block (upper-triangular tiles, mirrored into P itself);
+``tiles`` (k, 2) int32 within the block pair; ``rect`` = (a0, a1, b0, b1) the rows x columns of the pair those
+tiles cover; ``k`` the round (1-based) whose block is B and whose mirror buffer receives the transposes, 0 for
+the diagonal; ``works`` what the block's arrival is waited for with ([] when it is there)."""
+
+
+def plan_segments(rounds, rank, world, n_gene, k_chunk=0, single_launch=True, mirrored=False, skip_diag=False):
+    """The segments ``contract_plan`` launches, on the host: the diagonal block (unless ``skip_diag``), then each
+    non-empty block pair of ``rounds`` = [(src, parity, block, works)].  When the transposes are written
+    (``mirrored``) and the launch is one flag-driven pass, a block pair is cut into column strips, each a segment
+    of its own (same operands, its own ``done`` counter), so that a strip leaves while the next one is contracted
+    instead of the whole rectangle waiting for its last tile."""
+    blk = row_split(n_gene, world)
+    rows_a = block_rows(n_gene, world, rank)
+    if not rows_a:
+        return []
+    segs = []
+    if not skip_diag:
+        segs.append(Segment(rank, rows_a, rank * blk, True, engine.coex_tiles(rows_a), (0, rows_a, 0, rows_a), 0, []))
+    pairs = [(k, src, parity, works) for k, (src, parity, _, works) in enumerate(rounds, 1)
+             if block_rows(n_gene, world, src)]
+    flag_driven = single_launch and not k_chunk and all(len(r[3]) == 0 or isinstance(r[3][0], _FlagWork) for r in rounds)
+    for done, (k, src, parity, works) in enumerate(pairs):
+        rows_b = block_rows(n_gene, world, src)
+        tl = pair_tiles(rows_a, rows_b, parity)
+        n_sub = 1
+        if mirrored and len(tl) and flag_driven:
+            n_sub = max(1, min(PAIR_STRIPS, (MAX_SEGMENTS - len(segs)) // (len(pairs) - done)))
+        for sel, rect in pair_strips(tl, _segment_rect(rows_a, rows_b, parity), n_sub):
+            segs.append(Segment(src, rows_b, src * blk, False, sel, rect, k, works))
+    return segs
+
+
 def contract_plan(ctx, local, rounds, rank, world, n_gene, dof_a, n_products, k_chunk, out=None, events=None,
                   out_host=None, single_launch=True, home=None, skip_diag=False, gather=None):
     """Contract everything ``rank`` owns under the pairs schedule: the upper triangle of its diagonal
@@ -386,12 +419,12 @@ def contract_plan(ctx, local, rounds, rank, world, n_gene, dof_a, n_products, k_
     ``works``: [] when the block is already there (the one-GPU emulation of the schedule in
     tests/test_gpu_parity.py), a ``_FlagWork`` when a copy engine is bringing it and will set a device
     flag (the kernel waits for it), anything else with ``wait()`` (NCCL) is waited for on the stream.
-    One persistent launch over all segments (``nsr_contract_segments``) unless a block arrives over
-    NCCL - its kernels need SMs, which a waiting persistent launch would not release - or
-    ``single_launch`` is off; then one launch per block.  Returns (P, dot): rows of block ``rank`` x
+    One persistent launch over all segments (``plan_segments``, ``nsr_contract_segments``) unless a block
+    arrives over NCCL - its kernels need SMs, which a waiting persistent launch would not release - or
+    ``single_launch`` is off; then one launch per segment.  Returns (P, dot): rows of block ``rank`` x
     all n_gene columns, owned tiles filled in.
 
-    Where the results go besides (P, dot), each column block as soon as its tiles are finished, on a
+    Where the results go besides (P, dot), each segment as soon as its tiles are finished, on a
     side stream, while the launch continues:
       out_host = (P, dot) host tensors (rows of this rank, n_gene): the same layout as (P, dot);
       home     = (P, dot) host tensors (n_gene, n_gene), the FULL symmetric matrices of the reference
@@ -414,116 +447,86 @@ def contract_plan(ctx, local, rounds, rank, world, n_gene, dof_a, n_products, k_
     else:
         P, D = out
     local.rows = max(rows_a, 1)
-    if not rows_a:
-        return P, D
-    r0 = rank * blk
     mirrored = home is not None or gather is not None
-    to_host = out_host is not None or mirrored            # (gather: to the peers)
-    copy_stream = _side_stream2(dev) if to_host else None
-    main = torch.cuda.current_stream()
-
-    segs, tiles, extra = [], [], []
-    if not skip_diag:
-        segs.append(dict(B=local, rows_b=rows_a, col0=r0, diagonal=True))
-        if mirrored:
-            segs[0]["mirror"] = (P.data_ptr() + 8 * r0, D.data_ptr() + 8 * r0, P.stride(0))
-        tiles.append(engine.coex_tiles(rows_a))
-        extra.append(dict(works=[], rect=(0, rows_a, 0, rows_a), mbuf=None, src=rank))
-    n_pairs = sum(1 for r in rounds if block_rows(n_gene, world, r[0]))
-    pairs_done = 0
-    flag_driven = single_launch and not k_chunk and all(len(r[3]) == 0 or isinstance(r[3][0], _FlagWork) for r in rounds)
-    for k, (src, parity, buf, works) in enumerate(rounds, 1):
-        rows_b = block_rows(n_gene, world, src)
-        if not rows_b:
-            continue
-        buf.rows = rows_b
-        sg = dict(B=buf, rows_b=rows_b, col0=src * blk, diagonal=False)
-        mbuf = None
-        if mirrored:
-            mbuf = _mirror_pair(dev, k, blk)
-            sg["mirror"] = (mbuf[0].data_ptr(), mbuf[1].data_ptr(), blk)
-        tl = pair_tiles(rows_a, rows_b, parity)
-        a0, a1, b0, b1 = _segment_rect(rows_a, rows_b, parity)
-        # results travelling to the host: the block pair is cut into column strips, each a segment of its own
-        # (same operands, its own `done` counter), so that a strip leaves while the next one is contracted
-        # instead of the whole rectangle waiting for its last tile
-        n_sub = 1
-        if mirrored and len(tl) and flag_driven:
-            n_sub = max(1, min(PAIR_STRIPS, (MAX_SEGMENTS - len(segs)) // max(1, n_pairs - pairs_done)))
-        pairs_done += 1
-        for sel, rect in pair_strips(tl, (a0, a1, b0, b1), n_sub):
-            segs.append(dict(sg))
-            tiles.append(sel)
-            extra.append(dict(works=works, rect=rect, mbuf=mbuf, src=src))
-
-    def send(i):
-        """queue the device-to-host copies of segment i on the copy stream"""
-        sg, ex = segs[i], extra[i]
-        c0 = sg["col0"]
-        if out_host is not None:
-            for src_t, dst_t in ((P, out_host[0]), (D, out_host[1])):
-                engine.copy_rect_to_host(ctx, dst_t, 0, c0, src_t, 0, c0, rows_a, sg["rows_b"], stream=copy_stream)
-        if home is not None:
-            a0, a1, b0, b1 = ex["rect"]
-            for t, (src_t, dst_t) in enumerate(((P, home[0]), (D, home[1]))):
-                engine.copy_rect_to_host(ctx, dst_t, r0 + a0, c0 + b0, src_t, a0, c0 + b0, a1 - a0, b1 - b0,
-                                         stream=copy_stream)
-                if ex["mbuf"] is not None:
-                    engine.copy_rect_to_host(ctx, dst_t, c0 + b0, r0 + a0, ex["mbuf"][t], b0, a0, b1 - b0, a1 - a0,
-                                             stream=copy_stream)
-        if gather is not None and ex["mbuf"] is not None:
-            a0, a1, b0, b1 = ex["rect"]
-            for t in range(2):
-                engine.copy_rect_to_peer(ctx, gather[ex["src"]][t], b0, r0 + a0, ex["mbuf"][t], b0, a0, b1 - b0,
-                                         a1 - a0, stream=copy_stream)
-
+    segs = plan_segments(rounds, rank, world, n_gene, k_chunk, single_launch, mirrored, skip_diag)
     if not segs:
         return P, D
-    flagged = all(len(ex["works"]) == 0 or isinstance(ex["works"][0], _FlagWork) for ex in extra)
+    r0 = rank * blk
+    to_host = out_host is not None or mirrored            # (gather: to the peers)
+    copy_stream = _side_stream(dev, "send") if to_host else None
+    main = torch.cuda.current_stream()
+    mbufs = {sg.k: _mirror_pair(dev, sg.k, blk) for sg in segs if mirrored and not sg.diagonal}
+
+    def operands(sg):
+        """segment sg as engine.contract_segments takes it"""
+        B = local if sg.diagonal else rounds[sg.k - 1][2]
+        B.rows = sg.rows_b
+        op = dict(B=B, rows_b=sg.rows_b, col0=sg.col0, diagonal=sg.diagonal)
+        if mirrored and sg.diagonal:
+            op["mirror"] = (P.data_ptr() + 8 * r0, D.data_ptr() + 8 * r0, P.stride(0))
+        elif mirrored:
+            op["mirror"] = (mbufs[sg.k][0].data_ptr(), mbufs[sg.k][1].data_ptr(), blk)
+        return op
+
+    def send(sg):
+        """queue the copies of segment sg's results on the copy stream"""
+        c0 = sg.col0
+        a0, a1, b0, b1 = sg.rect
+        mbuf = mbufs.get(sg.k) if not sg.diagonal else None
+        if out_host is not None:
+            for src_t, dst_t in zip((P, D), out_host):
+                engine.copy_rect_to_host(ctx, dst_t, 0, c0, src_t, 0, c0, rows_a, sg.rows_b, stream=copy_stream)
+        if home is not None:
+            for t, (src_t, dst_t) in enumerate(zip((P, D), home)):
+                engine.copy_rect_to_host(ctx, dst_t, r0 + a0, c0 + b0, src_t, a0, c0 + b0, a1 - a0, b1 - b0,
+                                         stream=copy_stream)
+                if mbuf is not None:
+                    engine.copy_rect_to_host(ctx, dst_t, c0 + b0, r0 + a0, mbuf[t], b0, a0, b1 - b0, a1 - a0,
+                                             stream=copy_stream)
+        if gather is not None and mbuf is not None:
+            for t in range(2):
+                engine.copy_rect_to_peer(ctx, gather[sg.src][t], b0, r0 + a0, mbuf[t], b0, a0, b1 - b0, a1 - a0,
+                                         stream=copy_stream)
+
+    flagged = all(len(sg.works) == 0 or isinstance(sg.works[0], _FlagWork) for sg in segs)
     if single_launch and flagged and len(segs) <= MAX_SEGMENTS:
         sync = _sync_words(ctx)
-        for sg, ex in zip(segs, extra):
-            if ex["works"]:
-                sg["ready"] = (ex["works"][0].flag_ptr, ex["works"][0].value)
         track = to_host and not k_chunk
-        if track:
-            for i, sg in enumerate(segs):
-                sg["done"] = sync.done_ptr(i)
-        tl = np.concatenate([np.concatenate([np.full((len(t), 1), i, np.int32), t], axis=1) for i, t in enumerate(tiles)])
-        _timed(events, lambda: engine.contract_segments(ctx, local, segs, tl, dof_a, P, D, n_products, k_chunk=k_chunk))
+        ops = [operands(sg) for sg in segs]
+        for i, (sg, op) in enumerate(zip(segs, ops)):
+            if sg.works:
+                op["ready"] = (sg.works[0].flag_ptr, sg.works[0].value)
+            if track:
+                op["done"] = sync.done_ptr(i)
+        tl = np.concatenate([np.concatenate([np.full((len(sg.tiles), 1), i, np.int32), sg.tiles], axis=1)
+                             for i, sg in enumerate(segs)])
+        _timed(events, lambda: engine.contract_segments(ctx, local, ops, tl, dof_a, P, D, n_products, k_chunk=k_chunk))
         if to_host:
             if not track:
                 copy_stream.wait_stream(main)
-            for i in range(len(segs)):
+            for i, sg in enumerate(segs):
                 if track:
                     # the epilogue counts every finished tile of the segment once per epilogue warp
-                    sync.done_expected[i] += EPILOGUE_WARPS * len(tiles[i])
+                    sync.done_expected[i] += EPILOGUE_WARPS * len(sg.tiles)
                     engine.stream_wait_geq(ctx, sync.done_ptr(i), sync.done_expected[i], stream=copy_stream)
-                send(i)
+                send(sg)
             main.wait_stream(copy_stream)
         return P, D
 
-    for i, (sg, ex) in enumerate(zip(segs, extra)):
-        wait_block(ex["works"])
-        tl = np.concatenate([np.zeros((len(tiles[i]), 1), np.int32), tiles[i]], axis=1)
-        _timed(events, lambda: engine.contract_segments(ctx, local, [sg], tl, dof_a, P, D, n_products, k_chunk=k_chunk))
+    for sg in segs:
+        wait_block(sg.works)
+        tl = np.concatenate([np.zeros((len(sg.tiles), 1), np.int32), sg.tiles], axis=1)
+        _timed(events, lambda: engine.contract_segments(ctx, local, [operands(sg)], tl, dof_a, P, D, n_products,
+                                                        k_chunk=k_chunk))
         if to_host:
             copy_stream.wait_stream(main)
-            send(i)
+            send(sg)
     if copy_stream is not None:
         main.wait_stream(copy_stream)
     return P, D
 
 
 EPILOGUE_WARPS = 8        # epilogue warps of the tcgen05 kernel (each counts a finished tile once)
-_SIDE2 = {}
-
-
-def _side_stream2(device):
-    key = torch.device(device).index
-    if key not in _SIDE2:
-        _SIDE2[key] = torch.cuda.Stream(device=device)
-    return _SIDE2[key]
 
 
 def _coex_strip(ctx, local, n_gene, dof_a, n_products, group, out, events=None):
@@ -541,8 +544,8 @@ def _coex_strip(ctx, local, n_gene, dof_a, n_products, group, out, events=None):
     else:
         P, D = out
     if r1 > r0:
-        _timed(events, lambda: _contract_strip(ctx, MODE_COEX_UPPER, full, full, strip_tiles(t, a, b), dof_a, P, D,
-                                               r0, n_products))
+        _timed(events, lambda: engine.contract(ctx, MODE_COEX_UPPER, full, full, strip_tiles(t, a, b), dof_a, P, D,
+                                               n_products, row0=r0))
     return P, D, full.var[:n_gene], (r0, r1)
 
 
@@ -589,11 +592,7 @@ def coex_sharded(dt_block, dc, n_gene, group=None, precision="default", dimreduc
     ctx = engine.context(dt_block.device)
     n_slices, n_products = engine.PRESETS[precision]
     n = dt_block.shape[1]
-    Qt_dev, crank, _ = covariate_basis_device(ctx, dc)
-    if n <= crank + dimreduce + 1:
-        raise ValueError('Insufficient number of cells: must be greater than degrees of freedom '
-                         'removed + covariate + 1.')
-    dof_a = (n - 1 - crank - dimreduce) / 2
+    Qt_dev, _, _, dof_a = basis_and_dof(ctx, dc, n, dimreduce)
     blk = row_split(n_gene, world)
     symm = _symm_for(blk, n, n_slices, ctx.device, group) if (schedule == "pairs" and world > 1) else None
     local = _timed(proj_events, lambda: residualize_block(ctx, dt_block, Qt_dev, n_slices, blk,
@@ -641,17 +640,11 @@ def coex_host(dt_block_host, dc, n_gene, group=None, precision="default", dimred
     n_slices, n_products = engine.PRESETS[precision]
     xh = dt_block_host if isinstance(dt_block_host, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(dt_block_host))
     n = xh.shape[1]
-    Qt_dev, crank, _ = covariate_basis_device(ctx, dc)
-    if n <= crank + dimreduce + 1:
-        raise ValueError('Insufficient number of cells: must be greater than degrees of freedom '
-                         'removed + covariate + 1.')
-    dof_a = (n - 1 - crank - dimreduce) / 2
+    Qt_dev, _, _, dof_a = basis_and_dof(ctx, dc, n, dimreduce)
     with torch.cuda.device(ctx.device):
         blk = row_split(n_gene, world)
         symm = _symm_for(blk, n, n_slices, ctx.device, group) if (schedule == "pairs" and world > 1) else None
-        local = engine.Sliced(blk, n, n_slices, ctx.device, storage=None if symm is None else symm[0])
-        if xh.shape[0] < blk:
-            local.slices.zero_(); local.quantum.fill_(1.0); local.var.fill_(1.0)
+        local = _own_block(blk, xh.shape[0], n, n_slices, ctx.device, storage=None if symm is None else symm[0])
         tail = None
         streamed = home is not None and schedule == "pairs" and xh.shape[0] > 0 and STREAM_DIAGONAL
         if streamed:
@@ -782,31 +775,11 @@ class _Team:
 _STORES = {}
 
 
-def _pull_rounds(ctx, team, rank, world, local):
-    """Single-process counterpart of ``start_exchange_ce``: pull the blocks this device needs from the other
-    devices' buffers (cudaMemcpyPeerAsync on a side stream; each copy followed by the flag write the
-    persistent contraction launch waits for)."""
-    dev = local.slices.device
-    side = _side_stream(dev)
-    side.wait_stream(torch.cuda.current_stream())
-    sync = _sync_words(ctx)
-    sync.epoch += 1
-    nbytes = team.stores[rank].numel()
-    rounds = []
-    for d, (_, src, parity) in enumerate(exchange_plan(world, rank)):
-        key = (dev.index, d, nbytes)
-        if key not in _STORES:
-            _STORES[key] = torch.empty(nbytes, dtype=torch.uint8, device=dev)
-        store = _STORES[key]
-        side.wait_event(team.ready[src])
-        engine.copy_peer(ctx, store, team.stores[src], stream=side)
-        ev = torch.cuda.Event()
-        ev.record(side)
-        work = _FlagWork(ev, sync.ready_ptr(d + 1), sync.epoch)
-        engine.stream_signal(ctx, work.flag_ptr, work.value, stream=side)
-        buf = engine.Sliced(local.rows_alloc, local.n, local.n_slices, dev, storage=store, fresh=False)
-        rounds.append((src, parity, buf, [work]))
-    return rounds
+def _kept(key, make):
+    """``_STORES[key]``, made by ``make()`` on first use: device buffers the worker threads reuse across calls."""
+    if key not in _STORES:
+        _STORES[key] = make()
+    return _STORES[key]
 
 
 def _device_worker(team, rank, world, dev, xh, dc, n_gene, precision, dimreduce, home, var_out, net=None):
@@ -819,29 +792,15 @@ def _device_worker(team, rank, world, dev, xh, dc, n_gene, precision, dimreduce,
         ctx = engine.context(dev)
         n_slices, n_products = engine.PRESETS[precision]
         n = xh.shape[1]
-        Qt_dev, crank, _ = covariate_basis_device(ctx, dc)
-        if n <= crank + dimreduce + 1:
-            raise ValueError('Insufficient number of cells: must be greater than degrees of freedom '
-                             'removed + covariate + 1.')
-        dof_a = (n - 1 - crank - dimreduce) / 2
+        Qt_dev, _, _, dof_a = basis_and_dof(ctx, dc, n, dimreduce)
         blk = row_split(n_gene, world)
         rows_a = block_rows(n_gene, world, rank)
         r0 = rank * blk
         nbytes = engine.Sliced.storage_bytes(blk, n, n_slices)
-        key = (dev.index, "own", nbytes)
-        if key not in _STORES:
-            _STORES[key] = torch.empty(nbytes, dtype=torch.uint8, device=dev)
-        store = _STORES[key]
-        local = engine.Sliced(blk, n, n_slices, dev, storage=store)
-        if rows_a < blk:
-            local.slices[:, rows_a:].zero_()
-            local.quantum[rows_a:] = 1.0
-            local.var[rows_a:] = 1.0
-        okey = (dev.index, "out", max(rows_a, 1), n_gene)
-        if okey not in _STORES:
-            _STORES[okey] = (torch.zeros((max(rows_a, 1), n_gene), dtype=torch.float64, device=dev),
-                             torch.zeros((max(rows_a, 1), n_gene), dtype=torch.float64, device=dev))
-        out = _STORES[okey]
+        store = _kept((dev.index, "own", nbytes), lambda: torch.empty(nbytes, dtype=torch.uint8, device=dev))
+        local = _own_block(blk, rows_a, n, n_slices, dev, storage=store)
+        out = _kept((dev.index, "out", max(rows_a, 1), n_gene), lambda: tuple(
+            torch.zeros((max(rows_a, 1), n_gene), dtype=torch.float64, device=dev) for _ in range(2)))
         tail = None
         streamed = rows_a > 0 and STREAM_DIAGONAL and net is None       # (streamed: the diagonal block goes home)
         if streamed:
@@ -856,20 +815,16 @@ def _device_worker(team, rank, world, dev, xh, dc, n_gene, precision, dimreduce,
             team.outs[rank] = out
             gather = team.outs
         team.barrier.wait()                       # every block's event exists
-        rounds = _pull_rounds(ctx, team, rank, world, local)
-        contract_plan(ctx, local, rounds, rank, world, n_gene, dof_a, n_products, 0, out, None, None, home=home,
-                      skip_diag=streamed, gather=gather)
-        # the optimistic single pass over the cells is verified like in _coex_pairs
-        for r in rounds:
-            wait_block(r[3])
-        em_a = local.energy_max.cpu().numpy()
-        em_b = em_a
-        for r in rounds:
-            em_b = np.maximum(em_b, r[2].energy_max.cpu().numpy())     # NaN (non-finite input) propagates
-        k_chunk = engine.plan_k_chunk(local, local, n_products, energies=(em_a, em_b))
-        if k_chunk:
-            contract_plan(ctx, local, [(r[0], r[1], r[2], []) for r in rounds], rank, world, n_gene, dof_a,
-                          n_products, k_chunk, out, None, None, home=home, gather=gather)
+        stores = [_kept((dev.index, d, nbytes), lambda: torch.empty(nbytes, dtype=torch.uint8, device=dev))
+                  for d in range(len(exchange_plan(world, rank)))]
+
+        def pull(src, dst):
+            torch.cuda.current_stream().wait_event(team.ready[src])
+            engine.copy_peer(ctx, dst, team.stores[src])
+
+        rounds = _pull_rounds(ctx, local, rank, world, stores, pull)
+        _pairs(ctx, local, rounds, rank, world, n_gene, dof_a, n_products, out, home=home, skip_diag=streamed,
+               gather=gather)
         if rows_a:
             var_out[r0:r0 + rows_a].copy_(local.var[:rows_a], non_blocking=True)
         if net is not None:
@@ -1031,25 +986,6 @@ def de_all_devices(dx, dy, dc, devices="all", **ka):
     alpha = None if res[0][2] is None else np.concatenate([r[2] for r in res], axis=1)
     vary = np.concatenate([r[4] for r in res], axis=-1)
     return P, out2, alpha, res[0][3], vary
-
-
-def _contract_strip(ctx, mode, A, B, tiles, dof_a, P, D, row0, n_products, k_chunk=None):
-    """Contract with outputs stored from global row ``row0``: hand the C ABI a base pointer that
-    is row0 rows before the strip buffers (it only dereferences rows of the listed tiles)."""
-    from . import _lib
-    ld = D.stride(0)
-    tiles = np.ascontiguousarray(tiles, dtype=np.int32)
-    off = row0 * ld * 8
-    if k_chunk is None:
-        k_chunk = engine.plan_k_chunk(A, B, n_products)
-    st = ctx.lib.nsr_contract(
-        ctx.handle, engine._stream(), engine.ENGINE_UMMA, mode,
-        A.slices.data_ptr(), A.rows, A.rows_alloc, A.quantum.data_ptr(), A.var.data_ptr(),
-        B.slices.data_ptr(), B.rows, B.rows_alloc, B.quantum.data_ptr(), B.var.data_ptr(),
-        A.n, A.n_pad, A.n_slices, n_products, tiles.ctypes.data, tiles.shape[0], float(dof_a),
-        P.data_ptr() - off, D.data_ptr() - off, ld, int(k_chunk))
-    _lib.check(st, "nsr_contract")
-    engine.LAUNCHES += 1 if not k_chunk else -(-A.n_pad // k_chunk)
 
 
 def block_spans(n_gene, world, schedule="pairs"):

@@ -291,3 +291,26 @@ def test_coexnet_all_devices_one_process(problem, monkeypatch):
         _check_coexnet(dt, dc, 0.05, ref, devices=devices)
     monkeypatch.setattr(engine, "plan_k_chunk", lambda *a, **k: 1024)
     _check_coexnet(dt, dc, 0.05, _reference(dt, dc, 0.05), devices="all")
+
+
+@gpu
+@pytest.mark.parametrize("chunked", [False, True])
+def test_all_devices_routine_on_one_gpu(problem, monkeypatch, chunked):
+    """``coex_all_devices`` and ``coexnet_all_devices`` on ONE device: the per-device routine of the block-pair
+    schedule (own block, optimistic pass, int32 bound from the energies, redo in cell chunks) with no peers.
+    Bit-identical to coex and coexnet on one GPU, dense and CSR, in one pass and with the cell chunks forced."""
+    from normalisr_b200 import engine, parallel
+    from normalisr_b200 import normalisr as norm
+    dt, dc = problem
+    if chunked:
+        monkeypatch.setattr(engine, "plan_k_chunk", lambda *a, **k: 1024)
+    P, D, var = norm.coex(dt, dc)
+    got = parallel.coex_all_devices(dt, dc, devices=[0])
+    assert all(np.array_equal(g, w) for g, w in zip(got, (P, D, var)))
+    want, _ = norm.coexnet(dt, dc, 0.05)
+    net, v = parallel.coexnet_all_devices(dt, dc, 0.05, devices=[0])
+    assert net.dtype == np.bool_ and np.array_equal(net, want) and np.array_equal(v, var)
+    want = norm.coexnet(dt, dc, 0.05, sparse=True, edge_values=True)
+    got = parallel.coexnet_all_devices(dt, dc, 0.05, sparse=True, edge_values=True, devices=[0])
+    _same_csr(got[0], want[0].toarray())
+    assert all(np.array_equal(g, w) for g, w in zip(got[1:], want[1:])) and np.array_equal(got[1], var)

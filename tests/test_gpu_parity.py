@@ -614,13 +614,16 @@ def test_de_single4_config3_shape():
     assert ref[0].min() < 1e-20
 
 
-@pytest.mark.parametrize("world", [2, 3, 4, 8])
-def test_pairs_schedule_emulated(world):
+@pytest.mark.parametrize("world,gather", [pytest.param(w, False, id=str(w)) for w in (2, 3, 4, 8)] +
+                         [pytest.param(w, True, id="%d-gather" % w) for w in (2, 3, 4, 8)])
+def test_pairs_schedule_emulated(world, gather):
     """The multi-GPU block-pair schedule, emulated on ONE device: every rank's plan (diagonal block in
     NSR_MODE_COEX_UPPER, block pairs in NSR_MODE_COEX_RECT incl. the split pair at distance world/2)
     is run in turn through the product's own ``parallel.contract_plan`` and assembled with the
     product's own ``parallel.assemble_dense``; the result must equal the single-GPU NSR_MODE_COEX
-    matrices bit for bit (ragged last block: 1,900 genes)."""
+    matrices bit for bit (ragged last block: 1,900 genes).  Results go ``home`` (the full host matrices)
+    or, with ``gather``, the transposed rectangles go into the other ranks' outputs (``coexnet_all_devices``;
+    here copies within the one device), after which every rank holds complete rows."""
     from normalisr_b200 import parallel
     n_gene, n = 1900, 3000
     ctx = engine.context(0)
@@ -639,14 +642,26 @@ def test_pairs_schedule_emulated(world):
     # the kernel's mirrored stores) - what one caller gets back from the multi-GPU path
     home = (torch.full((n_gene, n_gene), -7.0, dtype=torch.float64).pin_memory(),
             torch.full((n_gene, n_gene), -7.0, dtype=torch.float64).pin_memory())
+    outs = [tuple(torch.zeros((parallel.block_rows(n_gene, world, r), n_gene), dtype=torch.float64, device="cuda")
+                  for _ in range(2)) for r in range(world)]
     for r in range(world):
         rounds = [(src, parity, blocks[src], []) for _, src, parity in parallel.exchange_plan(world, r)]
-        P, D = parallel.contract_plan(ctx, blocks[r], rounds, r, world, n_gene, dof, prods, 0, home=home,
-                                      single_launch=(r % 2 == 0))
+        if gather:
+            P, D = parallel.contract_plan(ctx, blocks[r], rounds, r, world, n_gene, dof, prods, 0, out=outs[r],
+                                          gather=outs, single_launch=(r % 2 == 0))
+        else:
+            P, D = parallel.contract_plan(ctx, blocks[r], rounds, r, world, n_gene, dof, prods, 0, home=home,
+                                          single_launch=(r % 2 == 0))
         Ps.append(P)
         Ds.append(D)
     torch.cuda.synchronize()
-    assert torch.equal(home[0], P1.cpu()) and torch.equal(home[1], D1.cpu())
+    if gather:
+        for r in range(world):
+            r0 = r * blk
+            assert torch.equal(outs[r][0], P1[r0:r0 + outs[r][0].shape[0]])
+            assert torch.equal(outs[r][1], D1[r0:r0 + outs[r][1].shape[0]])
+    else:
+        assert torch.equal(home[0], P1.cpu()) and torch.equal(home[1], D1.cpu())
     assert torch.equal(parallel.assemble_dense(Ps, n_gene, world), P1)
     assert torch.equal(parallel.assemble_dense(Ds, n_gene, world), D1)
     assert torch.equal(torch.cat([b.var[:parallel.block_rows(n_gene, world, r)] for r, b in enumerate(blocks)]), full.var)

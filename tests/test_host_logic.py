@@ -79,6 +79,35 @@ def test_tile_lists_cover_exactly_once():
     assert len(t) == 3 * 8 and len({tuple(x) for x in t}) == 24
 
 
+def _upper_loop(js_range, col_end, rows_of, strip=12):
+    out = []
+    for js in js_range:
+        je = min(js + strip, col_end)
+        for i in rows_of(je):
+            for j in range(max(i, js), je):
+                out.append((i, j))
+    return np.asarray(out, dtype=np.int32).reshape(-1, 2)
+
+
+def test_upper_tiles_equal_the_three_tile_lists_it_replaces():
+    """One generator stands for three tile lists whose ORDER is the L2 plan of the contraction: the full upper
+    triangle (``coex_tiles``), the tiles of a column range (the streamed host pipeline) and the upper triangle of a
+    strip of tile rows (the all-gather schedule's ``strip_tiles``).  Expected values are those functions' loops."""
+    from normalisr_b200 import parallel
+    for rows in (1, 128, 129, 1000, 1900, 5000, 12345, 20000):
+        t = (rows + 127) // 128
+        want = _upper_loop(range(0, t, 12), t, lambda je: range(0, je))
+        assert np.array_equal(engine.coex_tiles(rows), want)
+        for world in range(1, 9):
+            for a, b in parallel.strip_bounds(t, world):
+                want = _upper_loop(range(a, t, 12), t, lambda je: range(a, min(b, je)))
+                got = parallel.strip_tiles(t, a, b)
+                assert got.dtype == np.int32 and np.array_equal(got, want), (rows, world, a, b)
+    for t0, t1 in ((0, 1), (0, 12), (0, 13), (3, 5), (5, 29), (12, 24), (40, 157), (150, 157), (7, 7)):
+        want = _upper_loop(range(t0, t1, 12), t1, lambda je: range(0, je))
+        assert np.array_equal(engine.upper_tiles(0, t1, t0, t1), want), (t0, t1)
+
+
 @pytest.mark.parametrize("case", ["de_single4", "de_single4_rankdef"])
 def test_single4_closed_form_equals_reference(case):
     """loo_stats on exact float64 Gram matrices reproduces the reference's single=4 numbers."""

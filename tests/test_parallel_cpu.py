@@ -65,6 +65,44 @@ def test_home_rectangles_write_every_entry_exactly_once(rows, world):
     assert (count == 1).all()
 
 
+@pytest.mark.parametrize("rows", [130, 1900, 5000, 20000])
+@pytest.mark.parametrize("world", range(1, 9))
+@pytest.mark.parametrize("mirrored", [False, True])
+def test_segment_plan_covers_every_entry_exactly_once(rows, world, mirrored):
+    """The segments ``contract_plan`` launches, as ``plan_segments`` builds them (block pairs cut into column
+    strips when the transposes are written): their rects and the transposes of them cover the (rows x rows)
+    matrix exactly once, the diagonal block's upper-triangular tiles and their transposes cover its square,
+    and every block pair's tiles cover exactly its rect."""
+    blk = parallel.row_split(rows, world)
+    count = np.zeros((rows, rows), dtype=np.int32)
+    for rank in range(world):
+        rounds = [(src, parity, None, []) for _, src, parity in parallel.exchange_plan(world, rank)]
+        segs = parallel.plan_segments(rounds, rank, world, rows, mirrored=mirrored)
+        ra, r0 = parallel.block_rows(rows, world, rank), rank * blk
+        assert len(segs) <= parallel.MAX_SEGMENTS and (ra > 0 or not segs)
+        for sg in segs:
+            a0, a1, b0, b1 = sg.rect
+            rb, c0 = parallel.block_rows(rows, world, sg.src), sg.col0
+            assert c0 == sg.src * blk and sg.rows_b == rb and sg.tiles.dtype == np.int32
+            cover = np.zeros((ra, rb), dtype=bool)
+            for ti, tj in sg.tiles:
+                cover[ti * 128:(ti + 1) * 128, tj * 128:(tj + 1) * 128] = True
+            if sg.diagonal:
+                assert sg.src == rank and sg.k == 0 and sg.rect == (0, ra, 0, ra)
+                cover |= cover.T
+                count[r0:r0 + ra, r0:r0 + ra] += 1
+            else:
+                assert rounds[sg.k - 1][0] == sg.src
+                count[r0 + a0:r0 + a1, c0 + b0:c0 + b1] += 1                # direct
+                count[c0 + b0:c0 + b1, r0 + a0:r0 + a1] += 1                # transposed copy
+            want = np.zeros((ra, rb), dtype=bool)
+            want[a0:a1, b0:b1] = True
+            assert np.array_equal(cover, want)
+        if mirrored and world > 2 and rows >= 5000:
+            assert len(segs) > 1 + len(rounds)                          # block pairs leave in strips
+    assert (count == 1).all()
+
+
 @pytest.mark.parametrize("rows_a,rows_b,parity", [(2560, 2560, None), (2560, 2440, 0), (2500, 2560, 1), (130, 100, None),
                                                   (10000, 10000, 0), (128, 128, 1)])
 @pytest.mark.parametrize("n_sub", [1, 2, 4, 8, 50])
