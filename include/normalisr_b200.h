@@ -33,6 +33,7 @@ typedef struct nsr_ctx nsr_ctx;
 #define NSR_MAX_RANK 64          /* covariate rank handled by the projection kernels */
 #define NSR_MAX_SPLITS 64        /* cell splits of the projection kernels (depends on n only) */
 #define NSR_MAX_SEGMENTS 10      /* column segments of one nsr_contract_segments launch */
+#define NSR_TOPK_MAX 2048        /* largest k of nsr_topk_strip / nsr_topk_finish */
 
 /* contraction modes */
 #define NSR_MODE_COEX 0   /* A == B, symmetric: both triangles written, diagonal = 0,
@@ -424,6 +425,24 @@ int nsr_binnet_csr_fill(nsr_ctx* ctx, uintptr_t stream, const double* P, int64_t
                         int64_t ld, int64_t diag0, const double* thr, const int64_t* indptr,
                         void* indices, int index_bytes, const double* D, int64_t ld_d, double* p_out,
                         double* d_out, unsigned long long* err);
+
+/* Every gene's k strongest co-expression partners without a genes x genes matrix (coextop).  The caller
+ * contracts one strip of tile rows [r0, r1) at a time in NSR_MODE_COEX_UPPER into P and D (strip row 0 is
+ * gene r0, leading dimension ld >= G) and calls nsr_topk_strip after each, strips in increasing order from
+ * r0 = 0 and covering [0, G).  Row r >= r0 receives (i, P[i][r], D[i][r]) for r0 <= i < min(r1, r) and, when
+ * r0 <= r < r1, (j, P[r][j], D[r][j]) for j > r; only strictly-upper entries (j > i) are read.  Ranking key
+ * r2 = dot * dot / (var_i * var_j) in float64 without FMA; order: key descending, then column ascending.
+ * state: G x k slots of 32 bytes (key, P, dot as doubles, column as int32, 4 bytes of padding), owned by the
+ * caller and left alone between calls; the launch with r0 = 0 initialises it.  var: G residual variances
+ * (coex's var).  1 <= k <= min(G - 1, NSR_TOPK_MAX).  One launch, no atomics: the result does not depend on
+ * the strip heights. */
+int nsr_topk_strip(nsr_ctx* ctx, uintptr_t stream, const double* P, const double* D, int64_t ld, int64_t r0,
+                   int64_t r1, const double* var, int64_t G, int k, void* state);
+
+/* After the last strip: the slots of `state` in rank order as idx (G x k int64 column indices), P_k and
+ * dot_k (G x k float64), row-major. */
+int nsr_topk_finish(nsr_ctx* ctx, uintptr_t stream, const void* state, int64_t G, int k, int64_t* idx,
+                    double* P_k, double* dot_k);
 
 /* Strided copy on `stream` (cudaMemcpy2DAsync): lets the host layer return finished blocks of
  * P / dot while later tiles are still being computed.  kind: 0 = device to host, 1 = host to

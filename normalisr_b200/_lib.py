@@ -15,6 +15,7 @@ KBLOCK = 128
 MAX_RANK = 64
 MAX_SPLITS = 64
 MAX_SLICES = 4
+TOPK_MAX = 2048
 
 _lib = None
 
@@ -60,6 +61,8 @@ _SIGNATURES = {
                               ctypes.POINTER(c_int)]),
     "nsr_mtx_read": (c_int, [ctypes.c_char_p, c_i64, c_vp, c_vp, c_vp, ctypes.POINTER(c_int), c_int]),
     "nsr_pvalue": (c_int, [c_vp, c_up, c_vp, c_vp, c_i64, c_i64, c_vp]),
+    "nsr_topk_strip": (c_int, [c_vp, c_up, c_vp, c_vp, c_i64, c_i64, c_i64, c_vp, c_i64, c_int, c_vp]),
+    "nsr_topk_finish": (c_int, [c_vp, c_up, c_vp, c_i64, c_int, c_vp, c_vp, c_vp]),
     "nsr_copy2d": (c_int, [c_vp, c_up, c_vp, c_i64, c_vp, c_i64, c_i64, c_i64, c_int]),
     "nsr_host_copy2d": (c_int, [c_vp, c_i64, c_vp, c_i64, c_i64, c_i64, c_int]),
     "nsr_copy_peer": (c_int, [c_vp, c_up, c_vp, c_vp, c_int, c_i64]),

@@ -1,7 +1,12 @@
-"""``normalisr.coex.coex`` on the GPU (reference src/normalisr/coex.py:4-48), and ``coexnet``, the
-reference's ``coex`` -> ``binnet`` pipeline as one call (an extension)."""
+"""``normalisr.coex.coex`` on the GPU (reference src/normalisr/coex.py:4-48), and two extensions:
+``coexnet``, the reference's ``coex`` -> ``binnet`` pipeline as one call, and ``coextop``, every gene's k
+strongest partners without a genes x genes matrix."""
 import numpy as np
 import torch
+
+# Device bytes of the two strip buffers (P and dot) of coextop; the strip is the largest multiple of 128 rows
+# that fits, and at least 128 rows.
+_STRIP_BYTES = 1 << 30
 
 
 def coex(dt, dc, **ka):
@@ -74,3 +79,60 @@ def coexnet(dt, dc, qcut, sparse=False, edge_values=False, devices=None, device=
         if edge_values:
             return res[0], var, res[1], res[2]
         return res, var
+
+
+def coextop(dt, dc, k, device=None, precision='default', dimreduce=0):
+    """Every gene's k strongest co-expression partners: ``(idx, P_k, dot_k, var)``.
+
+    idx: (G, k) int64; row i holds the k columns j != i with the largest r2_ij = dot_ij^2 / (var_i var_j),
+    in descending order, ties to the smaller column.  P_k, dot_k: (G, k) float64, coex's P and dot at
+    those entries (bit for bit); var: coex's var.  r2 ranks pairs like P wherever P has not underflowed
+    (the degrees of freedom are common to all pairs), and unlike P it still ranks them at atlas sizes.
+
+    The genes x genes matrices never exist: the upper triangle is contracted one strip of 128-row tiles at a
+    time into two strip buffers of at most ``_STRIP_BYTES``, and after each strip one kernel folds the strip's
+    pairs into every row's running top k (32 B per slot, G k slots).  One GPU (``device``); numpy in -> numpy
+    out, CUDA tensors in -> CUDA tensors out.  1 <= k <= min(G - 1, 2048).  ``precision`` and ``dimreduce``
+    as for ``coex``."""
+    from . import engine
+    from ._lib import MODE_COEX_UPPER, TILE, TOPK_MAX
+    from .association import _is_dev, _outs, _residualize_any, basis_and_dof
+    if len(dt.shape) != 2 or len(dc.shape) != 2:
+        raise ValueError('Incorrect dx/dy/dc size.')
+    n_gene, n = dt.shape
+    if dc.shape[1] != n:
+        raise ValueError('Unmatching dx/dy/dc dimensions.')
+    if n_gene <= 1:
+        raise ValueError('Wrong shape of net or namet.')
+    if np.ndim(k) != 0 or int(k) != k or not 1 <= int(k) <= min(n_gene - 1, TOPK_MAX):
+        raise ValueError('k must be an integer in [1, min(n_gene - 1, {})].'.format(TOPK_MAX))
+    k = int(k)
+    if precision not in engine.PRESETS:
+        raise ValueError('Unknown precision {}'.format(precision))
+    if np.ndim(dimreduce) != 0:
+        raise ValueError('dimreduce must be a scalar.')
+    dimreduce = int(dimreduce)
+    to_host = not _is_dev(dt)
+    ctx = engine.context(device if device is not None else (dt.device if not to_host else None))
+    n_slices, n_products = engine.PRESETS[precision]
+    Qt_dev, _, _, dof_a = basis_and_dof(ctx, dc, n, dimreduce)
+    with torch.cuda.device(ctx.device):
+        A = _residualize_any(ctx, dt, Qt_dev, n_slices, False)
+        k_chunk = engine.plan_k_chunk(A, A, n_products)
+        n_tiles = (n_gene + TILE - 1) // TILE
+        strip = max(1, _STRIP_BYTES // (16 * TILE * n_gene))
+        rows = min(strip * TILE, n_gene)
+        Ps = torch.empty((rows, n_gene), dtype=torch.float64, device=ctx.device)
+        Ds = torch.empty_like(Ps)
+        state = torch.empty((n_gene, k, 4), dtype=torch.float64, device=ctx.device)
+        for a in range(0, n_tiles, strip):
+            b = min(a + strip, n_tiles)
+            r0, r1 = a * TILE, min(b * TILE, n_gene)
+            engine.contract(ctx, MODE_COEX_UPPER, A, A, engine.upper_tiles(a, b, a, n_tiles), dof_a, Ps, Ds,
+                            n_products, k_chunk=k_chunk, row0=r0)
+            engine.topk_strip(ctx, Ps, Ds, r0, r1, A.var, k, state)
+        del Ps, Ds
+        res = engine.topk_finish(ctx, state) + (A.var,)
+        if to_host:
+            res = _outs(res)
+    return res

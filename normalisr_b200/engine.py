@@ -515,6 +515,35 @@ def pvalue(ctx, r2, a):
     return P
 
 
+def topk_strip(ctx, P, D, r0, r1, var, k, state):
+    """One strip's top-k selection (nsr_topk_strip): row 0 of P, D is row r0 of the co-expression matrix and
+    rows [r0, r1) hold its upper triangle (strip buffers written by ``contract(..., row0=r0)``, unit column
+    stride), var the (G,) residual variances, state the (G, k, 4) float64 tensor of 32-byte slots that carries
+    the selection from strip to strip (the launch with r0 = 0 initialises it)."""
+    G = var.numel()
+    assert D.stride(1) == 1 and P.shape == D.shape and P.stride() == D.stride() and D.shape[1] == G
+    assert state.is_contiguous() and state.dtype == torch.float64 and state.shape == (G, k, 4)
+    ld = D.stride(0) if D.shape[0] > 1 else G
+    _lib.check(ctx.lib.nsr_topk_strip(ctx.handle, _stream(), P.data_ptr(), D.data_ptr(), ld, int(r0),
+                                      int(r1), var.data_ptr(), G, int(k), state.data_ptr()), "nsr_topk_strip")
+    global LAUNCHES
+    LAUNCHES += 1
+
+
+def topk_finish(ctx, state):
+    """(idx, P_k, dot_k) of a finished selection (nsr_topk_finish): (G, k) int64 / float64 / float64 in rank
+    order."""
+    G, k = state.shape[0], state.shape[1]
+    idx = torch.empty((G, k), dtype=torch.int64, device=state.device)
+    P_k = torch.empty((G, k), dtype=torch.float64, device=state.device)
+    dot_k = torch.empty_like(P_k)
+    _lib.check(ctx.lib.nsr_topk_finish(ctx.handle, _stream(), state.data_ptr(), G, int(k), idx.data_ptr(),
+                                       P_k.data_ptr(), dot_k.data_ptr()), "nsr_topk_finish")
+    global LAUNCHES
+    LAUNCHES += 1
+    return idx, P_k, dot_k
+
+
 def copy_block_to_host(ctx, dst_host, src_dev, r0, r1, c0, c1, stream=None):
     """dst_host[r0:r1, c0:c1] <- src_dev[r0:r1, c0:c1] (both 2-D float64, unit column stride),
     asynchronously on ``stream`` (default: current).  dst_host should be pinned."""

@@ -11,10 +11,11 @@ tensors out.
 
 Beyond the reference's names: ``coexnet(dt, dc, qcut)``, the reference's ``coex`` -> ``binnet`` pipeline
 (``cmd_coex.sh``) as one call that keeps P and dot on the GPUs, and ``binnet(..., sparse=True)``, the network in
-CSR form.  ``coexnet`` is importable from here but not listed in ``__all__``, which keeps the reference's
+CSR form, and ``coextop(dt, dc, k)``, every gene's k strongest partners by r^2 without a genes x genes matrix.
+``coexnet`` and ``coextop`` are importable from here but not listed in ``__all__``, which keeps the reference's
 names."""
 from .binnet import binnet
-from .coex import coex, coexnet  # noqa: F401 - coexnet: an extension, see above
+from .coex import coex, coexnet, coextop  # noqa: F401 - coexnet, coextop: extensions, see above
 from .de import de
 from .lcpm import lcpm
 from .norm import compute_var, normvar
