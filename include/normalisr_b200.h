@@ -34,6 +34,7 @@ typedef struct nsr_ctx nsr_ctx;
 #define NSR_MAX_SPLITS 64        /* cell splits of the projection kernels (depends on n only) */
 #define NSR_MAX_SEGMENTS 10      /* column segments of one nsr_contract_segments launch */
 #define NSR_TOPK_MAX 2048        /* largest k of nsr_topk_strip / nsr_topk_finish */
+#define NSR_TOPK_MAX_PARTS 16    /* partial selections one nsr_topk_merge launch merges */
 
 /* contraction modes */
 #define NSR_MODE_COEX 0   /* A == B, symmetric: both triangles written, diagonal = 0,
@@ -428,12 +429,14 @@ int nsr_binnet_csr_fill(nsr_ctx* ctx, uintptr_t stream, const double* P, int64_t
 
 /* Every gene's k strongest co-expression partners without a genes x genes matrix (coextop).  The caller
  * contracts one strip of tile rows [r0, r1) at a time in NSR_MODE_COEX_UPPER into P and D (strip row 0 is
- * gene r0, leading dimension ld >= G) and calls nsr_topk_strip after each, strips in increasing order from
- * r0 = 0 and covering [0, G).  Row r >= r0 receives (i, P[i][r], D[i][r]) for r0 <= i < min(r1, r) and, when
+ * gene r0, leading dimension ld >= G) and calls nsr_topk_strip after each.  Either the strips go in increasing
+ * order from r0 = 0 and cover [0, G), or the state was set empty by nsr_topk_reset first: then the strips may
+ * come in any order and start at any r0, and the state ends up holding, for each row, the top k of the pairs
+ * in those strips only (one GPU's share of the strips, for nsr_topk_merge).  Row r >= r0 receives (i, P[i][r], D[i][r]) for r0 <= i < min(r1, r) and, when
  * r0 <= r < r1, (j, P[r][j], D[r][j]) for j > r; only strictly-upper entries (j > i) are read.  Ranking key
  * r2 = dot * dot / (var_i * var_j) in float64 without FMA; order: key descending, then column ascending.
  * state: G x k slots of 32 bytes (key, P, dot as doubles, column as int32, 4 bytes of padding), owned by the
- * caller and left alone between calls; the launch with r0 = 0 initialises it.  var: G residual variances
+ * caller and left alone between calls; the launch with r0 = 0 initialises it unless it was reset.  var: G residual variances
  * (coex's var).  1 <= k <= min(G - 1, NSR_TOPK_MAX).  One launch, no atomics: the result does not depend on
  * the strip heights. */
 int nsr_topk_strip(nsr_ctx* ctx, uintptr_t stream, const double* P, const double* D, int64_t ld, int64_t r0,
@@ -443,6 +446,20 @@ int nsr_topk_strip(nsr_ctx* ctx, uintptr_t stream, const double* P, const double
  * dot_k (G x k float64), row-major. */
 int nsr_topk_finish(nsr_ctx* ctx, uintptr_t stream, const void* state, int64_t G, int k, int64_t* idx,
                     double* P_k, double* dot_k);
+
+/* Set the `rows` x k slots of `state` empty (key -1, column INT_MAX): the start of a selection over a subset
+ * of the strips of nsr_topk_strip, in any order. */
+int nsr_topk_reset(nsr_ctx* ctx, uintptr_t stream, void* state, int64_t rows, int k);
+
+/* Merge n_parts (1 .. NSR_TOPK_MAX_PARTS) partial selections of the same `rows` rows: parts is a host array of
+ * device pointers, each to rows x k slots as nsr_topk_strip leaves them (per row sorted, the filled slots
+ * first), where a column reaches a row in at most one part (each GPU selected over different strips).  Per
+ * row, the k best filled slots of the union in rank order go to idx, P_k and dot_k (rows x k, the layout of
+ * nsr_topk_finish).  A row whose parts hold fewer than k filled slots in all writes nothing and sets *status
+ * (device int) to 1; the caller zeroes it first and raises.  One launch, no atomics: a slot's output rank is
+ * its position in its part plus the number of slots of every other part that beat it. */
+int nsr_topk_merge(nsr_ctx* ctx, uintptr_t stream, const void* const* parts, int n_parts, int64_t rows, int k,
+                   int64_t* idx, double* P_k, double* dot_k, int* status);
 
 /* Strided copy on `stream` (cudaMemcpy2DAsync): lets the host layer return finished blocks of
  * P / dot while later tiles are still being computed.  kind: 0 = device to host, 1 = host to

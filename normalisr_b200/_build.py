@@ -6,8 +6,8 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libnsr_b200.so")
-SOURCES = ["api.cu", "basis.cu", "binnet.cu", "de4.cu", "grouped.cu", "lcpm.cu", "normvar.cu", "sympinv.cu", "textio.cu", "topk.cu", "hostcopy.cu", "residual.cu", "contract_simt.cu", "contract_umma.cu", "contract_umma_splitk.cu"]
-HEADERS = ["nsr_common.cuh", "epilogue.cuh", "pvalue.cuh", "contract_route.h", os.path.join("..", "..", "include", "normalisr_b200.h")]
+SOURCES = ["api.cu", "basis.cu", "binnet.cu", "de4.cu", "grouped.cu", "lcpm.cu", "normvar.cu", "sympinv.cu", "textio.cu", "topk.cu", "topk_merge.cu", "hostcopy.cu", "residual.cu", "contract_simt.cu", "contract_umma.cu", "contract_umma_splitk.cu"]
+HEADERS = ["nsr_common.cuh", "epilogue.cuh", "pvalue.cuh", "contract_route.h", "topk.cuh", os.path.join("..", "..", "include", "normalisr_b200.h")]
 INCLUDES = {"contract_umma_splitk.cu": ["contract_umma.cu"]}      # sources that #include another source
 
 

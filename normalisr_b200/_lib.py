@@ -16,6 +16,7 @@ MAX_RANK = 64
 MAX_SPLITS = 64
 MAX_SLICES = 4
 TOPK_MAX = 2048
+TOPK_MAX_PARTS = 16
 
 _lib = None
 
@@ -63,6 +64,8 @@ _SIGNATURES = {
     "nsr_pvalue": (c_int, [c_vp, c_up, c_vp, c_vp, c_i64, c_i64, c_vp]),
     "nsr_topk_strip": (c_int, [c_vp, c_up, c_vp, c_vp, c_i64, c_i64, c_i64, c_vp, c_i64, c_int, c_vp]),
     "nsr_topk_finish": (c_int, [c_vp, c_up, c_vp, c_i64, c_int, c_vp, c_vp, c_vp]),
+    "nsr_topk_reset": (c_int, [c_vp, c_up, c_vp, c_i64, c_int]),
+    "nsr_topk_merge": (c_int, [c_vp, c_up, ctypes.POINTER(c_vp), c_int, c_i64, c_int, c_vp, c_vp, c_vp, c_vp]),
     "nsr_copy2d": (c_int, [c_vp, c_up, c_vp, c_i64, c_vp, c_i64, c_i64, c_i64, c_int]),
     "nsr_host_copy2d": (c_int, [c_vp, c_i64, c_vp, c_i64, c_i64, c_i64, c_int]),
     "nsr_copy_peer": (c_int, [c_vp, c_up, c_vp, c_vp, c_int, c_i64]),

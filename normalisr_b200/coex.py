@@ -81,7 +81,7 @@ def coexnet(dt, dc, qcut, sparse=False, edge_values=False, devices=None, device=
         return res, var
 
 
-def coextop(dt, dc, k, device=None, precision='default', dimreduce=0):
+def coextop(dt, dc, k, device=None, precision='default', dimreduce=0, devices=None):
     """Every gene's k strongest co-expression partners: ``(idx, P_k, dot_k, var)``.
 
     idx: (G, k) int64; row i holds the k columns j != i with the largest r2_ij = dot_ij^2 / (var_i var_j),
@@ -92,10 +92,12 @@ def coextop(dt, dc, k, device=None, precision='default', dimreduce=0):
     The genes x genes matrices never exist: the upper triangle is contracted one strip of 128-row tiles at a
     time into two strip buffers of at most ``_STRIP_BYTES``, and after each strip one kernel folds the strip's
     pairs into every row's running top k (32 B per slot, G k slots).  One GPU (``device``); numpy in -> numpy
-    out, CUDA tensors in -> CUDA tensors out.  1 <= k <= min(G - 1, 2048).  ``precision`` and ``dimreduce``
-    as for ``coex``."""
-    from . import engine
-    from ._lib import MODE_COEX_UPPER, TILE, TOPK_MAX
+    out, CUDA tensors in -> CUDA tensors out.  ``devices`` with more than one GPU (host input, numpy out):
+    ``parallel.coextop_all_devices``, the strips dealt out to the GPUs and the partial lists merged on the
+    devices, bit-identical to one GPU; a list of one device runs the one-GPU path there.
+    1 <= k <= min(G - 1, 2048).  ``precision`` and ``dimreduce`` as for ``coex``."""
+    from . import engine, parallel
+    from ._lib import TILE, TOPK_MAX
     from .association import _is_dev, _outs, _residualize_any, basis_and_dof
     if len(dt.shape) != 2 or len(dc.shape) != 2:
         raise ValueError('Incorrect dx/dy/dc size.')
@@ -112,6 +114,13 @@ def coextop(dt, dc, k, device=None, precision='default', dimreduce=0):
     if np.ndim(dimreduce) != 0:
         raise ValueError('dimreduce must be a scalar.')
     dimreduce = int(dimreduce)
+    if devices is not None:
+        devs = parallel.visible_devices(devices)
+        if len(devs) > 1:
+            if _is_dev(dt) or device is not None:
+                raise ValueError('devices= takes host inputs (the matrices are spread over the GPUs).')
+            return parallel.coextop_all_devices(dt, dc, k, devices=devs, precision=precision, dimreduce=dimreduce)
+        device = devs[0]
     to_host = not _is_dev(dt)
     ctx = engine.context(device if device is not None else (dt.device if not to_host else None))
     n_slices, n_products = engine.PRESETS[precision]
@@ -119,20 +128,33 @@ def coextop(dt, dc, k, device=None, precision='default', dimreduce=0):
     with torch.cuda.device(ctx.device):
         A = _residualize_any(ctx, dt, Qt_dev, n_slices, False)
         k_chunk = engine.plan_k_chunk(A, A, n_products)
-        n_tiles = (n_gene + TILE - 1) // TILE
-        strip = max(1, _STRIP_BYTES // (16 * TILE * n_gene))
-        rows = min(strip * TILE, n_gene)
-        Ps = torch.empty((rows, n_gene), dtype=torch.float64, device=ctx.device)
-        Ds = torch.empty_like(Ps)
         state = torch.empty((n_gene, k, 4), dtype=torch.float64, device=ctx.device)
-        for a in range(0, n_tiles, strip):
-            b = min(a + strip, n_tiles)
-            r0, r1 = a * TILE, min(b * TILE, n_gene)
-            engine.contract(ctx, MODE_COEX_UPPER, A, A, engine.upper_tiles(a, b, a, n_tiles), dof_a, Ps, Ds,
-                            n_products, k_chunk=k_chunk, row0=r0)
-            engine.topk_strip(ctx, Ps, Ds, r0, r1, A.var, k, state)
-        del Ps, Ds
+        top_strips(ctx, A, dof_a, n_products, k_chunk, state, 0, (n_gene + TILE - 1) // TILE)
         res = engine.topk_finish(ctx, state) + (A.var,)
         if to_host:
             res = _outs(res)
     return res
+
+
+def top_strips(ctx, A, dof_a, n_products, k_chunk, state, a, b):
+    """coextop's selection over the strips of tile rows [a, b): each strip of at most ``_STRIP_BYTES`` is
+    contracted (upper triangle, columns from the strip's first row to G) and folded into ``state`` ((G, k, 4)
+    slots).  The range (0, n_tiles) is the whole selection and initialises the state; any other range needs a
+    state set empty by ``engine.topk_reset`` first and leaves the top k of its own pairs (``nsr_topk_merge``
+    then combines the ranges)."""
+    from . import engine
+    from ._lib import MODE_COEX_UPPER, TILE
+    n_gene, k = state.shape[0], state.shape[1]
+    n_tiles = (n_gene + TILE - 1) // TILE
+    strip = max(1, _STRIP_BYTES // (16 * TILE * n_gene))
+    if b <= a:
+        return
+    rows = min(min(strip, b - a) * TILE, n_gene)
+    Ps = torch.empty((rows, n_gene), dtype=torch.float64, device=ctx.device)
+    Ds = torch.empty_like(Ps)
+    for a0 in range(a, b, strip):
+        b0 = min(a0 + strip, b)
+        r0, r1 = a0 * TILE, min(b0 * TILE, n_gene)
+        engine.contract(ctx, MODE_COEX_UPPER, A, A, engine.upper_tiles(a0, b0, a0, n_tiles), dof_a, Ps, Ds,
+                        n_products, k_chunk=k_chunk, row0=r0)
+        engine.topk_strip(ctx, Ps, Ds, r0, r1, A.var, k, state)

@@ -26,6 +26,7 @@
 #include <algorithm>
 
 #include "nsr_common.cuh"
+#include "topk.cuh"
 
 namespace {
 
@@ -38,13 +39,6 @@ constexpr int kFlush = kBuf - 32;                // merge when more than this ma
 constexpr int kRowBuf = 512;                     // survivors buffered by a strip row's CTA
 constexpr int kRowFlush = kRowBuf - kThreads;    // ... merged when more than this many wait
 constexpr int kUnroll = 4;                       // a strip row's candidate loads in flight per thread
-constexpr int kEmptyCol = INT_MAX;
-
-struct __align__(16) Slot {                      // one of a row's k slots (32 B); empty: key < 0
-    double key, p, dot;
-    int32_t col, pad;
-};
-static_assert(sizeof(Slot) == 32, "Slot is 32 bytes (nsr_topk_strip's state layout)");
 
 struct RowState {                                // per output row of the CTA, shared memory
     double thr_key;                              // the k-th slot once all k are filled, else the empty key
@@ -53,10 +47,6 @@ struct RowState {                                // per output row of the CTA, s
     int n_valid;                                 // filled slots (a prefix of the k)
     int pad;
 };
-
-__device__ __forceinline__ bool beats(double ka, int ca, double kb, int cb) {
-    return ka > kb || (ka == kb && ca < cb);
-}
 
 __device__ __forceinline__ double r2_key(double dot, double vi, double vj) {
     return __ddiv_rn(__dmul_rn(dot, dot), __dmul_rn(vi, vj));

@@ -544,6 +544,38 @@ def topk_finish(ctx, state):
     return idx, P_k, dot_k
 
 
+def topk_reset(ctx, state):
+    """Set every slot of a (rows, k, 4) float64 state empty (nsr_topk_reset): ``topk_strip`` may then fold in
+    any subset of the strips, in any order, starting at any r0."""
+    assert state.is_contiguous() and state.dtype == torch.float64 and state.dim() == 3 and state.shape[2] == 4
+    _lib.check(ctx.lib.nsr_topk_reset(ctx.handle, _stream(), state.data_ptr(), state.shape[0], int(state.shape[1])),
+               "nsr_topk_reset")
+    global LAUNCHES
+    LAUNCHES += 1
+
+
+def topk_merge(ctx, parts):
+    """(idx, P_k, dot_k) of the union of partial selections of the same rows (nsr_topk_merge): ``parts`` are
+    (rows, k, 4) float64 states on ctx's device, each left by ``topk_strip`` over a different set of strips.
+    Raises when a row's parts hold fewer than k filled slots in all (a wait for the device)."""
+    rows, k = parts[0].shape[0], parts[0].shape[1]
+    assert 1 <= len(parts) <= _lib.TOPK_MAX_PARTS
+    for s in parts:
+        assert s.is_contiguous() and s.dtype == torch.float64 and s.shape == (rows, k, 4) and s.device == ctx.device
+    idx = torch.empty((rows, k), dtype=torch.int64, device=ctx.device)
+    P_k = torch.empty((rows, k), dtype=torch.float64, device=ctx.device)
+    dot_k = torch.empty_like(P_k)
+    status = torch.zeros(1, dtype=torch.int32, device=ctx.device)
+    ptrs = (ctypes.c_void_p * len(parts))(*[s.data_ptr() for s in parts])
+    _lib.check(ctx.lib.nsr_topk_merge(ctx.handle, _stream(), ptrs, len(parts), rows, int(k), idx.data_ptr(),
+                                      P_k.data_ptr(), dot_k.data_ptr(), status.data_ptr()), "nsr_topk_merge")
+    global LAUNCHES
+    LAUNCHES += 1
+    if int(status.item()):
+        raise _lib.NsrError("nsr_topk_merge: a row's partial selections hold fewer than k = %d partners" % k)
+    return idx, P_k, dot_k
+
+
 def copy_block_to_host(ctx, dst_host, src_dev, r0, r1, c0, c1, stream=None):
     """dst_host[r0:r1, c0:c1] <- src_dev[r0:r1, c0:c1] (both 2-D float64, unit column stride),
     asynchronously on ``stream`` (default: current).  dst_host should be pinned."""

@@ -11,7 +11,8 @@ tensors out.
 
 Beyond the reference's names: ``coexnet(dt, dc, qcut)``, the reference's ``coex`` -> ``binnet`` pipeline
 (``cmd_coex.sh``) as one call that keeps P and dot on the GPUs, and ``binnet(..., sparse=True)``, the network in
-CSR form, and ``coextop(dt, dc, k)``, every gene's k strongest partners by r^2 without a genes x genes matrix.
+CSR form, and ``coextop(dt, dc, k)``, every gene's k strongest partners by r^2 without a genes x genes matrix
+(on one GPU, or with ``devices=`` on several, bit-identical).
 ``coexnet`` and ``coextop`` are importable from here but not listed in ``__all__``, which keeps the reference's
 names."""
 from .binnet import binnet

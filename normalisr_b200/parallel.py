@@ -32,7 +32,7 @@ import torch
 import torch.distributed as dist
 
 from . import engine
-from ._lib import MAX_SEGMENTS, MODE_COEX_RECT, MODE_COEX_UPPER, MODE_DE, TILE
+from ._lib import MAX_SEGMENTS, MODE_COEX_RECT, MODE_COEX_UPPER, MODE_DE, TILE, TOPK_MAX_PARTS
 from .association import basis_and_dof, covariate_basis_device
 
 
@@ -759,17 +759,20 @@ def visible_devices(devices="all"):
 
 
 class _Team:
-    """What the per-GPU worker threads of one ``coex_all_devices`` call share."""
+    """What the per-GPU worker threads of one ``coex_all_devices``, ``coexnet_all_devices`` or
+    ``coextop_all_devices`` call share."""
 
     def __init__(self, world):
         import threading
         self.barrier = threading.Barrier(world)
-        self.stores = [None] * world          # peer-readable home of every device's block
+        self.stores = [None] * world          # peer-readable home of every device's block (coextop: its Sliced)
         self.ready = [None] * world           # CUDA event: block residualised
         self.errors = [None] * world
         self.outs = [None] * world            # coexnet: every device's (P, dot) rows, the targets of the peer copies
-        self.sent = [None] * world            # coexnet: CUDA event behind a device's copies to its peers
+        self.sent = [None] * world            # CUDA event behind a device's copies to its peers (coextop: its selection)
         self.nets = [None] * world            # coexnet: every device's part of the network (host)
+        self.energy = [None] * world          # coextop: every block's digit energies (host)
+        self.states = [None] * world          # coextop: every device's partial selection, (G, k, 4) slots
 
 
 _STORES = {}
@@ -873,14 +876,14 @@ def _net_rows(ctx, team, rank, world, out, rows_a, r0, job):
     team.nets[rank] = tuple(t.cpu().numpy() for t in piece[:4 if job.edge_values else 2])
 
 
-def _run_team(devs, xh, dc, n_gene, precision, dimreduce, home, var_out, net=None):
-    """One ``_device_worker`` thread per GPU; re-raises the first error of any of them."""
+def _run_team(label, devs, worker, *args):
+    """One ``worker(team, rank, world, device, *args)`` thread per GPU; re-raises the first error of any of them
+    (a worker that fails records its error in ``team.errors`` and aborts the barrier, releasing the others).
+    ``label``: the public entry point, named in the error of a worker stopped at a broken barrier."""
     import threading
     world = len(devs)
     team = _Team(world)
-    threads = [threading.Thread(target=_device_worker, name="nsr-gpu%d" % r,
-                                args=(team, r, world, devs[r], xh, dc, n_gene, precision, dimreduce, home, var_out,
-                                      net))
+    threads = [threading.Thread(target=worker, name="nsr-gpu%d" % r, args=(team, r, world, devs[r]) + args)
                for r in range(world)]
     for t in threads:
         t.start()
@@ -890,7 +893,7 @@ def _run_team(devs, xh, dc, n_gene, precision, dimreduce, home, var_out, net=Non
     if first:
         raise first[0]
     if any(e is not None for e in team.errors):
-        raise RuntimeError("coex_all_devices: a worker stopped at a broken barrier")
+        raise RuntimeError("%s: a worker stopped at a broken barrier" % label)
     return team
 
 
@@ -915,8 +918,8 @@ def coexnet_all_devices(dt, dc, qcut, sparse=False, edge_values=False, devices="
     n_gene = xh.shape[0]
     dense_out = None if sparse else torch.empty((n_gene, n_gene), dtype=torch.uint8, pin_memory=True)
     var_out = torch.empty(n_gene, dtype=torch.float64, pin_memory=True)
-    team = _run_team(devs, xh, dc, n_gene, precision, dimreduce, None, var_out,
-                     _NetJob(qcut, sparse, edge_values, dense_out))
+    team = _run_team("coexnet_all_devices", devs, _device_worker, xh, dc, n_gene, precision, dimreduce, None,
+                     var_out, _NetJob(qcut, sparse, edge_values, dense_out))
     var = var_out.numpy()
     if not sparse:
         if any(r[1] for r in team.nets):
@@ -948,8 +951,111 @@ def coex_all_devices(dt, dc, devices="all", precision="default", dimreduce=0, ou
         out = (torch.empty((n_gene, n_gene), dtype=torch.float64, pin_memory=True),
                torch.empty((n_gene, n_gene), dtype=torch.float64, pin_memory=True))
     var_out = torch.empty(n_gene, dtype=torch.float64, pin_memory=True)
-    _run_team(devs, xh, dc, n_gene, precision, dimreduce, out, var_out)
+    _run_team("coex_all_devices", devs, _device_worker, xh, dc, n_gene, precision, dimreduce, out, var_out)
     return out[0].numpy(), out[1].numpy(), var_out.numpy()
+
+
+TopDeal = collections.namedtuple("TopDeal", "a b lo hi pulls parts")
+TopDeal.__doc__ = """One GPU's share of ``coextop_all_devices``: the strips of tile rows [a, b) it selects over; the
+rows [lo, hi) of its gene block, which it residualises and whose final lists it merges; ``pulls``, the blocks it
+copies from their owners (every other block with rows in [a * TILE, G), the rows its strips read; none for an
+empty range); ``parts``, the ranks whose selections reach rows of its block (a non-empty range starting below
+hi: their merge parts)."""
+
+
+def coextop_deal(n_gene, world):
+    """[TopDeal] per rank: tile rows dealt out with ``strip_bounds`` (equal numbers of upper tiles, so the
+    contraction and the selection are balanced alike), gene blocks with ``row_split``.  A pair (i < j) lies in
+    the strip of row i and reaches rows i and j there; the GPU owning that strip touches only rows >= its first
+    strip row, which is what ``pulls`` and ``parts`` follow from."""
+    t = (n_gene + TILE - 1) // TILE
+    blk = row_split(n_gene, world)
+    spans = [(d * blk, d * blk + block_rows(n_gene, world, d)) for d in range(world)]
+    ranges = strip_bounds(t, world)
+    deal = []
+    for r in range(world):
+        (a, b), (lo, hi) = ranges[r], spans[r]
+        pulls = [d for d in range(world) if d != r and b > a and spans[d][1] > max(spans[d][0], a * TILE)]
+        parts = [w for w in range(world) if hi > lo and ranges[w][1] > ranges[w][0] and ranges[w][0] * TILE < hi]
+        deal.append(TopDeal(a, b, lo, hi, pulls, parts))
+    return deal
+
+
+def _top_worker(team, rank, world, dev, xh, dc, n_gene, k, precision, dimreduce, out):
+    """One GPU of ``coextop_all_devices``: residualise its block into a full G-row Sliced, pull the blocks its
+    strips read from their owners, select over its strips on a reset state, then merge the partial lists of its
+    block's rows from every GPU that touched them and copy the result into ``out`` = (idx, P_k, dot_k, var)."""
+    from .association import _residualize_any
+    from .coex import top_strips
+    try:
+        torch.cuda.set_device(dev)
+        ctx = engine.context(dev)
+        n_slices, n_products = engine.PRESETS[precision]
+        n = xh.shape[1]
+        Qt_dev, _, _, dof_a = basis_and_dof(ctx, dc, n, dimreduce)
+        deal = coextop_deal(n_gene, world)
+        me = deal[rank]
+        main = torch.cuda.current_stream()
+        full = engine.Sliced(n_gene, n, n_slices, dev)
+        if me.hi > me.lo:
+            _residualize_any(ctx, xh[me.lo:me.hi], Qt_dev, n_slices, False, out=full, row_offset=me.lo)
+        ev = torch.cuda.Event()
+        ev.record()
+        team.stores[rank], team.ready[rank] = full, ev
+        team.energy[rank] = full.energy_max.cpu().numpy()
+        team.barrier.wait()                       # every block's event and energies exist
+        for d in me.pulls:
+            lo, hi, src = deal[d].lo, deal[d].hi, team.stores[d]
+            main.wait_event(team.ready[d])
+            for s in range(n_slices):
+                engine.copy_peer(ctx, full.slices[s, lo:hi], src.slices[s, lo:hi])
+            engine.copy_peer(ctx, full.quantum[lo:hi], src.quantum[lo:hi])
+            engine.copy_peer(ctx, full.var[lo:hi], src.var[lo:hi])
+        em = np.maximum.reduce(team.energy)       # NaN (non-finite input) propagates
+        k_chunk = engine.plan_k_chunk(full, full, n_products, energies=(em, em))
+        state = torch.empty((n_gene, k, 4), dtype=torch.float64, device=dev)
+        engine.topk_reset(ctx, state)
+        top_strips(ctx, full, dof_a, n_products, k_chunk, state, me.a, me.b)
+        ev = torch.cuda.Event()
+        ev.record()
+        team.sent[rank], team.states[rank] = ev, state
+        team.barrier.wait()                       # every selection's event exists
+        if me.hi > me.lo:
+            parts = []
+            for w in me.parts:
+                if w == rank:
+                    parts.append(state[me.lo:me.hi])
+                    continue
+                main.wait_event(team.sent[w])
+                parts.append(torch.empty((me.hi - me.lo, k, 4), dtype=torch.float64, device=dev))
+                engine.copy_peer(ctx, parts[-1], team.states[w][me.lo:me.hi])
+            res = engine.topk_merge(ctx, parts) + (full.var[me.lo:me.hi],)
+            for t, o in zip(res, out):
+                o[me.lo:me.hi].copy_(t, non_blocking=True)
+        main.synchronize()
+        team.barrier.wait()                       # nobody still copies from this device's planes or state
+    except BaseException as e:                    # noqa: BLE001 - re-raised by the caller
+        team.errors[rank] = e
+        team.barrier.abort()
+
+
+def coextop_all_devices(dt, dc, k, devices="all", precision="default", dimreduce=0):
+    """``coex.coextop`` on every GPU of the box from ONE process: the strips of tile rows are dealt out
+    (``coextop_deal``), every GPU keeps a partial top k for each row over its strips, and the owner of each
+    gene block merges the partial lists of its rows (``nsr_topk_merge``).  The ranking order is total and the
+    sums are exact, so the result is bit-identical to one GPU.  dt: (n_gene, n_cell) numpy array or CPU tensor
+    (k already checked by ``coextop``).  Returns (idx, P_k, dot_k, var) as numpy arrays."""
+    devs = visible_devices(devices)
+    if len(devs) > TOPK_MAX_PARTS:
+        raise ValueError("coextop takes at most %d devices" % TOPK_MAX_PARTS)
+    xh = _host_f64(dt)
+    n_gene = xh.shape[0]
+    out = (torch.empty((n_gene, k), dtype=torch.int64, pin_memory=True),
+           torch.empty((n_gene, k), dtype=torch.float64, pin_memory=True),
+           torch.empty((n_gene, k), dtype=torch.float64, pin_memory=True),
+           torch.empty(n_gene, dtype=torch.float64, pin_memory=True))
+    _run_team("coextop_all_devices", devs, _top_worker, xh, dc, n_gene, k, precision, dimreduce, out)
+    return tuple(t.numpy() for t in out)
 
 
 def de_all_devices(dx, dy, dc, devices="all", **ka):

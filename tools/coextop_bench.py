@@ -13,8 +13,19 @@ Host clock around whole calls that end with their results where the caller wants
 for device results), arms alternated after one warm-up call of each; peak device memory from torch's allocator
 above what was allocated before the call.  The results of coextop are compared with the host top-k of coex's
 P, dot and var.  The card's name and power limit are read in the same run and recorded beside the numbers.
-python tools/coextop_bench.py --out profiles/coextop_b200.json"""
+python tools/coextop_bench.py --out profiles/coextop_b200.json
+
+With ``--devices all`` (or a list such as ``0,1``) the run measures the several-GPU path instead:
+  numpy input at 100,000 cells x 20,000 genes and at 150,000 genes x 4,096 cells, k = 50: coextop on one GPU
+  against parallel.coextop_all_devices (the team path, also with a single device), arms alternated after one
+  warm-up call of each, results compared bit for bit,
+  and the digit-plane bytes each GPU pulls from its peers (from the shapes and the dealing, not timed);
+  the merge kernel alone (nsr_topk_merge, CUDA events over --merge-reps launches): 8 parts of 18,750 rows with
+  k = 50 (one owner's share at 150,000 genes on 8 GPUs, 240 MB of slots: more than the L2) and 8 parts of 2,000
+  rows with k = 2,048.
+python tools/coextop_bench.py --devices all --out profiles/coextop_devices_b200.json"""
 import argparse
+import ctypes
 import json
 import os
 import subprocess
@@ -106,6 +117,90 @@ def kernel_split(dt, dc, k):
     return out
 
 
+def merge_kernel(n_parts, rows, k, reps):
+    """ms per nsr_topk_merge launch over ``reps`` back-to-back launches (CUDA events) on ``n_parts`` parts of
+    ``rows`` x k filled slots with random keys (columns disjoint across parts); the result is checked once
+    against a sort of the union."""
+    from normalisr_b200 import engine
+    ctx = engine.context(0)
+    g = torch.Generator(device="cuda").manual_seed(SEED)
+    parts, keys, cols = [], [], []
+    for q in range(n_parts):
+        key = torch.rand((rows, k), dtype=torch.float64, device="cuda", generator=g).sort(dim=1, descending=True)[0]
+        col = q + n_parts * torch.arange(k, device="cuda").expand(rows, k)
+        st = torch.empty((rows, k, 4), dtype=torch.float64, device="cuda")
+        st[..., 0], st[..., 1], st[..., 2] = key, -key, 2 * key
+        st.view(torch.int32).view(rows, k, 8)[..., 6:] = torch.stack([col, torch.zeros_like(col)], -1).to(torch.int32)
+        parts.append(st)
+        keys.append(key)
+        cols.append(col)
+    key, col = torch.cat(keys, 1), torch.cat(cols, 1)
+    o = torch.sort(col, dim=1, stable=True)[1]
+    o = o.gather(1, torch.sort(key.gather(1, o), dim=1, descending=True, stable=True)[1])[:, :k]
+    idx, P_k, dot_k = engine.topk_merge(ctx, parts)
+    ok = bool(torch.equal(idx, col.gather(1, o)) and torch.equal(P_k, -key.gather(1, o)) and
+              torch.equal(dot_k, 2 * key.gather(1, o)))
+    ptrs = (ctypes.c_void_p * n_parts)(*[t.data_ptr() for t in parts])
+    status = torch.zeros(1, dtype=torch.int32, device="cuda")
+
+    def launch():
+        engine._lib.check(ctx.lib.nsr_topk_merge(ctx.handle, torch.cuda.current_stream().cuda_stream, ptrs, n_parts,
+                                                 rows, k, idx.data_ptr(), P_k.data_ptr(), dot_k.data_ptr(),
+                                                 status.data_ptr()), "nsr_topk_merge")
+    for _ in range(10):
+        launch()
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    e0.record()
+    for _ in range(reps):
+        launch()
+    e1.record()
+    torch.cuda.synchronize()
+    ms = e0.elapsed_time(e1) / reps
+    nbytes = n_parts * rows * k * 32 + rows * k * 24
+    return {"parts": n_parts, "rows": rows, "k": k, "launches": reps, "ms_per_launch": ms,
+            "slot_bytes_read": n_parts * rows * k * 32, "output_bytes": rows * k * 24,
+            "GBps_on_those_bytes": nbytes / ms / 1e6, "identical_to_sort": ok and int(status.item()) == 0}
+
+
+def devices_run(args, res):
+    """One GPU against ``args.devices`` from numpy input at both shapes, and the merge kernel alone."""
+    from normalisr_b200 import engine, parallel, synth
+    from normalisr_b200 import normalisr as norm
+    devs = parallel.visible_devices(args.devices if args.devices == "all" else
+                                    [int(d) for d in args.devices.split(",")])
+    res["devices"] = [str(d) for d in devs]
+    k = args.k
+    res["merge_kernel"] = [merge_kernel(8, 18750, 50, args.merge_reps), merge_kernel(8, 2000, 2048, args.merge_reps)]
+    print(json.dumps({"merge_kernel": res["merge_kernel"]}), flush=True)
+    res["arms"] = []
+    for genes, cells in ((args.genes, args.cells), (args.big_genes, args.big_cells)):
+        p = synth.device_problem(SEED, genes, cells, "cuda")
+        dt_h, dc_h = p["dt"].cpu().numpy(), p["dc"].cpu().numpy()
+        del p
+        torch.cuda.empty_cache()
+        # the team path itself (coextop(devices=) sends a one-device list down the one-GPU path)
+        arms = {"one_gpu": lambda: norm.coextop(dt_h, dc_h, k),
+                "all_devices": lambda: parallel.coextop_all_devices(dt_h, dc_h, k, devices=devs)}
+        outs = {name: fn() for name, fn in arms.items()}
+        times = {name: [] for name in arms}
+        for _ in range(args.reps):
+            for name, fn in arms.items():
+                t = time.perf_counter()
+                fn()
+                times[name].append(time.perf_counter() - t)
+        deal = parallel.coextop_deal(genes, len(devs))
+        plane_bytes = engine.Sliced.storage_bytes(1, cells, engine.PRESETS["default"][0]) - \
+            engine.Sliced.storage_bytes(0, cells, engine.PRESETS["default"][0])
+        arm = {"genes": genes, "cells": cells, "k": k, "world": len(devs),
+               "s": times, "median_s": {name: float(np.median(v)) for name, v in times.items()},
+               "identical": same(outs["all_devices"], outs["one_gpu"]),
+               "pulled_plane_bytes_per_gpu_not_timed": [sum((deal[s].hi - deal[s].lo) * plane_bytes for s in d.pulls)
+                                                        for d in deal]}
+        res["arms"].append(arm)
+        print(json.dumps(arm), flush=True)
+        del outs, dt_h, dc_h
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--cells", type=int, default=100000)
@@ -114,11 +209,21 @@ def main():
     ap.add_argument("--reps", type=int, default=3)
     ap.add_argument("--big-genes", type=int, default=150000)
     ap.add_argument("--big-cells", type=int, default=4096)
+    ap.add_argument("--devices", default=None, help='"all" or a list like 0,1: the several-GPU runs instead')
+    ap.add_argument("--merge-reps", type=int, default=200)
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
     from normalisr_b200 import normalisr as norm, synth
     torch.cuda.set_device(0)
     res = {"card": card(), "shape": {"cells": args.cells, "genes": args.genes, "k": args.k}, "reps": args.reps}
+    if args.devices:
+        devices_run(args, res)
+        if args.out:
+            os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
+            with open(args.out, "w") as f:
+                json.dump(res, f, indent=1)
+        print(json.dumps(res))
+        return
     p = synth.device_problem(SEED, args.genes, args.cells, "cuda")
     dt_d, dc_d = p["dt"], p["dc"]
     dt_h, dc_h = dt_d.cpu().numpy(), dc_d.cpu().numpy()
